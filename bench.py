@@ -19,9 +19,12 @@ events on the launch stream), `e2e` (the same metric through `iLQRController.fit
 1, 3, 4, 5 and config 2 in fp64, a few steps each) and, for N > 1, `strong` (config 2's 4096 problems split over
 the ranks) and the timed final NCCL all-gather.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...          (one rank per GPU, no collective in
                                                                  the iteration, final NCCL gather)
+
+--dump-outputs DIR writes what the last timed pass left for a caller as DIR/<name>.npy, so that two builds can
+be compared output for output on the same seeded inputs (see dump_outputs).
 """
 import argparse
 import ctypes as C
@@ -36,6 +39,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 WORKLOADS = {
@@ -360,8 +364,31 @@ def build_solver(name, dtype, dev, rank, B=None):
     return w, solver, z0_h, U_h, lo, hi, alphas
 
 
-def measure(name, dtype, steps, warmup, dev, rank, world, dist, B=None, profile=True):
-    """Device-timed passes of one workload + per-kernel times from CUDA events on the launch stream."""
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(solver, out_dir, limit=DUMP_LIMIT_BYTES, seed=0):
+    """Writes what `iLQRController.fit` hands its caller after the last pass -- trajectories Z [B,N+1,nz], controls
+    U [B,N,nu], the gains of the last accepted step K [B,N,nu,nz], the accepted costs J_opt [B] and the per-problem
+    iLQRState [B] -- as <out_dir>/<name>.npy in the solver's dtype (state as float32), with problem_index.npy
+    (float64) naming the problems written.  When the whole batch would pass `limit` bytes, a fixed seeded sample
+    of problems is written instead."""
+    arrays = {"Z": solver.view("Z"), "U": solver.view("U"), "K": solver.matrices("K_nominal"), "J_opt": solver.J_opt,
+              "state": solver.state.float()}
+    per_problem = 8 + sum(t[0].numel() * t.element_size() for t in arrays.values())
+    room = limit - 128 * (len(arrays) + 1)                    # less one .npy header per file
+    idx = torch.arange(solver.B)
+    if per_problem * solver.B > room:
+        idx = torch.randperm(solver.B, generator=torch.Generator().manual_seed(seed))[:room // per_problem].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "problem_index.npy"), idx.double().numpy())
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t[idx.to(t.device)].cpu().numpy())
+
+
+def measure(name, dtype, steps, warmup, dev, rank, world, dist, B=None, profile=True, dump_dir=None):
+    """Device-timed passes of one workload + per-kernel times from CUDA events on the launch stream.  With
+    `dump_dir`, rank 0 writes the outputs of the last timed pass there (dump_outputs), before the profiled pass."""
     from pddp_b200 import _lib
     lib = _lib.load()
     w, solver, z0_h, U_h, lo, hi, alphas = build_solver(name, dtype, dev, rank, B)
@@ -397,6 +424,8 @@ def measure(name, dtype, steps, warmup, dev, rank, world, dist, B=None, profile=
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms = float(ms.item())
     not_pd = max(not_pd, int((solver.bw_status != 0).sum().item()))
+    if dump_dir is not None and rank == 0:
+        dump_outputs(solver, dump_dir)
     rec = {"w": w, "solver": solver, "ms_per_step": ms / steps, "value": world * w["B"] * w["N"] * steps / (ms * 1e-3),
            "launches": launches, "clocks": clocks, "not_pd": not_pd, "step": step, "sync_all": sync_all,
            "host": (z0_h, U_h, lo, hi, alphas), "kernels": None}
@@ -581,7 +610,11 @@ def main():
     ap.add_argument("--dtype", default="f32", choices=["f32", "f64"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-others", action="store_true", help="skip the other_workloads / strong sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed pass (rank 0's "
+                    "problems) as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -602,7 +635,7 @@ def main():
     dtype = torch.float32 if args.dtype == "f32" else torch.float64
     peaks = measured_peaks()
 
-    rec = measure(args.workload, dtype, args.steps, args.warmup, dev, rank, world, dist)
+    rec = measure(args.workload, dtype, args.steps, args.warmup, dev, rank, world, dist, dump_dir=args.dump_outputs)
     roofline = roofline_record(args.workload, rec, dtype, peaks)
     e2e = measure_e2e(args.workload, rec, dtype, args.steps, dev, world, dist)
 
@@ -682,4 +715,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True          # the tree may be read-only; nothing of a run is written into it
     main()

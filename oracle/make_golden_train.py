@@ -144,9 +144,11 @@ def run(tag, dropout, dtype, n_data, hidden, n_iter, batch_size, lr, reg_scale, 
         os.path.join(OUT, tag + ".npz"), dropout=0 if dropout == "concrete" else 1, hidden=np.array(hidden), n_iter=n_iter,
         batch_size=batch_size, lr=lr, reg_scale=reg_scale, X=X.numpy(), U=U.numpy(), dX=dX.numpy(), p_init=p_init.numpy(),
         p_final=p_final.numpy(), grads0=first_grads[0].numpy(), loss0=float(loss0), batch_idx=idx,
-        noise=noise.astype(np.float64 if dtype == torch.float64 else np.float32),
         X_mean=model.X_mean.numpy(), X_std_inv=model.X_std_inv.numpy(), dX_mean=model.dX_mean.numpy(),
         dX_std=model.dX_std.numpy(), rate=float(model.model.drop_0.rate), reg=float(model.model.drop_0.reg))
+    # the noise is most of the bytes and barely compresses: its own file keeps each under 1 MB (tests/train_util.py)
+    np.savez_compressed(os.path.join(OUT, tag + ".noise.npz"),
+                        noise=noise.astype(np.float64 if dtype == torch.float64 else np.float32))
     print("%-28s steps %d  batches of <= %d  loss0 %.6f  |dp| %.3e" % (tag, n_iter, bs, float(loss0),
                                                                       float((p_final - p_init).abs().max())))
 

@@ -1,4 +1,7 @@
-"""Loader of the BNN-training fixtures (tests/golden/train_*.npz, written by oracle/make_golden_train.py)."""
+"""Loader of the BNN-training fixtures (tests/golden/train_*.npz, written by oracle/make_golden_train.py).
+
+A fixture may keep some of its arrays in `<tag>.<name>.npz` beside `<tag>.npz` (the recorded dropout noise of a
+large network), so that no single file passes 1 MB; `load` merges the parts."""
 import glob
 import os
 
@@ -9,12 +12,15 @@ GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def train_tags():
-    return sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN_DIR, "train_*.npz")))
+    return sorted(t for t in (os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN_DIR, "train_*.npz")))
+                  if "." not in t)
 
 
 def load(tag):
-    raw = np.load(os.path.join(GOLDEN_DIR, tag + ".npz"))
-    fx = {k: (torch.from_numpy(np.array(raw[k])) if raw[k].ndim else raw[k].item()) for k in raw.files}
+    fx = {}
+    for path in [os.path.join(GOLDEN_DIR, tag + ".npz")] + sorted(glob.glob(os.path.join(GOLDEN_DIR, tag + ".*.npz"))):
+        raw = np.load(path)
+        fx.update({k: (torch.from_numpy(np.array(raw[k])) if raw[k].ndim else raw[k].item()) for k in raw.files})
     fx["dtype"] = fx["X"].dtype
     return fx
 
