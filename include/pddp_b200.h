@@ -45,7 +45,7 @@ extern "C" {
 #define PDDP_GEO_PENDULUM 0        /* D=2, angles {0}      */
 #define PDDP_GEO_CARTPOLE 1        /* D=4, angles {2}      */
 #define PDDP_GEO_DOUBLE_CARTPOLE 2 /* D=6, angles {2,4}    */
-#define PDDP_GEO_RENDEZVOUS 3      /* D=8, no angles, action_size 4 (pddp/examples/rendezvous/model.py; known dynamics only) */
+#define PDDP_GEO_RENDEZVOUS 3      /* D=8, no angles, action_size 4 (pddp/examples/rendezvous/model.py; known and BNN dynamics) */
 
 /* pddp/controllers/ilqr.py:35-64 (iLQRState) */
 #define PDDP_STATE_UNDEFINED 0
@@ -75,7 +75,7 @@ typedef struct pddp_shape {
     int32_t B;       /* independent problems */
     int32_t N;       /* horizon */
     int32_t nz;      /* encoded state size (must equal the encoding's size for geo's D) */
-    int32_t nu;      /* action size (1 for the three pendulum-family geometries; pddp_backward: 1..PDDP_MAX_NU) */
+    int32_t nu;      /* action size of the geometry: 1 for the three pendulum-family geometries, 4 for rendezvous */
 } pddp_shape;
 
 /* Constants of a QRCost on the angle-augmented state (host memory, doubles, row-major DAxDA).
@@ -199,7 +199,9 @@ int pddp_accept_update(const pddp_shape* shape, const void* J_new, const int32_t
  * (pddp/models/bnn/modules.py:287-386 + 200-264, eval mode; the infer_noise_variables /
  * sample_input_distribution options are pddp_bnn.input_mode, use_predicted_std is pddp_bnn.eps_out); pddp_rollout_bnn replaces
  * _control_law + _trajectory_cost for the same model.  `workspace` is a device scratch buffer of
- * at least pddp_bnn_workspace_bytes(...) bytes.                                               */
+ * at least pddp_bnn_workspace_bytes(...) bytes.  Every geometry has BNN kernels; shape.nu must be its
+ * action size, and U / u_min / u_max / k / K / F_u carry all nu components.  The rendezvous cost is the
+ * plain QR cost on the state (no angle augmentation), as in the known-dynamics path.          */
 int64_t pddp_bnn_workspace_bytes(const pddp_shape* shape, const pddp_bnn* bnn, int32_t A);
 
 int pddp_linearize_bnn(const pddp_shape* shape, const pddp_bnn* bnn, const pddp_cost* cost,

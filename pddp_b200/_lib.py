@@ -20,7 +20,7 @@ GEO_INFO = {  # geo -> (D, nu, angular, non-angular)
     GEO_PENDULUM: (2, 1, (0,), (1,)),
     GEO_CARTPOLE: (4, 1, (2,), (0, 1, 3)),
     GEO_DOUBLE_CARTPOLE: (6, 1, (2, 4), (0, 1, 3, 5)),
-    GEO_RENDEZVOUS: (8, 4, (), tuple(range(8))),       # known dynamics only (ref: examples/rendezvous)
+    GEO_RENDEZVOUS: (8, 4, (), tuple(range(8))),       # ref: examples/rendezvous (known dynamics and BNN)
 }
 
 

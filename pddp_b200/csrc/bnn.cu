@@ -16,6 +16,7 @@
 #include "bnn_mlp_iface.h"
 #include "kernels.h"
 #include "profile.h"
+#include "rdv_cost.cuh"
 #include <stdio.h>
 #include <stdlib.h>
 
@@ -70,10 +71,12 @@ __global__ void bnn_init_particles_kernel(const T* z, Layout lz, int t, int zdiv
 // ------------------------------------------------------------------------------------------
 // linearise: moment matching + Jacobian of one step, a team of 1 or 2 warps per problem
 // ------------------------------------------------------------------------------------------
+// per-warp slots of the cross-warp reduction scratch: the sums are D means or D (D + 1) / 2 covariance entries
+__host__ __device__ constexpr int moment_lin_red(int D) { return D * (D + 1) / 2 > 32 ? D * (D + 1) / 2 : 32; }
 // shared-memory elements of ONE problem in bnn_moment_lin_kernel (arrays padded to 16 bytes)
-template <int D, int WPP>
+template <int D, int NU, int WPP>
 __host__ __device__ constexpr int moment_lin_smem_elems(int P) {
-    return 2 * ((P * D + 3) & ~3) + ((P * (D + 1) * D + 3) & ~3) + (WPP > 1 ? WPP * 32 : 0);
+    return 2 * ((P * D + 3) & ~3) + ((P * (D + NU) * D + 3) & ~3) + (WPP > 1 ? WPP * moment_lin_red(D) : 0);
 }
 
 template <class T>
@@ -104,18 +107,19 @@ __device__ __forceinline__ void load_row(const T* p, T* out) {
 
 // One problem = a TEAM of WPP warps (4 warps per CTA).  Phase 1, lanes = particles: eps = (X - m) U^-1, X' and the
 // per-particle Jacobian [dX'/dX | dX'/du] staged in shared memory TRANSPOSED (row c = derivative w.r.t. input c, so
-// one direction reads one contiguous row), mean and covariance by warp shuffles (+ a shared-memory step across the
+// one direction reads one contiguous row; nu control rows follow the D state rows), mean and covariance by warp shuffles (+ a shared-memory step across the
 // team's warps).  Phase 2, lanes = (input direction j, 1 of SPLIT particle subsets): the tangent of every particle
 // along j, its mean and its second moment with the centred particles, then the encode differential.
 // For the sparse encodings (everything but FULL_COVARIANCE_MATRIX) a direction moves ONE component of the input
 // particle: dX_p = s_p e_c with s_p = 1 (mean directions), eps_p[r] dU_rr/dz_j (factor directions) -- or it is the
 // control direction -- so dX'_p is one scaled row of the staged Jacobian instead of a dense D x D product
-// (the dense form added exact zeros: same values).
+// (the dense form added exact zeros: same values).  The rendezvous geometry (D = 8, nu = 4) has up to 76 directions
+// (full covariance); it runs 4 warps per problem, and the directions loop when they outnumber the team's lanes.
 template <class T, int GEO, int ENC, int WPP>
-__global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::D <= 4) ? 8 : (sizeof(T) == 4 ? 4 : 1)) bnn_moment_lin_kernel(const MomentLinArgs<T> a) {
+__global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::D <= 4) ? 8 : (sizeof(T) == 4 && Geo<GEO>::D <= 6 ? 4 : 1)) bnn_moment_lin_kernel(const MomentLinArgs<T> a) {
     typedef Geo<GEO> G;
     constexpr int D = G::D, NU = G::NU, NZ = enc_size(D, ENC), NT = D * (D + 1) / 2, TL = WPP * 32, PPB = 4 / WPP;
-    static_assert(NU == 1, "BNN geometries are the action_size-1 problems");
+    constexpr int RED = moment_lin_red(D), NJAC = D * (D + NU);
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int slot = warp / WPP, wq = warp % WPP, tl = wq * 32 + lane;
@@ -123,14 +127,14 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
     if (b >= a.B) return;                                 // (the whole team leaves together)
     if (a.active && a.active[b] != 1) return;
     const int P = a.P, t = a.t;
-    const int PD4 = (P * D + 3) & ~3, PG4 = (P * (D + 1) * D + 3) & ~3;
-    T* sm = reinterpret_cast<T*>(smem_raw) + (size_t)slot * moment_lin_smem_elems<D, WPP>(P);
+    const int PD4 = (P * D + 3) & ~3, PG4 = (P * NJAC + 3) & ~3;
+    T* sm = reinterpret_cast<T*>(smem_raw) + (size_t)slot * moment_lin_smem_elems<D, NU, WPP>(P);
     T *s_eps = sm, *s_xc = sm + PD4, *s_G = sm + 2 * PD4, *s_red = s_G + PG4;   // eps, X'-M', [dX'/dX | dX'/du]^T, scratch
     auto team_sync = [&]() {
         if constexpr (WPP == 1) __syncwarp();
         else asm volatile("bar.sync %0, %1;" ::"r"(1 + slot), "r"(TL) : "memory");
     };
-    // sums of N <= 32 per-lane values over the team
+    // sums of N <= RED per-lane values over the team
     auto team_sum = [&](auto& v) {
         constexpr int N = (int)(sizeof(v) / sizeof(v[0]));
 #pragma unroll
@@ -138,14 +142,14 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
         if constexpr (WPP > 1) {
             if (lane == 0) {
 #pragma unroll
-                for (int i = 0; i < N; ++i) s_red[wq * 32 + i] = v[i];
+                for (int i = 0; i < N; ++i) s_red[wq * RED + i] = v[i];
             }
             team_sync();
 #pragma unroll
             for (int i = 0; i < N; ++i) {
                 T acc = s_red[i];
 #pragma unroll
-                for (int w2 = 1; w2 < WPP; ++w2) acc += s_red[w2 * 32 + i];
+                for (int w2 = 1; w2 < WPP; ++w2) acc += s_red[w2 * RED + i];
                 v[i] = acc;
             }
             team_sync();
@@ -164,11 +168,11 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
     for (int d = 0; d < D; ++d) msum[d] = T(0);
     for (int p = tl; p < P; p += TL) {
         const size_t g = (size_t)b * P + p;
-        alignas(16) T x[D], xn[D], jac[D * (D + 1)];
+        alignas(16) T x[D], xn[D], jac[NJAC];
         T delta[D], eps[D];
         load_row<D, T>(a.X + g * D, x);
         load_row<D, T>(a.Xn + g * D, xn);
-        load_row<D * (D + 1), T>(a.Jp + g * D * (D + 1), jac);
+        load_row<NJAC, T>(a.Jp + g * NJAC, jac);
 #pragma unroll
         for (int d = 0; d < D; ++d) delta[d] = x[d] - z[d];
         solve_right_upper<D, T>(U, delta, eps);
@@ -178,7 +182,7 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
             s_xc[p * D + d] = xn[d];
             msum[d] += xn[d];
 #pragma unroll
-            for (int c = 0; c <= D; ++c) s_G[(p * (D + 1) + c) * D + d] = jac[d * (D + 1) + c];
+            for (int c = 0; c < D + NU; ++c) s_G[(p * (D + NU) + c) * D + d] = jac[d * (D + NU) + c];
         }
     }
     T M[D];
@@ -241,6 +245,7 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
             for (int r = 0; r < D; ++r)
 #pragma unroll
                 for (int c = 0; c < D; ++c) dUd[r][c] = T(0);
+            const int ju = j >= NZ ? j - NZ : 0;      // control component of a control direction
             if (j >= NZ) du = T(1);
             else if (j >= D) {
                 // symmetrised direction (E_ab + E_ba)/2 through the Cholesky differential
@@ -254,11 +259,16 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
                 chol_upper_diff<D, T>(U, S, dUd);
             }
             for (int p = sub; p < P; p += SPLIT) {
-                alignas(16) T eps[D], xc[D], g[D + 1][D];
+                alignas(16) T eps[D], xc[D], g[D + 1][D];     // rows of dX'/dX, then the row of control ju
                 T dx[D];
                 load_row<D, T>(s_eps + p * D, eps);
                 load_row<D, T>(s_xc + p * D, xc);
-                load_row<(D + 1) * D, T>(s_G + p * (D + 1) * D, &g[0][0]);
+                if constexpr (NU == 1) {
+                    load_row<(D + 1) * D, T>(s_G + p * (D + 1) * D, &g[0][0]);
+                } else {
+                    load_row<D * D, T>(s_G + p * (D + NU) * D, &g[0][0]);
+                    load_row<D, T>(s_G + (p * (D + NU) + D + ju) * D, g[D]);
+                }
 #pragma unroll
                 for (int c = 0; c < D; ++c) {
                     T v = dm[c];
@@ -279,7 +289,7 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
         } else {
             // row of the staged Jacobian this direction reads, the eps component that scales it (-1: none) and
             // the constant factor dU_rr/dz_j
-            int row = j < D ? j : D, er = -1;
+            int row = j < D ? j : (j >= NZ ? D + j - NZ : D), er = -1;
             T wgt = T(1);
             if (j >= D && j < NZ) {
                 if (ENC == ENC_UT) {
@@ -297,7 +307,7 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
             }
             for (int p = sub; p < P; p += SPLIT) {
                 alignas(16) T xc[D], g[D];
-                load_row<D, T>(s_G + (p * (D + 1) + row) * D, g);
+                load_row<D, T>(s_G + (p * (D + NU) + row) * D, g);
                 T sc = T(1);
                 if (ENC != ENC_IGNORE && er >= 0) sc = s_eps[p * D + er] * wgt;
                 if (ENC != ENC_IGNORE) load_row<D, T>(s_xc + p * D, xc);
@@ -357,23 +367,25 @@ __global__ void __launch_bounds__(128, (sizeof(T) == 4 && WPP == 1 && Geo<GEO>::
             for (int r = 0; r < NZ; ++r) a.F_z[a.lFz.at(b, t, r * NZ + j)] = col[r];
         } else {
 #pragma unroll
-            for (int r = 0; r < NZ; ++r) a.F_u[a.lFu.at(b, t, r)] = col[r];
+            for (int r = 0; r < NZ; ++r) a.F_u[a.lFu.at(b, t, r * NU + (j - NZ))] = col[r];
         }
     }
 }
 
-// clamp the nominal controls of EVERY step into uall[t][b] (the MLP of step t reads row t) and park them in the
+// clamp the nominal controls of EVERY step into uall[t][b][nu] (the MLP of step t reads row t) and park them in the
 // problem layout for the cost pass -- one launch instead of one per time step (they do not depend on the state)
 template <class T>
-__global__ void bnn_lin_control_kernel(int B, int N, const T* U, Layout lU, const T* u_min, const T* u_max,
+__global__ void bnn_lin_control_kernel(int B, int N, int nu, const T* U, Layout lU, const T* u_min, const T* u_max,
                                        T* uall, T* U_clamped) {
     const long long id = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (id >= (long long)B * N) return;
     const int t = (int)(id / B), b = (int)(id - (long long)t * B);
-    T u = U[lU.at(b, t, 0)];
-    if (u_min && u_max) u = clampv(u, u_min[0], u_max[0]);
-    uall[id] = u;
-    U_clamped[lU.at(b, t, 0)] = u;
+    for (int j = 0; j < nu; ++j) {
+        T u = U[lU.at(b, t, j)];
+        if (u_min && u_max) u = clampv(u, u_min[j], u_max[j]);
+        uall[id * nu + j] = u;
+        U_clamped[lU.at(b, t, j)] = u;
+    }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -386,7 +398,7 @@ struct RollStepArgs {
     const T* Xn;                  // [B*A, P, D] particles after the MLP of step t
     const T* Z; const T* U; const T* k; const T* K; const T* alphas; const T* u_min; const T* u_max;
     const int32_t* active; const int32_t* bw_status;
-    T* Zall; T* Uall; T* ucur; T* J;          // [B*A, N+1, nz], [B*A, N], [B*A], [B*A]
+    T* Zall; T* Uall; T* ucur; T* J;          // [B*A, N+1, nz], [B*A, N, nu], [B*A, nu], [B*A]
     int32_t* status;
     Layout lZ, lU, lk, lK;
 };
@@ -395,14 +407,17 @@ struct RollStepArgs {
 // the [pair][particle][D] array: a single cp.async.bulk stages it in shared memory while the threads that will finish
 // the pairs already fetch their rows of the nominal trajectory and the gains (Z[t+1], K[t+1], k, U: ilqr.py:701-719).
 // Phase A: LPP (8 or 4) lanes per pair reduce mean and covariance from shared memory (xor-shuffles); phase B: the
-// first 256 / LPP threads, one per pair, do the encode (Cholesky), control law and moment-matched cost.
+// first 256 / LPP threads, one per pair, do the encode (Cholesky), control law and moment-matched cost.  With nu > 1
+// (rendezvous: K is 4 x nz, up to 288 values) the gains and the reference row are streamed inside the control law
+// instead of being prefetched into registers, and the cost is the rendezvous QR cost on the un-augmented state.
 // (History: one thread per pair issued 2 x P strided 4-byte loads per sector and ran at 9 % issue utilisation; 8 lanes
 // per pair reading global memory directly spent the launch in 2 x P / LPP dependent round trips to L2: 28 us.)
 // STAGE = false: the particles of 32 pairs do not fit shared memory (very large P): phase A reads them from global memory.
 template <class T, int GEO, int ENC, int LPP, bool STAGE = true>
 __global__ void __launch_bounds__(256) bnn_roll_step_kernel(const RollStepArgs<T> a) {
     typedef Geo<GEO> G;
-    constexpr int D = G::D, NZ = enc_size(D, ENC), NT = D * (D + 1) / 2, PPC = 256 / LPP;
+    constexpr int D = G::D, NU = G::NU, NZ = enc_size(D, ENC), NT = D * (D + 1) / 2, PPC = 256 / LPP;
+    constexpr int NZP = NU == 1 ? NZ : 1;                    // prefetched reference row and gains (nu == 1 only)
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ T s_mom[PPC][D + NT];
     __shared__ __align__(8) uint64_t s_bar;
@@ -425,14 +440,20 @@ __global__ void __launch_bounds__(256) bnn_roll_step_kernel(const RollStepArgs<T
     const bool fin = tid < PPC && sB < S;
     int b = 0, al = 0;
     bool run = false;
-    T zref[NZ], Krow[NZ], kk = T(0), uu = T(0), alpha = T(0), Jprev = T(0);
+    T zref[NZP], Krow[NZP], kk[NU], uu[NU], alpha = T(0), Jprev = T(0);
+#pragma unroll
+    for (int i = 0; i < NU; ++i) kk[i] = uu[i] = T(0);
     if (fin) {
         b = (int)(sB / a.A); al = (int)(sB - (long long)b * a.A);
         run = !((a.active && a.active[b] == 0) || (a.bw_status && a.bw_status[b] != 0));
         if (run && t1 < a.N) {
+            if constexpr (NU == 1) {
 #pragma unroll
-            for (int e = 0; e < NZ; ++e) { zref[e] = a.Z[a.lZ.at(b, t1, e)]; Krow[e] = a.K[a.lK.at(b, t1, e)]; }
-            kk = a.k[a.lk.at(b, t1, 0)]; uu = a.U[a.lU.at(b, t1, 0)]; alpha = a.alphas[al];
+                for (int e = 0; e < NZ; ++e) { zref[e] = a.Z[a.lZ.at(b, t1, e)]; Krow[e] = a.K[a.lK.at(b, t1, e)]; }
+            }
+#pragma unroll
+            for (int i = 0; i < NU; ++i) { kk[i] = a.k[a.lk.at(b, t1, i)]; uu[i] = a.U[a.lU.at(b, t1, i)]; }
+            alpha = a.alphas[al];
         }
         if (run && a.t >= 0) Jprev = a.J[sB];
     }
@@ -511,25 +532,47 @@ __global__ void __launch_bounds__(256) bnn_roll_step_kernel(const RollStepArgs<T
     if (!ok && a.status) atomicOr(&a.status[b], 2);
     T J = Jprev;
     if (t1 < a.N) {                                       // control law (ref: ilqr.py:701-719)
-        T du = alpha * kk;
+        T du[NU];
 #pragma unroll
-        for (int e = 0; e < NZ; ++e) du += (zn[e] - zref[e]) * Krow[e];
-        T u = uu + du;
-        if (a.u_min && a.u_max) u = clampv(u, a.u_min[0], a.u_max[0]);
-        a.ucur[s] = u;
-        a.Uall[(size_t)s * a.N + t1] = u;
-        T la, lu, luu;
-        cost_action(a.cost, u, la, lu, luu);
-        J += cost_state<GEO, ENC, T, T>(a.cost, zn, false) + la;
+        for (int i = 0; i < NU; ++i) du[i] = alpha * kk[i];
+        if constexpr (NU == 1) {
+#pragma unroll
+            for (int e = 0; e < NZ; ++e) du[0] += (zn[e] - zref[e]) * Krow[e];
+        } else {
+            const T* pK = a.K + a.lK.at(b, t1, 0);
+            const int64_t seK = a.lK.se;
+#pragma unroll 4
+            for (int e = 0; e < NZ; ++e) {
+                const T dz = zn[e] - a.Z[a.lZ.at(b, t1, e)];
+#pragma unroll
+                for (int i = 0; i < NU; ++i) du[i] += dz * pK[(i * NZ + e) * seK];
+            }
+        }
+        T u[NU];
+#pragma unroll
+        for (int i = 0; i < NU; ++i) {
+            u[i] = uu[i] + du[i];
+            if (a.u_min && a.u_max) u[i] = clampv(u[i], a.u_min[i], a.u_max[i]);
+            a.ucur[s * NU + i] = u[i];
+            a.Uall[((size_t)s * a.N + t1) * NU + i] = u[i];
+        }
+        if constexpr (GEO == GEO_RENDEZVOUS) {
+            J += rdv_cost_state<ENC, T>(a.cost, zn, false) + rdv_cost_action(a.cost, u);
+        } else {
+            T la, lu, luu;
+            cost_action(a.cost, u[0], la, lu, luu);
+            J += cost_state<GEO, ENC, T, T>(a.cost, zn, false) + la;
+        }
     } else {
-        J += cost_state<GEO, ENC, T, T>(a.cost, zn, true);
+        if constexpr (GEO == GEO_RENDEZVOUS) J += rdv_cost_state<ENC, T>(a.cost, zn, true);
+        else J += cost_state<GEO, ENC, T, T>(a.cost, zn, true);
     }
     a.J[s] = J;
 }
 
 // argmin over alphas (torch semantics) + copy of the winner, one warp per problem
 template <class T>
-__global__ void bnn_roll_select_kernel(int B, int N, int A, int nz, const T* J, const T* Zall, const T* Uall,
+__global__ void bnn_roll_select_kernel(int B, int N, int A, int nz, int nu, const T* J, const T* Zall, const T* Uall,
                                        const int32_t* active, const int32_t* bw_status, T* J_all,
                                        int32_t* amin, T* J_new, T* Z_new, T* U_new, Layout lZ, Layout lU) {
     const int lane = threadIdx.x & 31;
@@ -548,7 +591,7 @@ __global__ void bnn_roll_select_kernel(int B, int N, int A, int nz, const T* J, 
     if (lane == 0) { amin[b] = best; J_new[b] = bj; }
     const size_t s = (size_t)b * A + best;
     for (int i = lane; i < (N + 1) * nz; i += 32) Z_new[lZ.at(b, i / nz, i % nz)] = Zall[s * (N + 1) * nz + i];
-    for (int i = lane; i < N; i += 32) U_new[lU.at(b, i, 0)] = Uall[s * N + i];
+    for (int i = lane; i < N * nu; i += 32) U_new[lU.at(b, i / nu, i % nu)] = Uall[s * N * nu + i];
 }
 
 // ------------------------------------------------------------------------------------------
@@ -563,9 +606,9 @@ struct Workspace {
 
 template <class T>
 static Workspace<T> carve(void* base, const pddp_shape* s, const pddp_bnn* n, int A) {
-    const int D = s->geo == GEO_PENDULUM ? 2 : s->geo == GEO_CARTPOLE ? 4 : 6;
-    const int DA = s->geo == GEO_PENDULUM ? 3 : s->geo == GEO_CARTPOLE ? 5 : 8;
-    const size_t K0 = DA + 1, S = (size_t)s->B * (A > 1 ? A : 1), P = n->P;
+    const GeoDims gd = geo_dims(s->geo);
+    const int D = gd.D, NU = gd.NU;
+    const size_t K0 = gd.DA + NU, S = (size_t)s->B * (A > 1 ? A : 1), P = n->P;
     Workspace<T> w;
     size_t off = 0;
     auto take = [&](size_t elems) { T* p = reinterpret_cast<T*>(reinterpret_cast<char*>(base) + off); off += ((elems * sizeof(T) + 255) / 256) * 256; return p; };
@@ -576,11 +619,11 @@ static Workspace<T> carve(void* base, const pddp_shape* s, const pddp_bnn* n, in
     w.m1T = take((size_t)n->H1 * P);
     w.Xa = take(S * P * D);
     w.Xb = take(S * P * D);
-    w.Jp = take((size_t)s->B * P * D * (D + 1));
-    w.ucur = take(S);
+    w.Jp = take((size_t)s->B * P * D * (D + NU));
+    w.ucur = take(S * NU);
     w.J = take(S);
     w.Zall = take(S * (s->N + 1) * s->nz);
-    w.Uall = take(S * s->N);
+    w.Uall = take(S * s->N * NU);
     w.im.W1img = reinterpret_cast<unsigned char*>(take(P * tc::IMG_W1_PSTRIDE / sizeof(T)));        // per-particle (compacted) images
     w.im.W0img = reinterpret_cast<unsigned char*>(take(P * tc::IMG_W0_PSTRIDE / sizeof(T)));
     w.im.W2p = reinterpret_cast<float*>(take(P * (size_t)tc::IMG_TILE_N * 8 * sizeof(float) / sizeof(T)));
@@ -608,9 +651,9 @@ static BnnNet<T> make_net(const pddp_bnn* n, const Workspace<T>& w) {
 
 template <class T>
 static cudaError_t prep_weights(const pddp_shape* s, const pddp_bnn* n, const Workspace<T>& w, cudaStream_t st) {
-    const int D = s->geo == GEO_PENDULUM ? 2 : s->geo == GEO_CARTPOLE ? 4 : 6;
-    const int DA = s->geo == GEO_PENDULUM ? 3 : s->geo == GEO_CARTPOLE ? 5 : 8;
-    bnn_transpose_kernel<T><<<8, 256, 0, st>>>((const T*)n->W0, n->H0, DA + 1, n->H0, w.W0T);
+    const GeoDims gd = geo_dims(s->geo);
+    const int D = gd.D;
+    bnn_transpose_kernel<T><<<8, 256, 0, st>>>((const T*)n->W0, n->H0, gd.DA + gd.NU, n->H0, w.W0T);
     bnn_transpose_kernel<T><<<64, 256, 0, st>>>((const T*)n->W1, n->H1, n->H0, n->H1, w.W1T);
     bnn_transpose_kernel<T><<<8, 256, 0, st>>>((const T*)n->W2, 2 * D, n->H1, n->eps_out ? 2 * D : D, w.W2T);
     bnn_transpose_kernel<T><<<16, 256, 0, st>>>((const T*)n->mask0, n->P, n->H0, n->P, w.m0T);
@@ -673,20 +716,21 @@ static cudaError_t linearize_bnn_impl(const BnnCall& c) {
     MomentLinArgs<T> m;
     m.B = B; m.N = N; m.P = P; m.Jp = w.Jp; m.active = c.active; m.Z = Z; m.F_z = (T*)c.F_z; m.F_u = (T*)c.F_u;
     m.status = c.status; m.lZ = lZ; m.lFz = make_layout(ly, B, N, nz * nz); m.lFu = make_layout(ly, B, N, nz * nu);
-    // warps per problem: two when there are more input directions than lanes (double cartpole, full covariance: 43)
-    constexpr int WPP = enc_size(D, ENC) + G::NU > 32 ? 2 : 1, ppb = 4 / WPP;
-    const size_t msmem = (size_t)ppb * moment_lin_smem_elems<D, WPP>(P) * sizeof(T);
+    // warps per problem: two when there are more input directions than lanes (double cartpole, full covariance: 43);
+    // four for the rendezvous encodings with more than 32 (UT: 48, full covariance: 76)
+    constexpr int NJ = enc_size(D, ENC) + G::NU, WPP = NJ > 32 ? (GEO == GEO_RENDEZVOUS ? 4 : 2) : 1, ppb = 4 / WPP;
+    const size_t msmem = (size_t)ppb * moment_lin_smem_elems<D, G::NU, WPP>(P) * sizeof(T);
     auto mk = bnn_moment_lin_kernel<T, GEO, ENC, WPP>;
     CK(cudaFuncSetAttribute(mk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem));
 
     BnnMlpArgs<T> a;
     a.net = net; a.Jp = w.Jp; a.total = total;
     T *cur = w.Xa, *nxt = w.Xb;
-    // (w.Uall is [B * N] in this pass: the all-alpha control buffer of the rollout pass, free here)
+    // (w.Uall is [N, B, nu] in this pass: the all-alpha control buffer of the rollout pass, free here)
     bnn_lin_control_kernel<T><<<(unsigned)(((long long)B * N + 255) / 256), 256, 0, c.st>>>(
-        B, N, (const T*)c.U, lU, (const T*)c.u_min, (const T*)c.u_max, w.Uall, (T*)c.L_u);
+        B, N, nu, (const T*)c.U, lU, (const T*)c.u_min, (const T*)c.u_max, w.Uall, (T*)c.L_u);
     for (int t = 0; t < N; ++t) {
-        a.u = w.Uall + (size_t)t * B;
+        a.u = w.Uall + (size_t)t * B * nu;
         if (mode != PDDP_BNN_INPUT_INFER && t > 0)
             bnn_init_particles_kernel<T, GEO, ENC><<<igrid, 128, 0, c.st>>>(Z, lZ, t, 1, 1, B, P, eps_of(t), c.active, 1,
                                                                             nullptr, cur, c.status);
@@ -712,10 +756,13 @@ static cudaError_t linearize_bnn_impl(const BnnCall& c) {
     cd.lZ = lZ; cd.lU = lU; cd.lL = make_layout(ly, B, N + 1, 1); cd.lLz = make_layout(ly, B, N + 1, nz);
     cd.lLu = make_layout(ly, B, N, nu); cd.lLzz = make_layout(ly, B, N + 1, nz * nz);
     cd.lLuz = make_layout(ly, B, N, nu * nz); cd.lLuu = make_layout(ly, B, N, nu * nu);
-    note_launches((use_tensor_cores<T>(c.n->H0, c.n->H1) ? 10 : 5) + 3 + 2LL * N + 2 + (s->enc == PDDP_ENC_FULL_COVARIANCE_MATRIX ? 1 : 0)
+    note_launches((use_tensor_cores<T>(c.n->H0, c.n->H1) ? 10 : 5) + 3 + 2LL * N + 2
+                  + (s->enc == PDDP_ENC_FULL_COVARIANCE_MATRIX && GEO != GEO_RENDEZVOUS ? 1 : 0)
                   + (mode != PDDP_BNN_INPUT_INFER ? N - 1 : 0));
     prof_begin(PROF_COST, c.st);
-    cudaError_t ce = cost_derivatives<T>(s->geo, s->enc, cd, c.st);
+    // rendezvous: the closed-form QR cost on the un-augmented state (the known-dynamics path's cost kernel)
+    cudaError_t ce = GEO == GEO_RENDEZVOUS ? cost_derivatives_lq<T>(s->enc, cd, c.st)
+                                           : cost_derivatives<T>(s->geo, s->enc, cd, c.st);
     prof_end(PROF_COST, c.st);
     return ce;
 }
@@ -786,7 +833,7 @@ static cudaError_t rollout_bnn_impl(const BnnRollCall& c) {
         T* tmp = cur; cur = nxt; nxt = tmp;
     }
     bnn_roll_select_kernel<T><<<(unsigned)(((long long)B * 32 + 127) / 128), 128, 0, c.st>>>(
-        B, N, A, nz, w.J, w.Zall, w.Uall, c.active, c.bw_status, (T*)c.J_all, c.amin, (T*)c.J_new, (T*)c.Z_new,
+        B, N, A, nz, nu, w.J, w.Zall, w.Uall, c.active, c.bw_status, (T*)c.J_all, c.amin, (T*)c.J_new, (T*)c.Z_new,
         (T*)c.U_new, r.lZ, r.lU);
     note_launches((use_tensor_cores<T>(c.n->H0, c.n->H1) ? 10 : 5) + 2 + 2LL * N + 1 + (mode != PDDP_BNN_INPUT_INFER ? N - 1 : 0));
     return cudaGetLastError();
@@ -809,6 +856,11 @@ static cudaError_t rollout_bnn_impl(const BnnRollCall& c) {
         case GEO_DOUBLE_CARTPOLE * 8 + ENC_FULL: return IMPL<T, GEO_DOUBLE_CARTPOLE, ENC_FULL>(call);     \
         case GEO_DOUBLE_CARTPOLE * 8 + ENC_UT: return IMPL<T, GEO_DOUBLE_CARTPOLE, ENC_UT>(call);         \
         case GEO_DOUBLE_CARTPOLE * 8 + ENC_IGNORE: return IMPL<T, GEO_DOUBLE_CARTPOLE, ENC_IGNORE>(call); \
+        case GEO_RENDEZVOUS * 8 + ENC_FULL: return IMPL<T, GEO_RENDEZVOUS, ENC_FULL>(call);               \
+        case GEO_RENDEZVOUS * 8 + ENC_UT: return IMPL<T, GEO_RENDEZVOUS, ENC_UT>(call);                   \
+        case GEO_RENDEZVOUS * 8 + ENC_VAR: return IMPL<T, GEO_RENDEZVOUS, ENC_VAR>(call);                 \
+        case GEO_RENDEZVOUS * 8 + ENC_STD: return IMPL<T, GEO_RENDEZVOUS, ENC_STD>(call);                 \
+        case GEO_RENDEZVOUS * 8 + ENC_IGNORE: return IMPL<T, GEO_RENDEZVOUS, ENC_IGNORE>(call);           \
         default: return cudaErrorInvalidValue;                                                            \
     }
 
@@ -826,7 +878,7 @@ int pddp_capi_check_shape(const pddp_shape* s);         // capi.cu
 static int check_bnn(const pddp_shape* s, const pddp_bnn* n) {
     if (int e = pddp_capi_check_shape(s)) return e;
     if (s->layout != PDDP_PROBLEM_MAJOR) return pddp_capi_fail(PDDP_E_UNSUPPORTED, "BNN path uses PDDP_PROBLEM_MAJOR");
-    if (s->geo > GEO_DOUBLE_CARTPOLE) return pddp_capi_fail(PDDP_E_UNSUPPORTED, "BNN kernels exist for the pendulum, cartpole and double-cartpole geometries (action_size 1)");
+    if (s->geo > GEO_RENDEZVOUS) return pddp_capi_fail(PDDP_E_UNSUPPORTED, "BNN kernels exist for the pendulum, cartpole, double-cartpole and rendezvous geometries");
     if (!n) return pddp_capi_fail(PDDP_E_BADARG, "bnn is NULL");
     if (n->P < 2 || n->P > 1024) return pddp_capi_fail(PDDP_E_BADARG, "2 <= particles <= 1024");
     if (n->H0 < 1 || n->H1 < 1 || n->H0 > 256 || n->H1 > 256) return pddp_capi_fail(PDDP_E_UNSUPPORTED, "hidden widths must be in [1,256]");

@@ -35,8 +35,8 @@ template <> bool use_tensor_cores<float>(int H0, int H1) {
 
 
 cudaError_t bnn_mlp_prep_images(int geo, const pddp_bnn* n, const tc::Images& im, cudaStream_t st) {
-    const int D = geo == GEO_PENDULUM ? 2 : geo == GEO_CARTPOLE ? 4 : 6;
-    const int DA = geo == GEO_PENDULUM ? 3 : geo == GEO_CARTPOLE ? 5 : 8;
+    const GeoDims g = geo_dims(geo);
+    const int D = g.D, K0 = g.DA + g.NU;
     struct { tc::Images im; } w = {im};
         // PDDP_MLP_COMPACT=0 keeps every hidden unit (A/B measurements; the images are then the same for all particles)
         static int compact = -1;
@@ -48,12 +48,12 @@ cudaError_t bnn_mlp_prep_images(int geo, const pddp_bnn* n, const tc::Images& im
                                                  const_cast<float*>(w.im.scale));
         tc::prep_w1_kernel<<<592, 256, 0, st>>>((const float*)n->W1, (const float*)n->b1, n->P, n->H0, n->H1, w.im.idx0, w.im.idx1,
                                                 meta, w.im.scale, const_cast<unsigned char*>(w.im.W1img));
-        if (DA + 2 <= 8)
+        if (K0 + 1 <= 8)
             tc::prep_w0_kernel<8><<<64, 256, 0, st>>>((const float*)n->W0, (const float*)n->b0, (const float*)n->mask0,
-                                                       n->P, n->H0, DA + 1, w.im.idx0, meta, const_cast<unsigned char*>(w.im.W0img));
+                                                       n->P, n->H0, K0, w.im.idx0, meta, const_cast<unsigned char*>(w.im.W0img));
         else
             tc::prep_w0_kernel<16><<<64, 256, 0, st>>>((const float*)n->W0, (const float*)n->b0, (const float*)n->mask0,
-                                                        n->P, n->H0, DA + 1, w.im.idx0, meta, const_cast<unsigned char*>(w.im.W0img));
+                                                        n->P, n->H0, K0, w.im.idx0, meta, const_cast<unsigned char*>(w.im.W0img));
         tc::prep_w2_kernel<<<64, 256, 0, st>>>((const float*)n->W2, (const float*)n->mask1, n->P, n->H1, D, D <= 4 ? 4 : 8,
                                                w.im.idx1, meta, w.im.scale, const_cast<float*>(w.im.W2p));
     return cudaGetLastError();
@@ -116,6 +116,8 @@ cudaError_t bnn_mlp_launch(int geo, bool tan, const BnnMlpArgs<T>& a, const tc::
         case GEO_CARTPOLE * 2 + 1: return launch_mlp<T, GEO_CARTPOLE, true>(a, im, st);
         case GEO_DOUBLE_CARTPOLE * 2: return launch_mlp<T, GEO_DOUBLE_CARTPOLE, false>(a, im, st);
         case GEO_DOUBLE_CARTPOLE * 2 + 1: return launch_mlp<T, GEO_DOUBLE_CARTPOLE, true>(a, im, st);
+        case GEO_RENDEZVOUS * 2: return launch_mlp<T, GEO_RENDEZVOUS, false>(a, im, st);
+        case GEO_RENDEZVOUS * 2 + 1: return launch_mlp<T, GEO_RENDEZVOUS, true>(a, im, st);
     }
     return cudaErrorInvalidValue;
 }

@@ -10,11 +10,22 @@ template <class T>
 struct BnnMlpArgs {
     BnnNet<T> net;
     const T* X;        // [S, P, D] particles in
-    const T* u;        // [S] action per particle group (nu == 1)
+    const T* u;        // [S, nu] action per particle group
     T* Xn;             // [S, P, D] particles out
     T* Jp;             // [S, P, D, D+nu] per-particle Jacobian (TAN only)
     long long total;   // S * P
 };
+
+// sizes of a BNN geometry for host code that dispatches on the runtime geometry id
+struct GeoDims { int D, NU, DA; };
+inline GeoDims geo_dims(int geo) {
+    switch (geo) {
+        case GEO_PENDULUM: return {Geo<GEO_PENDULUM>::D, Geo<GEO_PENDULUM>::NU, Geo<GEO_PENDULUM>::DA};
+        case GEO_CARTPOLE: return {Geo<GEO_CARTPOLE>::D, Geo<GEO_CARTPOLE>::NU, Geo<GEO_CARTPOLE>::DA};
+        case GEO_DOUBLE_CARTPOLE: return {Geo<GEO_DOUBLE_CARTPOLE>::D, Geo<GEO_DOUBLE_CARTPOLE>::NU, Geo<GEO_DOUBLE_CARTPOLE>::DA};
+        default: return {Geo<GEO_RENDEZVOUS>::D, Geo<GEO_RENDEZVOUS>::NU, Geo<GEO_RENDEZVOUS>::DA};
+    }
+}
 
 namespace tc {
 // sizes of the tcgen05 kernel's global images (bnn_mlp_tc.cuh has the layouts)

@@ -17,7 +17,7 @@ namespace pddp {
 
 
 constexpr int MLP_KC = 16;
-constexpr int MLP_KP = 16;   // padded layer-0 input width (K0 = DA + nu <= 9)
+constexpr int MLP_KP = 16;   // padded layer-0 input width (K0 = DA + nu <= 12)
 
 // PSTD: use_predicted_std=True -- the log-std head of the output layer (rows D..2D-1 of fc_out) is evaluated
 // too and exp(log_std) * eps_out[i] is added to every particle (ref: modules.py:242-262).
@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(256) bnn_mlp_simt_kernel(const BnnMlpArgs<T> a
         __syncthreads();
         if (tid < NPART && g0 + tid < a.total) {
             const long long g = g0 + tid;
-            const T u = a.u[g / P];
+            const T* u = a.u + (g / P) * G::NU;
             T x[D], in[K0], sc[K0];
 #pragma unroll
             for (int d = 0; d < D; ++d) { x[d] = a.X[g * D + d]; xs[tid * D + d] = x[d]; }
@@ -70,7 +70,8 @@ __global__ void __launch_bounds__(256) bnn_mlp_simt_kernel(const BnnMlpArgs<T> a
             for (int i = 0; i < NNA; ++i) in[i] = x[G::nonang(i)];
 #pragma unroll
             for (int i = 0; i < NANG; ++i) { in[NNA + 2 * i] = jsin(x[G::ang(i)]); in[NNA + 2 * i + 1] = jcos(x[G::ang(i)]); }
-            in[DA] = u;
+#pragma unroll
+            for (int j = 0; j < G::NU; ++j) in[DA + j] = u[j];
             T* r0 = A0 + (size_t)tid * RPP * MLP_KP;
 #pragma unroll
             for (int k = 0; k < K0; ++k) r0[k] = (in[k] - (n.X_mean ? n.X_mean[k] : T(0))) * sc[k];
@@ -82,7 +83,8 @@ __global__ void __launch_bounds__(256) bnn_mlp_simt_kernel(const BnnMlpArgs<T> a
                     r0[(1 + G::ang(i)) * MLP_KP + NNA + 2 * i] = in[NNA + 2 * i + 1] * sc[NNA + 2 * i];        // d sin = cos
                     r0[(1 + G::ang(i)) * MLP_KP + NNA + 2 * i + 1] = -in[NNA + 2 * i] * sc[NNA + 2 * i + 1];   // d cos = -sin
                 }
-                r0[(1 + D) * MLP_KP + DA] = sc[DA];
+#pragma unroll
+                for (int j = 0; j < G::NU; ++j) r0[(1 + D + j) * MLP_KP + DA + j] = sc[DA + j];
             }
         }
         __syncthreads();

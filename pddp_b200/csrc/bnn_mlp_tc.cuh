@@ -749,7 +749,8 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                     for (int i2 = 0; i2 < NNA; ++i2) inn[i2] = x[G::nonang(i2)];
 #pragma unroll
                     for (int i2 = 0; i2 < NANG; ++i2) { inn[NNA + 2 * i2] = sinf(x[G::ang(i2)]); inn[NNA + 2 * i2 + 1] = cosf(x[G::ang(i2)]); }
-                    inn[DA] = __ldg(a.u + i);
+#pragma unroll
+                    for (int j = 0; j < G::NU; ++j) inn[DA + j] = __ldg(a.u + (size_t)i * G::NU + j);
                 }
             };
             auto write_a0 = [&](int d) {       // [norm(aug(x), u), 1] (d == 0) or its tangent along direction d-1
@@ -773,7 +774,8 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                             row[NNA + 2 * i2] = inc[NNA + 2 * i2 + 1] * sc[NNA + 2 * i2];          // d sin = cos
                             row[NNA + 2 * i2 + 1] = -inc[NNA + 2 * i2] * sc[NNA + 2 * i2 + 1];     // d cos = -sin
                         }
-                        if (dir == D) row[DA] = sc[DA];
+#pragma unroll
+                        for (int j = 0; j < G::NU; ++j) if (dir == D + j) row[DA + j] = sc[DA + j];
                     }
                 }
                 uint32_t x0[K0P / 2], x1[K0P / 2];       // fp16 pairs: x0 = fp16(row), x1 = fp16(row - x0)

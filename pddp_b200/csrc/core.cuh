@@ -10,7 +10,7 @@ namespace pddp {
 
 // ---- enums shared with include/pddp_b200.h -------------------------------------------------
 enum { ENC_FULL = 0, ENC_UT = 1, ENC_VAR = 2, ENC_STD = 3, ENC_IGNORE = 4 };      // ref: utils/encoding.py:25-33
-enum { GEO_PENDULUM = 0, GEO_CARTPOLE = 1, GEO_DOUBLE_CARTPOLE = 2, GEO_RENDEZVOUS = 3 };   // 3: known_lq.cu
+enum { GEO_PENDULUM = 0, GEO_CARTPOLE = 1, GEO_DOUBLE_CARTPOLE = 2, GEO_RENDEZVOUS = 3 };
 enum { ST_UNDEFINED = 0, ST_ACCEPTED = 1, ST_REJECTED = 2, ST_NOT_PD = 3, ST_MAX_REG = 4,
        ST_CONVERGED = 5 };                                                       // ref: controllers/ilqr.py:35-64
 enum { LAYOUT_PROBLEM_MAJOR = 0, LAYOUT_BATCH_INNER = 1 };
@@ -34,6 +34,13 @@ template <> struct Geo<GEO_DOUBLE_CARTPOLE> {
     static constexpr int D = 6, NU = 1, NANG = 2, NNA = 4, DA = 8;
     PDDP_HD static constexpr int ang(int i) { return i == 0 ? 2 : 4; }
     PDDP_HD static constexpr int nonang(int i) { return i == 0 ? 0 : (i == 1 ? 1 : (i == 2 ? 3 : 5)); }
+};
+// two point masses in the plane (ref: examples/rendezvous/model.py): no angles, so the augmented state is the state.
+// The known-dynamics path (known_lq.cu) does not use this struct; the BNN path does, with the QR cost of rdv_cost.cuh.
+template <> struct Geo<GEO_RENDEZVOUS> {
+    static constexpr int D = 8, NU = 4, NANG = 0, NNA = 8, DA = 8;
+    PDDP_HD static constexpr int ang(int) { return 0; }      // (never called: NANG == 0)
+    PDDP_HD static constexpr int nonang(int i) { return i; }
 };
 
 PDDP_HD constexpr int enc_size(int D, int enc) {          // ref: utils/encoding.py:46-67
@@ -122,7 +129,7 @@ PDDP_HD void decode_var(const S* z, S (&V)[D]) {
 // dynamics of the same step (the rollout of the closed-form models is bound by instruction issue, and the three
 // separate sinf / cosf calls per pendulum step were a third of it)
 template <int GEO, class S>
-struct StateTrig { S s[Geo<GEO>::NANG], c[Geo<GEO>::NANG]; };
+struct StateTrig { S s[Geo<GEO>::NANG > 0 ? Geo<GEO>::NANG : 1], c[Geo<GEO>::NANG > 0 ? Geo<GEO>::NANG : 1]; };
 template <int GEO, class S>
 PDDP_HD void state_trig(const S* z, StateTrig<GEO, S>& tr) {
 #pragma unroll
@@ -135,7 +142,7 @@ PDDP_HD S cost_state(const CostParams<T>& cp, const S* z, bool terminal, const S
     constexpr int D = G::D, DA = G::DA, NNA = G::NNA, NANG = G::NANG;
     const T* Q = terminal ? cp.Qt : cp.Q;
     S Ma[DA];
-    S sn[NANG], cs[NANG];
+    S sn[NANG > 0 ? NANG : 1], cs[NANG > 0 ? NANG : 1];
     if (ENC == ENC_IGNORE) {                              // ref: utils/angular.py:251-286
 #pragma unroll
         for (int i = 0; i < NNA; ++i) Ma[i] = z[G::nonang(i)];

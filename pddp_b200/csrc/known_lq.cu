@@ -15,12 +15,13 @@
 // the encoded state (nz <= 72) lives in a per-thread array.
 #include "bnn_common.cuh"
 #include "kernels.h"
+#include "rdv_cost.cuh"
 
 namespace pddp {
 
 namespace {
 
-constexpr int RD = 8, RNU = 4;
+constexpr int RD = RDV_D, RNU = RDV_NU;
 
 template <class T>
 struct RdvModel { T dt, fr, gu, dvv, dvu; };   // acc = vel * fr + u * gu ; d vel'/d vel = dvv, d vel'/d u = dvu
@@ -85,54 +86,6 @@ __device__ __forceinline__ bool rdv_uncertainty_step(const T* z, T* zn, T (&U)[R
         return ok;
     }
     return true;
-}
-
-// state part of the QR cost: (m - xg)^T Q (m - xg) + sum_ij C_ij Q_ji   ref: costs/quadratic.py:80-97
-template <int ENC, class T>
-__device__ __forceinline__ T rdv_cost_state(const CostParams<T>& cp, const T* z, bool terminal) {
-    constexpr int D = RD;
-    const T* Q = terminal ? cp.Qt : cp.Q;
-    T val = T(0);
-#pragma unroll
-    for (int i = 0; i < D; ++i) {
-        T row = T(0);
-#pragma unroll
-        for (int j = 0; j < D; ++j) row += (z[j] - cp.xg[j]) * Q[j * D + i];
-        val += row * (z[i] - cp.xg[i]);
-    }
-    if (ENC == ENC_FULL) {
-#pragma unroll 1
-        for (int i = 0; i < D; ++i)
-            for (int j = 0; j < D; ++j) val += z[D + i * D + j] * Q[j * D + i];
-    } else if (ENC == ENC_UT) {
-        for (int i = 0; i < D; ++i)
-            for (int j = 0; j < D; ++j) {
-                T c = T(0);
-                const int m = i < j ? i : j;
-                for (int k = 0; k <= m; ++k) c += z[D + tri<D>(k, i)] * z[D + tri<D>(k, j)];
-                val += c * Q[j * D + i];
-            }
-    } else if (ENC == ENC_VAR) {
-#pragma unroll
-        for (int a = 0; a < D; ++a) val += z[D + a] * Q[a * D + a];
-    } else if (ENC == ENC_STD) {
-#pragma unroll
-        for (int a = 0; a < D; ++a) val += z[D + a] * z[D + a] * Q[a * D + a];
-    }
-    return val;
-}
-
-template <class T>
-__device__ __forceinline__ T rdv_cost_action(const CostParams<T>& cp, const T* u) {
-    T val = T(0);
-#pragma unroll
-    for (int i = 0; i < RNU; ++i) {
-        T row = T(0);
-#pragma unroll
-        for (int j = 0; j < RNU; ++j) row += (u[j] - cp.ug[j]) * cp.R[j * RNU + i];
-        val += row * (u[i] - cp.ug[i]);
-    }
-    return val;
 }
 
 // ------------------------------------------------------------------------------------------

@@ -196,24 +196,28 @@ def bnn_dynamics_model_factory(state_size, action_size, hidden_features, angular
         raise NotImplementedError("pddp_b200: bnn_dynamics_model_factory(constrain_min / constrain_max / particles) "
                                   "is not built (the reference squashes U through constrain() in forward and fit, "
                                   "modules.py:118-121,162,227; the kernels do not)")
-    if action_size != 1 or len(hidden_features) != 2:
-        raise NotImplementedError("pddp_b200: BNN kernels need action_size == 1 and two hidden layers")
+    if len(hidden_features) != 2:
+        raise NotImplementedError("pddp_b200: BNN kernels need two hidden layers")
     ang = [] if angular_indices is None else [int(i) for i in angular_indices]
     non = [i for i in range(state_size) if i not in ang]
     geo = geometry_of(state_size, ang)
+    nu = _lib.GEO_INFO[geo][1]
+    if action_size != nu:
+        raise NotImplementedError("pddp_b200: the BNN kernels of this state geometry (D=%d, angles %s) take action_size "
+                                  "%d; got %d" % (state_size, tuple(ang), nu, action_size))
     DA = infer_augmented_state_size(ang, non)
     _state_size, _ang = state_size, ang
 
     class BNNDynamicsModel(DynamicsModel):
         state_size = _state_size
-        action_size = 1
+        action_size = nu
         angular_indices = torch.tensor(_ang).long()
         non_angular_indices = torch.tensor(non).long()
         is_bnn = True
 
         def __init__(self, n_particles=100):
             super().__init__()
-            self.model = bayesian_model(DA + 1, 2 * _state_size, list(hidden_features), **kwargs)
+            self.model = bayesian_model(DA + nu, 2 * _state_size, list(hidden_features), **kwargs)
             self.n_particles = n_particles
             for n, v in (("X_mean", 0.0), ("X_std", 1.0), ("X_std_inv", 1.0), ("dX_mean", 0.0), ("dX_std", 1.0),
                          ("dX_std_inv", 1.0)):
@@ -317,11 +321,7 @@ def bnn_dynamics_model_factory(state_size, action_size, hidden_features, angular
             concrete = isinstance(drops[0], CDropout)
             if any(isinstance(d, CDropout) != concrete for d in drops):
                 raise NotImplementedError("pddp_b200: both dropout layers must be of the same kind")
-            cfg = TrainConfig(_lib.dtype_code(dtype), DA + 1, H0, H1, _state_size, Nd, bs, n_iter, 0 if concrete else 1,
-                              float(learning_rate), 0.9, 0.999, 1e-8, float(reg_scale),
-                              float(drops[0].temperature) if concrete else 0.0, float(drops[0].reg), float(drops[1].reg),
-                              float(drops[0].rate), float(drops[1].rate),
-                              int(torch.seed() if seed is None else seed) & ((1 << 63) - 1))
+            cfg = self.train_config(dtype, Nd, bs, n_iter, learning_rate, reg_scale, seed)
             lib = _lib.load()
             params = self.flat_parameters(dtype, dev).contiguous()
             grads = torch.zeros_like(params)
@@ -349,6 +349,17 @@ def bnn_dynamics_model_factory(state_size, action_size, hidden_features, angular
             if return_diagnostics:
                 return loss, grads
             return None
+
+        def train_config(self, dtype, n_data, batch, n_iter, learning_rate, reg_scale, seed=None):
+            """The pddp_bnn_train configuration of fit(): input width K0 = augmented state + action."""
+            drops = self._dropouts()
+            concrete = isinstance(drops[0], CDropout)
+            H0, H1 = self.model.fc_0.out_features, self.model.fc_1.out_features
+            return TrainConfig(_lib.dtype_code(dtype), DA + nu, H0, H1, _state_size, n_data, batch, n_iter,
+                               0 if concrete else 1, float(learning_rate), 0.9, 0.999, 1e-8, float(reg_scale),
+                               float(drops[0].temperature) if concrete else 0.0, float(drops[0].reg),
+                               float(drops[1].reg), float(drops[0].rate), float(drops[1].rate),
+                               int(torch.seed() if seed is None else seed) & ((1 << 63) - 1))
 
         # ------------------------------------------------------------------ what the kernels read
         def descriptor(self, model_opts=None, N=None):
