@@ -18,7 +18,7 @@
 //     accumulation: fp32-class accuracy from three FP16 passes and 4 operand bytes per element;
 //   * tangents are pass-major: a super-tile is the primal pass followed by one pass per direction
 //     over the same 128 items, so a thread meets the primal and the tangent pre-activation of the
-//     same (item, hidden unit) and the ReLU gate is a register bit mask, never a shuffle;
+//     same (item, hidden unit) and the ReLU gate is a per-thread bit mask, never a shuffle;
 //   * two independent tile "tracks" per CTA consume the same streamed W1 K-block (16 wide,
 //     SWIZZLE_64B rows of [b0 | b1]): half the L2->smem traffic per row.  Track 1 runs half a tile behind track 0,
 //     and each track has its own layer-1 issuer thread, so one track's epilogue is covered by the
@@ -159,6 +159,14 @@ __device__ __forceinline__ void sts128(uint32_t addr, uint32_t x, uint32_t y, ui
 __device__ __forceinline__ void sts128f(uint32_t addr, float x, float y, float z, float w) {
     sts128(addr, __float_as_uint(x), __float_as_uint(y), __float_as_uint(z), __float_as_uint(w));
 }
+__device__ __forceinline__ void sts32(uint32_t addr, uint32_t x) {
+    asm volatile("st.shared.b32 [%0], %1;" ::"r"(addr), "r"(x) : "memory");
+}
+__device__ __forceinline__ uint32_t lds32(uint32_t addr) {
+    uint32_t x;
+    asm volatile("ld.shared.b32 %0, [%1];" : "=r"(x) : "r"(addr));
+    return x;
+}
 __device__ __forceinline__ float4 lds128f(uint32_t addr) {
     float4 v;
     asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
@@ -283,7 +291,8 @@ struct Cfg {
     static constexpr int W2_OFF = W0_OFF + 2 * W0_SMEM;
     static constexpr int BAR_OFF = W2_OFF + 2 * W2_BYTES;
     static constexpr int NBARS = 2 * NB + 4 * NS + 14;
-    static constexpr int TOTAL = BAR_OFF + NBARS * 8 + 16;
+    static constexpr int GATE_OFF = BAR_OFF + NBARS * 8 + 16;    // epilogue gate words (TAN): [track][trip][row]
+    static constexpr int TOTAL = GATE_OFF + 2 * MAX_NCH * TILE_M * 4;
     static constexpr int ALIGN_PAD = 512;
 };
 
@@ -469,6 +478,17 @@ struct TrackIter {
         if (tau >= seg_end) locate(seg_end, T1, tiles_p, t, meta);
     }
 };
+
+// What the epilogue's column loop does to one layer-1 pre-activation v, element e of a gate word of NE bits:
+// EPI_RELU (rollout) and EPI_PRIMAL (first pass of a linearisation super-tile) apply the ReLU, EPI_PRIMAL also shifts the
+// sign of v into the word (element e ends at bit NE-1-e); EPI_TANGENT zeroes v where the primal's sign bit is set.
+enum { EPI_RELU, EPI_PRIMAL, EPI_TANGENT };
+template <int KIND, int NE>
+__device__ __forceinline__ float epi_act(float v, uint32_t& word, int e) {
+    if constexpr (KIND == EPI_PRIMAL) word = __funnelshift_l(__float_as_uint(v), word, 1);
+    if constexpr (KIND == EPI_TANGENT) return (word & (1u << (NE - 1 - e))) ? 0.f : v;
+    else return fmaxf(v, 0.f);
+}
 
 template <int GEO, bool TAN>
 __global__ void __launch_bounds__(THREADS, 1)
@@ -930,9 +950,8 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
             const int q4 = lane & 3, rq = lane >> 2;
             int curp = -1;
             uint32_t w2loads = 0;
-            uint32_t gate[7];                  // sign bits of this thread's (up to 208) primal pre-activations (TAN)
-#pragma unroll
-            for (int j = 0; j < 7; ++j) gate[j] = 0;
+            // sign bits of this thread's (up to 208) primal pre-activations (TAN), one word per 32-column trip
+            const uint32_t gate_s = smem_u32(smem + C::GATE_OFF) + (uint32_t)(t * MAX_NCH * TILE_M + r) * 4u;
             int d = 0;
             for (int k = 0; cur.valid(); ++k) {   // k = tiles of this track so far (accumulator phase)
 #ifdef PDDP_EXP_EPI_SHORT            // timing experiment only (wrong results): the epilogue drains 16 columns
@@ -981,9 +1000,9 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
 #endif
                 tc_fence_after();
                 // half = 16 columns (two 8-column groups) of both row halves; consumes fragment buffer fb and
-                // shifts / tests bits [ebase, ebase+16) of the current gate word
-                auto half = [&](const int c0, float (&fb)[2][8], uint32_t& word, auto ebase_tag, auto ne_tag) {
-                    constexpr int EBASE = decltype(ebase_tag)::value, NE = decltype(ne_tag)::value;
+                // shifts (EPI_PRIMAL) / tests (EPI_TANGENT) bits [ebase, ebase+16) of the current gate word
+                auto half = [&](const int c0, float (&fb)[2][8], uint32_t& word, auto kind_tag, auto ebase_tag, auto ne_tag) {
+                    constexpr int KIND = decltype(kind_tag)::value, EBASE = decltype(ebase_tag)::value, NE = decltype(ne_tag)::value;
                     if constexpr (PK) {
 #pragma unroll
                         for (int gi = 0; gi < 2; ++gi) {
@@ -1005,16 +1024,7 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                                     float vv[2];
 #pragma unroll
                                     for (int cc = 0; cc < 2; ++cc) {
-                                        vv[cc] = fb[hf][4 * gi + 2 * hb + cc];
-                                        const int e = EBASE + (gi * 2 + hf) * 4 + 2 * hb + cc;
-                                        if (!TAN) {
-                                            vv[cc] = fmaxf(vv[cc], 0.f);
-                                        } else if (d == 0) {
-                                            word = __funnelshift_l(__float_as_uint(vv[cc]), word, 1);   // element e ends at bit NE-1-e
-                                            vv[cc] = fmaxf(vv[cc], 0.f);
-                                        } else {
-                                            vv[cc] = (word & (1u << (NE - 1 - e))) ? 0.f : vv[cc];
-                                        }
+                                        vv[cc] = epi_act<KIND, NE>(fb[hf][4 * gi + 2 * hb + cc], word, EBASE + (gi * 2 + hf) * 4 + 2 * hb + cc);
                                     }
                                     const unsigned long long vp = pack2(vv[0], vv[1]);
 #pragma unroll
@@ -1037,16 +1047,7 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                                 for (int hb = 0; hb < 2; ++hb)
 #pragma unroll
                                     for (int cc = 0; cc < 2; ++cc) {
-                                        float vv = fb[hf][4 * gi + 2 * hb + cc];
-                                        const int e = EBASE + (gi * 2 + hf) * 4 + 2 * hb + cc;
-                                        if (!TAN) {
-                                            vv = fmaxf(vv, 0.f);
-                                        } else if (d == 0) {
-                                            word = __funnelshift_l(__float_as_uint(vv), word, 1);   // element e ends at bit NE-1-e
-                                            vv = fmaxf(vv, 0.f);
-                                        } else {
-                                            vv = (word & (1u << (NE - 1 - e))) ? 0.f : vv;
-                                        }
+                                        const float vv = epi_act<KIND, NE>(fb[hf][4 * gi + 2 * hb + cc], word, EBASE + (gi * 2 + hf) * 4 + 2 * hb + cc);
 #pragma unroll
                                         for (int o = 0; o < D; ++o) y[2 * hf + hb][o] += vv * w2[cc][o];
                                     }
@@ -1058,43 +1059,46 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                     tc_ld_16x256b_x2(ta, fb[0]);
                     tc_ld_16x256b_x2(ta + (16u << 16), fb[1]);
                 };
-                // gate word of 32-column trip j: written by the primal pass, read by the tangent passes (register
-                // selects: the trip count depends on the particle, so the words cannot sit in a rotating queue)
-                auto gate_put = [&](int j, uint32_t word) {
-#pragma unroll
-                    for (int jj = 0; jj < 7; ++jj) if (jj == j) gate[jj] = word;
-                };
-                auto gate_get = [&](int j) -> uint32_t {
-                    uint32_t word = 0;
-#pragma unroll
-                    for (int jj = 0; jj < 7; ++jj) if (jj == j) word = gate[jj];
-                    return word;
-                };
+                // gate word of 32-column trip j: written by the primal pass, read by the tangent passes.  In shared
+                // memory, not registers: the epilogue runs at the register cap, and a register array indexed by the
+                // trip costs a 7-way select per trip.
+                auto gate_put = [&](int j, uint32_t word) { sts32(gate_s + (uint32_t)(j * TILE_M * 4), word); };
+                auto gate_get = [&](int j) -> uint32_t { return lds32(gate_s + (uint32_t)(j * TILE_M * 4)); };
                 // ncol / 16 sixteen-column batches, two per trip of a ROLLED loop (a fully unrolled epilogue is 1 400 SASS
                 // instructions: with five roles resident, instruction-cache misses were 26 % of its stall samples),
                 // software pipelined over two fragment buffers: the TMEM loads of the next batch are issued right
                 // after the wait for the current one (tcgen05.wait::ld waits for everything outstanding).
+                // The pass kind is chosen once per tile: each kind has its own copy of the loop, carrying only its own
+                // per-element work (a runtime kind inside the loop costs every element the work of all kinds).
+                // (The fragment buffers live outside the lambda: declared inside it, they change how nvcc schedules the
+                // rollout instantiation, whose code this split leaves as it was.)
                 float fa[2][8], fb2[2][8];
                 const int cfull = ncol & ~31;               // columns covered by whole 32-column trips
-                issue(0, fa);
-                int j = 0;
+                auto columns = [&](auto kind_tag) {
+                    constexpr int KIND = decltype(kind_tag)::value;
+                    issue(0, fa);
+                    int j = 0;
 #pragma unroll 1
-                for (int c0 = 0; c0 < cfull; c0 += 32, ++j) {
-                    uint32_t word = (TAN && d != 0) ? gate_get(j) : 0u;
-                    tc_wait_ld8(fa[0]); tc_wait_ld8(fa[1]);
-                    issue(c0 + 16, fb2);
-                    half(c0, fa, word, std::integral_constant<int, 0>(), std::integral_constant<int, 32>());
-                    tc_wait_ld8(fb2[0]); tc_wait_ld8(fb2[1]);
-                    if (c0 + 32 < ncol) issue(c0 + 32, fa);
-                    half(c0 + 16, fb2, word, std::integral_constant<int, 16>(), std::integral_constant<int, 32>());
-                    if (TAN && d == 0) gate_put(j, word);
-                }
-                if (cfull < ncol) {                          // one more 16-column batch
-                    uint32_t word = (TAN && d != 0) ? gate_get(j) : 0u;
-                    tc_wait_ld8(fa[0]); tc_wait_ld8(fa[1]);
-                    half(cfull, fa, word, std::integral_constant<int, 0>(), std::integral_constant<int, 16>());
-                    if (TAN && d == 0) gate_put(j, word);
-                }
+                    for (int c0 = 0; c0 < cfull; c0 += 32, ++j) {
+                        uint32_t word = KIND == EPI_TANGENT ? gate_get(j) : 0u;
+                        tc_wait_ld8(fa[0]); tc_wait_ld8(fa[1]);
+                        issue(c0 + 16, fb2);
+                        half(c0, fa, word, kind_tag, std::integral_constant<int, 0>(), std::integral_constant<int, 32>());
+                        tc_wait_ld8(fb2[0]); tc_wait_ld8(fb2[1]);
+                        if (c0 + 32 < ncol) issue(c0 + 32, fa);
+                        half(c0 + 16, fb2, word, kind_tag, std::integral_constant<int, 16>(), std::integral_constant<int, 32>());
+                        if (KIND == EPI_PRIMAL) gate_put(j, word);
+                    }
+                    if (cfull < ncol) {                      // one more 16-column batch
+                        uint32_t word = KIND == EPI_TANGENT ? gate_get(j) : 0u;
+                        tc_wait_ld8(fa[0]); tc_wait_ld8(fa[1]);
+                        half(cfull, fa, word, kind_tag, std::integral_constant<int, 0>(), std::integral_constant<int, 16>());
+                        if (KIND == EPI_PRIMAL) gate_put(j, word);
+                    }
+                };
+                if constexpr (!TAN) columns(std::integral_constant<int, EPI_RELU>());
+                else if (d == 0) columns(std::integral_constant<int, EPI_PRIMAL>());
+                else columns(std::integral_constant<int, EPI_TANGENT>());
                 tc_fence_before();
                 mbar_arrive(&acc1_empty[t]);
 #ifdef PDDP_EXP_TRACE
