@@ -15,15 +15,14 @@
 // Roofline: HBM -- per trajectory-step 2nz^2+2nz*nu+nz+nu+nu^2 elements read, nu+nu*nz written.
 #include "core.cuh"
 #include "kernels.h"
-#include <stdlib.h>
 
 namespace pddp {
 
 constexpr int MNU = MAX_NU;
 
-// TEAM threads own one problem: a whole CTA (256), a warp (32), or a SUB-WARP team of 4 / 8 / 16 lanes -- several
+// TEAM threads own one problem: a whole CTA (256), a warp (32), or a SUB-WARP team of 4 / 8 lanes -- several
 // problems per warp, so the team-uniform scalar algebra (Jacobi sweeps, box-QP Newton iterations) that every lane
-// executes redundantly is paid once per 8 / 4 / 2 problems instead of once per problem, and with the
+// executes redundantly is paid once per 8 / 4 problems instead of once per problem, and with the
 // BATCH_INNER layout the lanes that hold the same element of consecutive problems read full 32-byte sectors.
 template <int TEAM>
 __device__ __forceinline__ unsigned nu_team_mask() {
@@ -345,15 +344,15 @@ __host__ __device__ inline int backward_nu_stride(int nz, int nu, int team) {
 // NZC / NUC > 0: state / action sizes known at compile time (the loops unroll and the index divisions become shifts:
 // with run-time sizes the matrix phases of the rendezvous problem were 9.6 k instructions per warp and time step).
 //
-// HO (hand-off, sub-warp teams only): the small dense part is data dependent (Jacobi sweeps, box-QP iterations) and
-// team-uniform, so a warp of 32 / TEAM teams paid the union of its problems' paths once per 32 / TEAM problems: for
-// the rendezvous shape 6.8 k of the 10 k instructions per warp and time step.  With HO every team parks Q_uu / Q_u in
-// its shared-memory region and ONE warp of the CTA solves all of the CTA's problems, a problem per lane (the warm
+// HO (hand-off, sub-warp teams): the small dense part is data dependent (Jacobi sweeps, box-QP iterations) and
+// team-uniform, so a warp of 32 / TEAM teams would pay the union of its problems' paths once per 32 / TEAM problems:
+// for the rendezvous shape 6.8 k of the 10 k instructions per warp and time step.  Instead every team parks Q_uu / Q_u
+// in its shared-memory region and ONE warp of the CTA solves all of the CTA's problems, a problem per lane (the warm
 // start k[t+1] stays in that lane's registers); the other warps wait at the CTA barrier (other CTAs of the SM run
 // their matrix phases meanwhile).  Teams without work (b >= B, inactive, failed) keep taking part in the barriers.
-template <class T, int TEAM, int NZC = 0, int NUC = 0, bool HO = false>
-__global__ void __launch_bounds__(TEAM <= 32 ? 128 : TEAM, (HO && sizeof(T) == 4) ? 4 : 1) backward_nu_kernel(const BackwardArgs<T> a) {
-    static_assert(!HO || TEAM < 32, "hand-off is for sub-warp teams");
+template <class T, int TEAM, int NZC = 0, int NUC = 0>
+__global__ void __launch_bounds__(TEAM <= 32 ? 128 : TEAM, (TEAM < 32 && sizeof(T) == 4) ? 4 : 1) backward_nu_kernel(const BackwardArgs<T> a) {
+    constexpr bool HO = TEAM < 32;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x % TEAM, warp = threadIdx.x / TEAM, wpb = blockDim.x / TEAM;
     const int b = blockIdx.x * wpb + warp;
@@ -586,16 +585,12 @@ __global__ void __launch_bounds__(TEAM <= 32 ? 128 : TEAM, (HO && sizeof(T) == 4
 }
 
 template <class T, int TEAM, int NZC = 0, int NUC = 0>
-static cudaError_t launch_nu_teams(const BackwardArgs<T>& a, size_t, cudaStream_t s) {
+static cudaError_t launch_nu_teams(const BackwardArgs<T>& a, cudaStream_t s) {
     const size_t per_team = (size_t)backward_nu_stride(a.nz, a.nu, TEAM) * sizeof(T);
     int tpb = 128 / TEAM;                                   // teams (problems) per CTA
     while (tpb > 1 && per_team * tpb > 200 * 1024) tpb >>= 1;
     const size_t smem = per_team * tpb;
-    // PDDP_BACKWARD_NU_HANDOFF=0: every team solves its own small dense part (A/B measurements)
-    static int handoff = -1;
-    if (handoff < 0) { const char* e = getenv("PDDP_BACKWARD_NU_HANDOFF"); handoff = (e && e[0] == '0') ? 0 : 1; }
-    auto kern = backward_nu_kernel<T, TEAM, NZC, NUC, false>;
-    if constexpr (TEAM < 32) { if (handoff) kern = backward_nu_kernel<T, TEAM, NZC, NUC, true>; }
+    auto kern = backward_nu_kernel<T, TEAM, NZC, NUC>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kern<<<(a.B + tpb - 1) / tpb, tpb * TEAM, smem, s>>>(a);
@@ -613,16 +608,11 @@ cudaError_t backward_pass_nu(const BackwardArgs<T>& a, cudaStream_t s) {
         backward_nu_kernel<T, 256><<<a.B, 256, per_team, s>>>(a);
         return cudaGetLastError();
     }
-    // small states: sub-warp teams (nz <= 8: 4 lanes, 8 problems per warp; nz <= 12: 8 lanes).  PDDP_BACKWARD_NU_TEAM
-    // overrides the choice (A/B measurements).
-    static int forced_team = -1;
-    if (forced_team < 0) { const char* e = getenv("PDDP_BACKWARD_NU_TEAM"); forced_team = e ? atoi(e) : 0; }
-    const int team = forced_team ? forced_team : a.nz <= 8 ? 4 : a.nz <= 12 ? 8 : 32;
-    if (team == 4 && a.nz == 8 && a.nu == 4) return launch_nu_teams<T, 4, 8, 4>(a, per_team, s);    // rendezvous, IGNORE_UNCERTAINTY
-    if (team == 4) return launch_nu_teams<T, 4>(a, per_team, s);
-    if (team == 8) return launch_nu_teams<T, 8>(a, per_team, s);
-    if (team == 16) return launch_nu_teams<T, 16>(a, per_team, s);
-    return launch_nu_teams<T, 32>(a, per_team, s);
+    // small states: sub-warp teams (nz <= 8: 4 lanes, 8 problems per warp; nz <= 12: 8 lanes), else a warp per problem
+    if (a.nz == 8 && a.nu == 4) return launch_nu_teams<T, 4, 8, 4>(a, s);    // rendezvous, IGNORE_UNCERTAINTY
+    if (a.nz <= 8) return launch_nu_teams<T, 4>(a, s);
+    if (a.nz <= 12) return launch_nu_teams<T, 8>(a, s);
+    return launch_nu_teams<T, 32>(a, s);
 }
 template cudaError_t backward_pass_nu<float>(const BackwardArgs<float>&, cudaStream_t);
 template cudaError_t backward_pass_nu<double>(const BackwardArgs<double>&, cudaStream_t);

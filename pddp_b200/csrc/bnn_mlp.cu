@@ -37,25 +37,21 @@ template <> bool use_tensor_cores<float>(int H0, int H1) {
 cudaError_t bnn_mlp_prep_images(int geo, const pddp_bnn* n, const tc::Images& im, cudaStream_t st) {
     const GeoDims g = geo_dims(geo);
     const int D = g.D, K0 = g.DA + g.NU;
-    struct { tc::Images im; } w = {im};
-        // PDDP_MLP_COMPACT=0 keeps every hidden unit (A/B measurements; the images are then the same for all particles)
-        static int compact = -1;
-        if (compact < 0) { const char* e = getenv("PDDP_MLP_COMPACT"); compact = (e && e[0] == '0') ? 0 : 1; }
-        int* meta = const_cast<int*>(w.im.meta);
-        tc::prep_index_kernel<<<(n->P + 63) / 64, 64, 0, st>>>((const float*)n->mask0, (const float*)n->mask1, n->P, n->H0, n->H1,
-                                                               compact, w.im.idx0, w.im.idx1, meta);
-        tc::prep_scale_kernel<<<1, 256, 0, st>>>((const float*)n->W1, (const float*)n->b1, n->H0, n->H1,
-                                                 const_cast<float*>(w.im.scale));
-        tc::prep_w1_kernel<<<592, 256, 0, st>>>((const float*)n->W1, (const float*)n->b1, n->P, n->H0, n->H1, w.im.idx0, w.im.idx1,
-                                                meta, w.im.scale, const_cast<unsigned char*>(w.im.W1img));
-        if (K0 + 1 <= 8)
-            tc::prep_w0_kernel<8><<<64, 256, 0, st>>>((const float*)n->W0, (const float*)n->b0, (const float*)n->mask0,
-                                                       n->P, n->H0, K0, w.im.idx0, meta, const_cast<unsigned char*>(w.im.W0img));
-        else
-            tc::prep_w0_kernel<16><<<64, 256, 0, st>>>((const float*)n->W0, (const float*)n->b0, (const float*)n->mask0,
-                                                        n->P, n->H0, K0, w.im.idx0, meta, const_cast<unsigned char*>(w.im.W0img));
-        tc::prep_w2_kernel<<<64, 256, 0, st>>>((const float*)n->W2, (const float*)n->mask1, n->P, n->H1, D, D <= 4 ? 4 : 8,
-                                               w.im.idx1, meta, w.im.scale, const_cast<float*>(w.im.W2p));
+    int* meta = const_cast<int*>(im.meta);
+    tc::prep_index_kernel<<<(n->P + 63) / 64, 64, 0, st>>>((const float*)n->mask0, (const float*)n->mask1, n->P, n->H0, n->H1,
+                                                           im.idx0, im.idx1, meta);
+    tc::prep_scale_kernel<<<1, 256, 0, st>>>((const float*)n->W1, (const float*)n->b1, n->H0, n->H1,
+                                             const_cast<float*>(im.scale));
+    tc::prep_w1_kernel<<<592, 256, 0, st>>>((const float*)n->W1, (const float*)n->b1, n->P, n->H0, n->H1, im.idx0, im.idx1,
+                                            meta, im.scale, const_cast<unsigned char*>(im.W1img));
+    if (K0 + 1 <= 8)
+        tc::prep_w0_kernel<8><<<64, 256, 0, st>>>((const float*)n->W0, (const float*)n->b0, (const float*)n->mask0,
+                                                   n->P, n->H0, K0, im.idx0, meta, const_cast<unsigned char*>(im.W0img));
+    else
+        tc::prep_w0_kernel<16><<<64, 256, 0, st>>>((const float*)n->W0, (const float*)n->b0, (const float*)n->mask0,
+                                                    n->P, n->H0, K0, im.idx0, meta, const_cast<unsigned char*>(im.W0img));
+    tc::prep_w2_kernel<<<64, 256, 0, st>>>((const float*)n->W2, (const float*)n->mask1, n->P, n->H1, D, D <= 4 ? 4 : 8,
+                                           im.idx1, meta, im.scale, const_cast<float*>(im.W2p));
     return cudaGetLastError();
 }
 

@@ -48,6 +48,8 @@ namespace tc {
 
 #ifdef PDDP_EXP_TRACE
 // Timeline experiment: CTA 0 records clock64() stamps per role (regions of 8192 entries) for the LAST launch.
+// Without PDDP_EXP_TRACE, TCLK() is a constant 0 and TR() is empty, so the stamps and per-tile sums in the role
+// loops compile to nothing.
 __device__ long long g_trace[8 * 8192];
 #define TR_ON (blockIdx.x == 0)
 #define TR(region, idx, val) do { if (TR_ON && (idx) < 8192) g_trace[(region) * 8192 + (idx)] = (val); } while (0)
@@ -71,11 +73,7 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
 // try_wait with a suspend-time hint: the thread sleeps in hardware until the phase completes or the
 // hint expires.  Without a hint the default window is ~50 cycles: the waiting roles re-polled 60 M
 // times per launch, and the kernel runs into the board's power cap.
-#ifdef PDDP_EXP_SUSPEND_NS
-constexpr uint32_t MBAR_SUSPEND_NS = PDDP_EXP_SUSPEND_NS;
-#else
 constexpr uint32_t MBAR_SUSPEND_NS = 20000;
-#endif
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
@@ -107,11 +105,6 @@ constexpr int TILE_M = 128, TILE_N = 208, KB = 16, MAX_NKB = 13, MAX_NCH = 7, N0
 // parts stay normal); the scale is undone inside the per-particle output weights.  Hidden
 // activations must stay below 65504 (they are O(1) for any network that rolls out finitely).
 constexpr int B_STAGE = TILE_N * 64;   // W1 K-block: 208 rows x [b0 (16 fp16) | b1 (16 fp16)], 13 312 B
-#ifdef PDDP_EXP_BSTAGE
-constexpr int B_SSTAGE = PDDP_EXP_BSTAGE;   // (timing experiment) shared-memory stride of a W1 stage
-#else
-constexpr int B_SSTAGE = B_STAGE;
-#endif
 constexpr int A1_SLOT = TILE_M * 64;   // 128 rows x [a0 (16 fp16) | a1 (16 fp16)], 8 192 B
 constexpr int THREADS = 20 * 32;
 constexpr int TM_ACC1 = 0, TM_ACC0 = 208, TM_TRACK = 256;
@@ -269,26 +262,17 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
 
 template <int K0P, int DP>
 struct Cfg {
-#if defined(PDDP_EXP_NB) && defined(PDDP_EXP_NS)
-    static constexpr int NB = PDDP_EXP_NB, NS = PDDP_EXP_NS;
-#else
     static constexpr int NB = K0P == 8 ? 5 : 4;    // W1 K-block stages
     static constexpr int NS = K0P == 8 ? 6 : 4;    // layer-1 A-operand slots per track
-#endif
     static constexpr int ROWB0 = K0P * 4;          // layer-0 operand row [x0 (K0P fp16) | x1 (K0P fp16)]: SWIZZLE_32B / 64B
     static constexpr int A0_BYTES = TILE_M * ROWB0;
     static constexpr int W0_CHUNK_PART = N0 * ROWB0, W0_CHUNK = 2 * W0_CHUNK_PART, W0_BYTES = MAX_NCH * W0_CHUNK;
-#ifdef PDDP_EXP_W0CH
-    static constexpr int W0_SMEM = PDDP_EXP_W0CH * W0_CHUNK;     // (experiment) chunks resident in shared memory
-#else
-    static constexpr int W0_SMEM = W0_BYTES;
-#endif
     static constexpr int W2_BYTES = TILE_N * DP * 4;
     static constexpr int B_OFF = 0;
-    static constexpr int A1_OFF = B_OFF + NB * B_SSTAGE;
+    static constexpr int A1_OFF = B_OFF + NB * B_STAGE;
     static constexpr int A0_OFF = A1_OFF + 2 * NS * A1_SLOT;
     static constexpr int W0_OFF = A0_OFF + 2 * A0_BYTES;
-    static constexpr int W2_OFF = W0_OFF + 2 * W0_SMEM;
+    static constexpr int W2_OFF = W0_OFF + 2 * W0_BYTES;
     static constexpr int BAR_OFF = W2_OFF + 2 * W2_BYTES;
     static constexpr int NBARS = 2 * NB + 4 * NS + 14;
     static constexpr int GATE_OFF = BAR_OFF + NBARS * 8 + 16;    // epilogue gate words (TAN): [track][trip][row]
@@ -326,14 +310,14 @@ constexpr float DROP_BELOW = 5.9604645e-8f;    // 2^-24
 constexpr int META = 4;
 static_assert(META == IMG_META, "bnn_mlp_iface.h sizes");
 __global__ void prep_index_kernel(const float* mask0 /*[P][H0]*/, const float* mask1 /*[P][H1]*/, int P, int H0, int H1,
-                                  int compact, int* idx0 /*[P][TILE_N]*/, int* idx1 /*[P][TILE_N]*/, int* meta /*[P][META]*/) {
+                                  int* idx0 /*[P][TILE_N]*/, int* idx1 /*[P][TILE_N]*/, int* meta /*[P][META]*/) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P) return;
     int n0 = 0, n1 = 0;
     for (int n = 0; n < H0; ++n)
-        if (!compact || !(mask0[(size_t)p * H0 + n] < DROP_BELOW)) idx0[(size_t)p * TILE_N + n0++] = n;
+        if (!(mask0[(size_t)p * H0 + n] < DROP_BELOW)) idx0[(size_t)p * TILE_N + n0++] = n;
     for (int c = 0; c < H1; ++c)
-        if (!compact || !(mask1[(size_t)p * H1 + c] < DROP_BELOW)) idx1[(size_t)p * TILE_N + n1++] = c;
+        if (!(mask1[(size_t)p * H1 + c] < DROP_BELOW)) idx1[(size_t)p * TILE_N + n1++] = c;
     const int ncol = (n1 + 15) & ~15;
     meta[p * META + 0] = (n0 + 1 + KB - 1) / KB;
     meta[p * META + 1] = ncol < 16 ? 16 : ncol;
@@ -427,6 +411,9 @@ __global__ void prep_w2_kernel(const float* W2 /*[2D][H1]*/, const float* mask1 
 struct Seg {
     int ta, cnt, p, nkb, ncol, skew, n[2], len;
 };
+// K-blocks by which track 1 trails track 0 in the W1 stream of a particle with nkb K-blocks: about half a tile, and
+// even, because a layer-0 chunk (32 hidden units) is two K-blocks and the tracks walk them from chunk boundaries
+__device__ __forceinline__ int track_skew(int nkb) { return (nkb / 2) & ~1; }
 __device__ __forceinline__ bool seg_at(int ta, int T1, int tiles_p, const int* meta, int rpp, Seg& s) {
     if (ta >= T1) return false;
     s.ta = ta;
@@ -435,11 +422,7 @@ __device__ __forceinline__ bool seg_at(int ta, int T1, int tiles_p, const int* m
     s.cnt = end - ta;
     s.nkb = __ldg(meta + s.p * META);
     s.ncol = __ldg(meta + s.p * META + 1);
-    #ifdef PDDP_EXP_SKEW
-    s.skew = PDDP_EXP_SKEW;
-#else
-    s.skew = (s.nkb / 2) & ~1;
-#endif
+    s.skew = track_skew(s.nkb);
     s.n[0] = ((s.cnt + 1) / 2) * rpp;
     s.n[1] = (s.cnt / 2) * rpp;
     const int len0 = s.n[0] * s.nkb, len1 = s.n[1] ? s.skew + s.n[1] * s.nkb : 0;
@@ -454,11 +437,7 @@ struct TrackIter {
     __device__ __forceinline__ bool valid() const { return tau >= 0; }
     __device__ __forceinline__ int nkb() const { return kn & 255; }
     __device__ __forceinline__ int ncol() const { return kn >> 8; }
-    #ifdef PDDP_EXP_SKEW
-    __device__ __forceinline__ int skew() const { return PDDP_EXP_SKEW; }
-#else
-    __device__ __forceinline__ int skew() const { return (nkb() / 2) & ~1; }
-#endif
+    __device__ __forceinline__ int skew() const { return track_skew(nkb()); }
     __device__ __forceinline__ int p(int tiles_p) const { return tau / tiles_p; }
     __device__ __forceinline__ void locate(int seg_start, int T1, int tiles_p, int t, const int* meta) {
         tau = -1;
@@ -571,7 +550,7 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                 for (int nb = 0; nb < sg.len; ++nb) {
                     mbar_wait(&b_empty[s], ph);
                     mbar_expect_tx(&b_full[s], bytes);
-                    bulk_g2s(smem + C::B_OFF + s * B_SSTAGE, img + (size_t)kb * B_STAGE, bytes, &b_full[s]);
+                    bulk_g2s(smem + C::B_OFF + s * B_STAGE, img + (size_t)kb * B_STAGE, bytes, &b_full[s]);
                     if (++s == NB) { s = 0; ph ^= 1; }
                     if (++kb == sg.nkb) kb = 0;
                 }
@@ -612,7 +591,7 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                     const int nk = kb + 1 < nkb ? 2 : 1, j = kb >> 1;
                     const uint32_t d_tmem = tmem_base + (uint32_t)(t * TM_TRACK + TM_ACC0);
                     const uint32_t a0 = smem_u32(smem + C::A0_OFF + t * C::A0_BYTES);
-                    const uint32_t b0 = smem_u32(smem + C::W0_OFF + t * C::W0_SMEM + j * C::W0_CHUNK);
+                    const uint32_t b0 = smem_u32(smem + C::W0_OFF + t * C::W0_BYTES + j * C::W0_CHUNK);
                     const uint64_t ad = make_desc<ROWB0>(a0);
                     const uint64_t bx = make_desc<ROWB0>(b0), by = make_desc<ROWB0>(b0 + C::W0_CHUNK_PART);
                     // one K-step = 32 B of a row = 16 fp16: K0P = 8 -> [a0 | a1] in one step; K0P = 16 -> a0, then a1
@@ -647,86 +626,50 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
             uint64_t* const a1e = a1_empty + t * NS;
             uint32_t s = 0, bph = 0, slot = 0, sph = 0;
             int kg = 0;                                      // tiles of this track so far (accumulator phase)
-#ifdef PDDP_EXP_TRACE
             long long tr_wb = 0, tr_wa = 0, tr_is = 0;
-#endif
-#ifdef PDDP_EXP_ALT
-            int obase = 0;                                   // tiles of the OTHER track in the segments before this one
-#endif
             Seg sg;
             for (bool live = seg_at(T0, T1, tiles_p, im.meta, RPP, sg); live; live = seg_at(sg.ta + sg.cnt, T1, tiles_p, im.meta, RPP, sg)) {
             const int ntiles = t == 0 ? sg.n[0] : sg.n[1], first_blk = t * sg.skew, nkb = sg.nkb;
             const uint32_t IDESC1 = idesc_f16(TILE_M, sg.ncol);
-#ifdef PDDP_EXP_ALT
-            const int n_other = t == 0 ? sg.n[1] : sg.n[0];
-            const int lag = sg.skew > nkb - sg.skew ? sg.skew : nkb - sg.skew;
-            const bool alt_ok = sg.n[1] > 0 && NB >= lag + 1;
-#endif
             int k = 0, pos = 0;
             for (int nb = 0; nb < sg.len; ++nb) {
-#ifdef PDDP_EXP_TRACE
                 long long tq0 = TCLK();
-#endif
                 mbar_wait(&b_full[s], bph);
-#ifdef PDDP_EXP_TRACE
                 tr_wb += TCLK() - tq0;
-#endif
                 if (nb < first_blk || k >= ntiles) {
                     if (leader) mbar_arrive(&b_empty[s]);   // this track does not use the block
                 } else {
-#ifdef PDDP_EXP_ALT
-                    // strict alternation of the two tracks' MMA phases: tile m of track 1 starts when tile m of track 0
-                    // is complete, tile m + 1 of track 0 when tile m of track 1 is (so one track's MMAs run while the
-                    // other's accumulator is held by its epilogue).  Needs W1 stages for the lag between the tracks.
-                    if (pos == 0 && alt_ok) {
-                        const int c = t == 1 ? obase + k + 1 : obase + (k < n_other ? k : n_other);
-                        if (c > 0) mbar_wait(&acc1_full[1 - t], (uint32_t)(c - 1) & 1);
-                    }
-#endif
-#ifdef PDDP_EXP_TRACE
                     long long tq1 = TCLK();
                     if (pos == 0) { if (leader) TR(t, kg * 8 + 0, tq1); }
-#endif
                     if (pos == 0) mbar_wait(&acc1_empty[t], ((uint32_t)kg & 1) ^ 1);
-#ifdef PDDP_EXP_TRACE
                     long long tq2 = TCLK();
                     if (pos == 0) { if (leader) TR(t, kg * 8 + 1, tq2); }
-#endif
                     mbar_wait(&a1f[slot], sph);
-#ifdef PDDP_EXP_TRACE
                     long long tq3 = TCLK();
                     tr_wa += tq3 - tq2;
-#endif
                     tc_fence_after();
                     if (leader) {
                         const uint64_t ad = desc_hi | (uint64_t)(a_lo0 + slot * (A1_SLOT >> 4));
-                        const uint64_t bd = desc_hi | (uint64_t)(b_lo0 + s * (B_SSTAGE >> 4));
+                        const uint64_t bd = desc_hi | (uint64_t)(b_lo0 + s * (B_STAGE >> 4));
                         // one UMMA K-step = 32 B of a row = 16 fp16: [x0 | x1] halves are +2 apart in the >>4 address field
                         tc_mma_f16(d_tmem, ad, bd, IDESC1, pos != 0);     // a0 * b0
-#ifndef PDDP_EXP_ONE_PASS            // (timing experiment: a single FP16 pass)
                         tc_mma_f16(d_tmem, ad, bd + 2, IDESC1, 1);        // a0 * b1
                         tc_mma_f16(d_tmem, ad + 2, bd, IDESC1, 1);        // a1 * b0
-#endif
                         tc_commit(&a1e[slot]);
                         tc_commit(&b_empty[s]);
                         if (pos == nkb - 1) tc_commit(&acc1_full[t]);
                     }
                     __syncwarp();
-#ifdef PDDP_EXP_TRACE
                     tr_is += TCLK() - tq3;
                     if (pos == nkb - 1 && leader) {
                         TR(t, kg * 8 + 2, TCLK()); TR(t, kg * 8 + 3, tr_wb); TR(t, kg * 8 + 4, tr_wa); TR(t, kg * 8 + 5, tr_is);
                         tr_wb = tr_wa = tr_is = 0;
                     }
-#endif
                     if (++slot == NS) { slot = 0; sph ^= 1; }
                     if (++pos == nkb) { pos = 0; ++k; ++kg; }
                 }
                 if (++s == NB) { s = 0; bph ^= 1; }
             }
-#ifdef PDDP_EXP_ALT
-            obase += n_other;
-#endif
             }
         }
     }
@@ -816,7 +759,7 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
             auto load_w0 = [&](int p, int nkb_p) {     // the chunks this particle uses: 32 hidden units = 2 K-blocks each
                 const uint32_t w0_bytes = (uint32_t)((nkb_p + 1) / 2) * C::W0_CHUNK;
                 mbar_expect_tx(&w0_full[t], w0_bytes);
-                bulk_g2s(smem + C::W0_OFF + t * C::W0_SMEM, im.W0img + (size_t)p * C::W0_BYTES, w0_bytes, &w0_full[t]);
+                bulk_g2s(smem + C::W0_OFF + t * C::W0_BYTES, im.W0img + (size_t)p * C::W0_BYTES, w0_bytes, &w0_full[t]);
             };
             int curp = cur.p(tiles_p);
             if (r == 0) load_w0(curp, cur.nkb());
@@ -829,13 +772,9 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
             TrackIter nxt = cur;
             nxt.next(T1, tiles_p, t, im.meta);
             int d = 0;                         // pass of the current tile inside its super-tile
-#ifdef PDDP_EXP_TRACE
             int tr_k = 0;
-#endif
             while (cur.valid()) {
-#ifdef PDDP_EXP_TRACE
                 long long tr_w0 = 0, tr_w1 = 0, tr_t0 = TCLK();
-#endif
                 const bool last_pass = d == RPP - 1;
                 const bool more = !last_pass || nxt.valid();        // another tile follows on this track
                 const int nkb = cur.nkb(), kb0 = t * cur.skew();
@@ -845,13 +784,9 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                     if (kb >= nkb) kb -= nkb;
                     const int nk = kb + 1 < nkb ? 2 : 1, j = kb >> 1;
                     float v[32];
-#ifdef PDDP_EXP_TRACE
                     long long tq0 = TCLK();
-#endif
                     mbar_wait(&acc0_full[t], ci & 1);
-#ifdef PDDP_EXP_TRACE
                     tr_w0 += TCLK() - tq0;
-#endif
                     ++ci;
                     tc_fence_after();
                     tc_ld32(lane_taddr + TM_ACC0, v);
@@ -893,50 +828,32 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
 #pragma unroll
                     for (int h = 0; h < 2; ++h) {
                         if (h < nk) {
-#ifdef PDDP_EXP_TRACE
                             long long tq1 = TCLK();
-#endif
                             mbar_wait(&a1_empty[t * NS + slot], sph);
-#ifdef PDDP_EXP_TRACE
                             tr_w1 += TCLK() - tq1;
-#endif
                             const uint32_t A1 = smem_u32(smem + C::A1_OFF + (t * NS + slot) * A1_SLOT) + row_off;
                             uint32_t a0[8], a1[8];            // fp16 pairs: a0 = fp16(v), a1 = fp16(v - a0)
 #pragma unroll
                             for (int e = 0; e < 8; ++e) {
                                 const float v0 = v[16 * h + 2 * e], v1 = v[16 * h + 2 * e + 1];
                                 a0[e] = pack_f16(v0, v1);
-#ifdef PDDP_EXP_MID_CHEAP            // timing experiment only (wrong results): no lo part
-                                a1[e] = 0u;
-#else
                                 const float2 back = unpack_f16(a0[e]);
                                 a1[e] = pack_f16(v0 - back.x, v1 - back.y);
-#endif
                             }
 #pragma unroll
                             for (int c = 0; c < 2; ++c) {     // 16-byte chunks 0,1 = a0[0..7], a0[8..15]; 2,3 = a1
                                 sts128(A1 + ((c ^ row_sw) << 4), a0[4 * c], a0[4 * c + 1], a0[4 * c + 2], a0[4 * c + 3]);
                                 sts128(A1 + (((2 + c) ^ row_sw) << 4), a1[4 * c], a1[4 * c + 1], a1[4 * c + 2], a1[4 * c + 3]);
                             }
-#ifdef PDDP_EXP_FENCE_MERGE           // one proxy fence per chunk: both K-blocks are published after the second one's stores
-                            if (h == nk - 1) {
-                                fence_async_smem();
-                                if (nk == 2) mbar_arrive(&a1_full[t * NS + (slot == 0 ? NS - 1 : slot - 1)]);
-                                mbar_arrive(&a1_full[t * NS + slot]);
-                            }
-#else
                             fence_async_smem();
                             mbar_arrive(&a1_full[t * NS + slot]);
-#endif
                             if (++slot == NS) { slot = 0; sph ^= 1; }
                         }
                     }
                     pos += nk;
                 }
-#ifdef PDDP_EXP_TRACE
                 if (r == 0) { TR(4 + t, tr_k * 4 + 0, tr_t0); TR(4 + t, tr_k * 4 + 1, TCLK()); TR(4 + t, tr_k * 4 + 2, tr_w0); TR(4 + t, tr_k * 4 + 3, tr_w1); }
                 ++tr_k;
-#endif
                 if (++d == RPP) { d = 0; cur = nxt; nxt.next(T1, tiles_p, t, im.meta); }
             }
         } else {
@@ -954,11 +871,7 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
             const uint32_t gate_s = smem_u32(smem + C::GATE_OFF) + (uint32_t)(t * MAX_NCH * TILE_M + r) * 4u;
             int d = 0;
             for (int k = 0; cur.valid(); ++k) {   // k = tiles of this track so far (accumulator phase)
-#ifdef PDDP_EXP_EPI_SHORT            // timing experiment only (wrong results): the epilogue drains 16 columns
-                const int p = cur.p(tiles_p), l = cur.tau - p * tiles_p, ncol = 16;
-#else
                 const int p = cur.p(tiles_p), l = cur.tau - p * tiles_p, ncol = cur.ncol();
-#endif
                 if (p != curp) {
                     named_bar_sync(1 + t, 128);      // every warp of the team is done with the old weights
                     if (r == 0) {
@@ -991,13 +904,9 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                             xin[jr][oo] = (i < S && o < D) ? __ldg(a.X + ((size_t)i * P + p) * D + o) : 0.f;
                         }
                 }
-#ifdef PDDP_EXP_TRACE
                 if (r == 0) TR(2 + t, k * 4 + 0, TCLK());
-#endif
                 mbar_wait(&acc1_full[t], (uint32_t)k & 1);
-#ifdef PDDP_EXP_TRACE
                 if (r == 0) TR(2 + t, k * 4 + 1, TCLK());
-#endif
                 tc_fence_after();
                 // half = 16 columns (two 8-column groups) of both row halves; consumes fragment buffer fb and
                 // shifts (EPI_PRIMAL) / tests (EPI_TANGENT) bits [ebase, ebase+16) of the current gate word
@@ -1101,9 +1010,7 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
                 else columns(std::integral_constant<int, EPI_TANGENT>());
                 tc_fence_before();
                 mbar_arrive(&acc1_empty[t]);
-#ifdef PDDP_EXP_TRACE
                 if (r == 0) TR(2 + t, k * 4 + 2, TCLK());
-#endif
                 // complete the column sums across the quad, then lane q4 writes outputs o = q4 (and q4 + 4)
 #pragma unroll
                 for (int jr = 0; jr < 4; ++jr)
@@ -1126,18 +1033,13 @@ bnn_mlp_tc_kernel(const BnnMlpArgs<float> a, const Images im, int S, int tiles_p
 #pragma unroll
                                 for (int o2 = 0; o2 < D; ++o2) if (o2 == o) yo = y[jr][o2];
                                 const size_t g = (size_t)i * P + p;
-#ifdef PDDP_EXP_NO_STORE             // timing experiment only: one store per tile
-                                if (i != 0) continue;
-#endif
                                 if (!TAN || d == 0) a.Xn[g * D + o] = xin[jr][oo] + ((yo + bo) * sd + mn);
                                 else a.Jp[(g * D + o) * TD + (d - 1)] = ((d - 1) == o ? 1.f : 0.f) + yo * sd;
                             }
                         }
                     }
                 }
-#ifdef PDDP_EXP_TRACE
                 if (r == 0) TR(2 + t, k * 4 + 3, TCLK());
-#endif
                 if (++d == RPP) { d = 0; cur.next(T1, tiles_p, t, im.meta); }
             }
         }

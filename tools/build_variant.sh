@@ -1,7 +1,7 @@
 #!/bin/bash
 # Builds a timing-experiment variant of the library: bnn_mlp.cu recompiled with extra -D flags, linked with the
 # product's other objects into pddp_b200/lib/variants/libpddp_<name>.so (load it with PDDP_B200_LIB=<path>).
-#   tools/build_variant.sh nb7 -DPDDP_EXP_NB=7 -DPDDP_EXP_NS=6 -DPDDP_EXP_BSTAGE=12288
+#   tools/build_variant.sh trace -DPDDP_EXP_TRACE
 set -e
 name=$1; shift
 root=$(cd "$(dirname "$0")/.." && pwd)
