@@ -79,13 +79,19 @@ typedef struct pddp_shape {
 } pddp_shape;
 
 /* Constants of a QRCost on the angle-augmented state (host memory, doubles, row-major DAxDA).
- * Replaces: pddp/costs/quadratic.py:39-58 + pddp/examples/<problem>/cost.py constructor. */
+ * Replaces: pddp/costs/quadratic.py:39-58 + pddp/examples/<problem>/cost.py constructor.
+ * x_goal_b / u_goal_b give every problem of the batch its own goal, in the cost's coordinates (the angle-augmented
+ * state for the pendulum family, e.g. cartpole [x, xdot, thetadot, sin theta, cos theta]; the state for rendezvous).
+ * Either may be given on its own; pddp_linearize_known / _bnn, pddp_rollout_known / _bnn and pddp_cost_derivatives
+ * read them.  A zero-initialised struct (both NULL) steers every problem to x_goal / u_goal. */
 typedef struct pddp_cost {
     double Q[PDDP_MAX_DA * PDDP_MAX_DA];
     double Q_term[PDDP_MAX_DA * PDDP_MAX_DA];
     double R[PDDP_MAX_NU * PDDP_MAX_NU];   /* row-major nu x nu (stride nu) */
     double x_goal[PDDP_MAX_DA];
     double u_goal[PDDP_MAX_NU];
+    const void* x_goal_b;   /* [B, DA] device, shape.dtype, row-major whatever shape.layout; NULL = x_goal above */
+    const void* u_goal_b;   /* [B, nu] device, shape.dtype;                                   NULL = u_goal above */
 } pddp_cost;
 
 /* Known-dynamics constants (host memory). p[] = pendulum: dt,m,l,mu,g ; cartpole: dt,mc,mp,l,mu,g ;

@@ -34,6 +34,13 @@ class Cost(C.Structure):
                 ("u_goal", C.c_double * MAX_NU)]
 
 
+class CostGoals(Cost):
+    """The whole pddp_cost: the constants above plus the per-problem goals x_goal_b [B, DA] / u_goal_b [B, nu]
+    (device pointers, NULL = the shared x_goal / u_goal).  The C entry points take this type, so a bare Cost, which
+    is shorter than pddp_cost, cannot reach them."""
+    _fields_ = [("x_goal_b", C.c_void_p), ("u_goal_b", C.c_void_p)]
+
+
 class KnownDynamics(C.Structure):
     _fields_ = [("p", C.c_double * 8)]
 
@@ -49,18 +56,18 @@ _P = C.c_void_p
 _SIGNATURES = {
     "pddp_version": (C.c_char_p, []),
     "pddp_last_error": (C.c_char_p, []),
-    "pddp_linearize_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamics), C.POINTER(Cost)]
+    "pddp_linearize_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamics), C.POINTER(CostGoals)]
                              + [_P] * 17),
     "pddp_backward": (C.c_int, [C.POINTER(Shape)] + [_P] * 16),
-    "pddp_rollout_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamics), C.POINTER(Cost)]
+    "pddp_rollout_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamics), C.POINTER(CostGoals)]
                            + [_P] * 5 + [C.c_int32] + [_P] * 10),
     "pddp_accept_update": (C.c_int, [C.POINTER(Shape)] + [_P] * 4 + [C.c_double, C.c_double]
                            + [_P] * 13),
-    "pddp_cost_derivatives": (C.c_int, [C.POINTER(Shape), C.POINTER(Cost)] + [_P] * 11),
+    "pddp_cost_derivatives": (C.c_int, [C.POINTER(Shape), C.POINTER(CostGoals)] + [_P] * 11),
     "pddp_bnn_workspace_bytes": (C.c_int64, [C.POINTER(Shape), C.POINTER(BNN), C.c_int32]),
-    "pddp_linearize_bnn": (C.c_int, [C.POINTER(Shape), C.POINTER(BNN), C.POINTER(Cost)] + [_P] * 16
+    "pddp_linearize_bnn": (C.c_int, [C.POINTER(Shape), C.POINTER(BNN), C.POINTER(CostGoals)] + [_P] * 16
                            + [_P, C.c_int64, _P]),
-    "pddp_rollout_bnn": (C.c_int, [C.POINTER(Shape), C.POINTER(BNN), C.POINTER(Cost)] + [_P] * 5
+    "pddp_rollout_bnn": (C.c_int, [C.POINTER(Shape), C.POINTER(BNN), C.POINTER(CostGoals)] + [_P] * 5
                          + [C.c_int32] + [_P] * 10 + [_P, C.c_int64, _P]),
     "pddp_bnn_train_workspace_bytes": (C.c_int64, [_P]),
     "pddp_bnn_train": (C.c_int, [_P] * 12 + [_P, C.c_int64, _P]),

@@ -15,7 +15,7 @@ import torch
 
 from .. import _lib, sharding
 from ..models.bnn.modules import check_model_opts
-from ..solver import LIN_NAMES, cached_solver, expand_bound, fit_alphas, step_alphas
+from ..solver import LIN_NAMES, cached_solver, check_goals, expand_bound, fit_alphas, step_alphas
 from ..utils.encoding import StateEncoding, decode_mean
 from .base import Controller
 
@@ -34,6 +34,12 @@ class iLQRState(IntEnum):
 
     def is_terminal(self):
         return self in (iLQRState.CONVERGED, iLQRState.MAX_REG)
+
+
+def _no_goals_unbatched(batched, x_goal, u_goal):
+    if not batched and (x_goal is not None or u_goal is not None):
+        raise ValueError("per-problem x_goal / u_goal need a batched call (U [B, N, nu]); a single problem's goal "
+                         "is its cost's x_goal / u_goal")
 
 
 def _bounds(u_min, u_max):
@@ -89,13 +95,16 @@ class iLQRController(Controller):
         return Z[0], U[0], iLQRState(int(s.state[0]))
 
     def step(self, z0, U=None, i=0, encoding=StateEncoding.DEFAULT, batch_rollout=True, alphas=None, u_min=None,
-             u_max=None, on_iteration=None, tol=5e-6, max_reg=1e10, _keep_reg=True, **kwargs):
+             u_max=None, on_iteration=None, tol=5e-6, max_reg=1e10, _keep_reg=True, x_goal=None, u_goal=None,
+             **kwargs):
         """One optimisation step: linearise once, then retry backward + rollout with a larger
         regularisation while the state is NOT_PD / REJECTED (ref: ilqr.py:183-235).  `batch_rollout` is accepted
-        for signature compatibility: the kernels always evaluate every alpha and every tangent in parallel."""
+        for signature compatibility: the kernels always evaluate every alpha and every tangent in parallel.
+        With a batched U, x_goal [B, DA] / u_goal [B, nu] give every problem its own goal (see `fit`)."""
         if U is None:
             U = self._U_nominal
         _lib.require_cuda(U, "U")
+        _no_goals_unbatched(U.dim() == 3, x_goal, u_goal)
         self._batched = U.dim() == 3
         Ub = U if self._batched else U.unsqueeze(0)
         zb = z0.reshape(Ub.shape[0], -1)
@@ -103,7 +112,8 @@ class iLQRController(Controller):
         u_min, u_max = _bounds(u_min, u_max)
         s = self._get_solver(Ub.shape[0], Ub.shape[1], encoding, U.dtype, U.device, int(alphas.numel()))
         mu, delta = s.mu.clone(), s.delta.clone()
-        s.set_problem(zb.to(device=U.device, dtype=U.dtype), Ub, u_min, u_max, alphas=alphas, iterations=1)
+        s.set_problem(zb.to(device=U.device, dtype=U.dtype), Ub, u_min, u_max, alphas=alphas, iterations=1,
+                      x_goal=x_goal, u_goal=u_goal)
         if _keep_reg:            # regularisation persists across steps of one fit (ilqr.py:277 resets per fit)
             s.mu.copy_(mu)
             s.delta.copy_(delta)
@@ -120,7 +130,8 @@ class iLQRController(Controller):
         return s.state.clone() if self._batched else iLQRState(int(s.state[0]))
 
     def fit(self, U, encoding=StateEncoding.DEFAULT, n_iterations=50, tol=5e-6, max_reg=1e10, batch_rollout=True,
-            quiet=False, on_iteration=None, u_min=None, u_max=None, z0=None, shard=None, max_passes=None, **kwargs):
+            quiet=False, on_iteration=None, u_min=None, u_max=None, z0=None, shard=None, max_passes=None, x_goal=None,
+            u_goal=None, **kwargs):
         """ref: pddp/controllers/ilqr.py:237-316.  U: [N, nu] (z0 read from env.get_state() unless
         given) or [B, N, nu] with z0 [B, nz].  Returns (Z, U, state).
 
@@ -128,8 +139,14 @@ class iLQRController(Controller):
         batched call, every rank passes the SAME full batch; each optimises its contiguous share of the problems
         -- no collective inside the iteration -- and ONE all-gather at the end gives every rank the full
         (Z, U, K, state).  shard=False keeps the whole batch on this rank.  max_passes bounds the number of
-        whole-batch passes (a pass = linearise / backward / rollout / accept for every problem still in play)."""
+        whole-batch passes (a pass = linearise / backward / rollout / accept for every problem still in play).
+
+        Per-problem goals (batched calls only): x_goal [B, DA] in the cost's coordinates -- the angle-augmented state
+        for the pendulum family (cartpole: [x, xdot, thetadot, sin theta, cos theta]), the state for rendezvous -- and
+        u_goal [B, nu], CUDA tensors.  Either may be given alone; a goal not given is the cost's x_goal / u_goal.
+        A sharded fit splits them like z0."""
         _lib.require_cuda(U, "U")
+        _no_goals_unbatched(U.dim() == 3, x_goal, u_goal)
         self._batched = U.dim() == 3
         Ub = (U if self._batched else U.unsqueeze(0)).detach()
         if z0 is None:
@@ -139,8 +156,11 @@ class iLQRController(Controller):
         world, rank = sharding.world_and_rank()
         sharded = self._batched and world > 1 and shard is not False and Ub.shape[0] >= world
         B_total = Ub.shape[0]
+        if self._batched:
+            x_goal, u_goal = check_goals(x_goal, u_goal, B_total, self.cost.geometry(), U.dtype)
         if sharded:
             Ub, zb = sharding.shard(Ub, world, rank).contiguous(), sharding.shard(zb, world, rank).contiguous()
+            x_goal, u_goal = (None if g is None else sharding.shard(g, world, rank).contiguous() for g in (x_goal, u_goal))
         s = self._get_solver(Ub.shape[0], Ub.shape[1], encoding, U.dtype, U.device, 10)
         it = [0]
 
@@ -156,7 +176,7 @@ class iLQRController(Controller):
                     it[0] += 1
 
         s.fit(zb, Ub, n_iterations=n_iterations, tol=tol, max_reg=max_reg, u_min=u_min, u_max=u_max,
-              alphas=fit_alphas(U.dtype), on_pass=on_pass, max_passes=max_passes)
+              alphas=fit_alphas(U.dtype), on_pass=on_pass, max_passes=max_passes, x_goal=x_goal, u_goal=u_goal)
         if bool((s.state == int(iLQRState.MAX_REG)).any()):
             warnings.warn("exceeded max regularization term")
         if not sharded:
@@ -293,14 +313,22 @@ def _control_law(model, Z, U, k, K, alpha, encoding=StateEncoding.DEFAULT, model
 
 @torch.no_grad()
 def _trajectory_cost(cost, Z, U, encoding=StateEncoding.DEFAULT, cost_opts={}):
-    """ref: pddp/controllers/ilqr.py:764-791 -> J (scalar, or [A] for Z [N+1, A, nz])."""
+    """ref: pddp/controllers/ilqr.py:764-791 -> J (scalar, or [A] for Z [N+1, A, nz]).  The reference hands cost_opts
+    to the cost; here they may carry per-trajectory goals: for Z [N+1, B, nz], cost_opts["x_goal"] [B, DA] /
+    cost_opts["u_goal"] [B, nu] give trajectory b its own goal (as in iLQRController.fit)."""
     batched = Z.dim() == 3
+    x_goal, u_goal = cost_opts.get("x_goal"), cost_opts.get("u_goal")
+    _no_goals_unbatched(batched, x_goal, u_goal)
     Zb = Z.permute(1, 0, 2) if batched else Z.unsqueeze(0)
     Ub = U.permute(1, 0, 2) if batched else U.unsqueeze(0)
     s = cached_solver(None, cost, encoding, Zb.shape[0], Ub.shape[1], Z.dtype, Z.device, layout=_lib.PROBLEM_MAJOR)
+    s.set_goals(x_goal, u_goal)
     s.store("Z", Zb.detach())
     s.store("U", Ub.detach())
-    s.cost_only()
+    try:
+        s.cost_only()
+    finally:
+        s.set_goals()           # the solver is cached and shared with cost-only entry points that take no goals
     J = s.J_opt.clone()
     return J if batched else J[0]
 

@@ -530,6 +530,7 @@ __global__ void __launch_bounds__(256) bnn_roll_step_kernel(const RollStepArgs<T
 #pragma unroll
     for (int e = 0; e < NZ; ++e) zrow[e] = zn[e];
     if (!ok && a.status) atomicOr(&a.status[b], 2);
+    const auto goal = problem_goal<GEO>(a.cost, b);
     T J = Jprev;
     if (t1 < a.N) {                                       // control law (ref: ilqr.py:701-719)
         T du[NU];
@@ -557,15 +558,15 @@ __global__ void __launch_bounds__(256) bnn_roll_step_kernel(const RollStepArgs<T
             a.Uall[((size_t)s * a.N + t1) * NU + i] = u[i];
         }
         if constexpr (GEO == GEO_RENDEZVOUS) {
-            J += rdv_cost_state<ENC, T>(a.cost, zn, false) + rdv_cost_action(a.cost, u);
+            J += rdv_cost_state<ENC, T>(a.cost, goal.x, zn, false) + rdv_cost_action(a.cost, goal.u, u);
         } else {
             T la, lu, luu;
-            cost_action(a.cost, u[0], la, lu, luu);
-            J += cost_state<GEO, ENC, T, T>(a.cost, zn, false) + la;
+            cost_action(a.cost, goal.u[0], u[0], la, lu, luu);
+            J += cost_state<GEO, ENC, T, T>(a.cost, goal.x, zn, false) + la;
         }
     } else {
-        if constexpr (GEO == GEO_RENDEZVOUS) J += rdv_cost_state<ENC, T>(a.cost, zn, true);
-        else J += cost_state<GEO, ENC, T, T>(a.cost, zn, true);
+        if constexpr (GEO == GEO_RENDEZVOUS) J += rdv_cost_state<ENC, T>(a.cost, goal.x, zn, true);
+        else J += cost_state<GEO, ENC, T, T>(a.cost, goal.x, zn, true);
     }
     a.J[s] = J;
 }
@@ -670,16 +671,6 @@ struct BnnCall {
 };
 
 template <class T>
-static void fill_cost_params(const pddp_cost* c, int DA, CostParams<T>& out) {
-    memset(&out, 0, sizeof(out));
-    for (int i = 0; i < DA * DA; ++i) { out.Q[i] = (T)c->Q[i]; out.Qt[i] = (T)c->Q_term[i]; }
-    for (int i = 0; i < DA; ++i) out.xg[i] = (T)c->x_goal[i];
-    for (int i = 0; i < MAX_NU * MAX_NU; ++i) out.R[i] = (T)c->R[i];
-    for (int i = 0; i < MAX_NU; ++i) out.ug[i] = (T)c->u_goal[i];
-}
-
-
-template <class T>
 __global__ void bnn_set_z0_kernel(int B, int nz, const T* z0, T* Z, Layout lZ, const int32_t* active) {
     const int id = blockIdx.x * blockDim.x + threadIdx.x;
     if (id >= B * nz) return;
@@ -749,7 +740,7 @@ static cudaError_t linearize_bnn_impl(const BnnCall& c) {
     // cost value / gradient / Hessian over the whole nominal trajectory (clamped u parked in L_u)
     CostDerivArgs<T> cd;
     cd.B = B; cd.N = N;
-    fill_cost_params<T>(c.cost, G::DA, cd.cost);
+    fill_cost<T>(c.cost, G::DA, cd.cost);
     cd.Z = Z; cd.U = (const T*)c.L_u; cd.active = c.active;
     cd.L = (T*)c.L; cd.L_z = (T*)c.L_z; cd.L_u = (T*)c.L_u; cd.L_zz = (T*)c.L_zz; cd.L_uz = (T*)c.L_uz;
     cd.L_uu = (T*)c.L_uu; cd.J_opt = (T*)c.J_opt;
@@ -786,7 +777,7 @@ static cudaError_t rollout_bnn_impl(const BnnRollCall& c) {
     const long long S = (long long)B * A, total = S * P;
     RollStepArgs<T> r;
     r.B = B; r.N = N; r.A = A; r.P = P;
-    fill_cost_params<T>(c.cost, G::DA, r.cost);
+    fill_cost<T>(c.cost, G::DA, r.cost);
     r.Z = (const T*)c.Z; r.U = (const T*)c.U; r.k = (const T*)c.k; r.K = (const T*)c.K; r.alphas = (const T*)c.alphas;
     r.u_min = (const T*)c.u_min; r.u_max = (const T*)c.u_max; r.active = c.active; r.bw_status = c.bw_status;
     r.Zall = w.Zall; r.Uall = w.Uall; r.ucur = w.ucur; r.J = w.J; r.status = c.status;

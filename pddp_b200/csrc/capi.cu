@@ -37,13 +37,17 @@ static int check_shape(const pddp_shape* s) {
 }
 
 template <class T>
-static void fill_cost(const pddp_cost* c, int DA, CostParams<T>& out) {
+void pddp::fill_cost(const pddp_cost* c, int DA, CostParams<T>& out) {
     memset(&out, 0, sizeof(out));
     for (int i = 0; i < DA * DA; ++i) { out.Q[i] = (T)c->Q[i]; out.Qt[i] = (T)c->Q_term[i]; }
     for (int i = 0; i < DA; ++i) out.xg[i] = (T)c->x_goal[i];
     for (int i = 0; i < MAX_NU * MAX_NU; ++i) out.R[i] = (T)c->R[i];
     for (int i = 0; i < MAX_NU; ++i) out.ug[i] = (T)c->u_goal[i];
+    out.xg_b = (const T*)c->x_goal_b;
+    out.ug_b = (const T*)c->u_goal_b;
 }
+template void pddp::fill_cost<float>(const pddp_cost*, int, CostParams<float>&);
+template void pddp::fill_cost<double>(const pddp_cost*, int, CostParams<double>&);
 
 // pddp_backward only sees derivative tensors: no geometry / encoding constraints
 static int check_shape_backward(const pddp_shape* s) {
@@ -60,7 +64,7 @@ int pddp_capi_fail(int code, const char* msg) { return fail(code, msg); }
 int pddp_capi_cuda(cudaError_t e, const char* what) { return cuda_result(e, what); }
 int pddp_capi_check_shape(const pddp_shape* s) { return check_shape(s); }
 
-extern "C" const char* pddp_version(void) { return "pddp_b200 0.1 (sm_100a)"; }
+extern "C" const char* pddp_version(void) { return "pddp_b200 0.2 (sm_100a)"; }
 extern "C" const char* pddp_last_error(void) { return g_err; }
 
 // ---------------------------------------------------------------------------------------------

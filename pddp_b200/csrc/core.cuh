@@ -72,7 +72,26 @@ struct CostParams {          // ref: costs/quadratic.py:39-58 ; Q acts on the AU
     T R[MAX_NU * MAX_NU];
     T xg[MAX_DA];
     T ug[MAX_NU];
+    const T* xg_b;           // [B, DA] goal of every problem, or NULL: every problem steers to xg
+    const T* ug_b;           // [B, nu] or NULL: ug
 };
+
+// The goal of problem b, loaded once into registers by every kernel that evaluates the cost.
+template <class T, int DA, int NU>
+struct Goal { T x[DA]; T u[NU]; };
+template <int DA, int NU, class T>
+PDDP_HD Goal<T, DA, NU> problem_goal(const CostParams<T>& cp, int64_t b) {
+    Goal<T, DA, NU> g;
+#pragma unroll
+    for (int j = 0; j < DA; ++j) g.x[j] = cp.xg_b ? cp.xg_b[b * DA + j] : cp.xg[j];
+#pragma unroll
+    for (int j = 0; j < NU; ++j) g.u[j] = cp.ug_b ? cp.ug_b[b * NU + j] : cp.ug[j];
+    return g;
+}
+template <int GEO, class T>
+PDDP_HD Goal<T, Geo<GEO>::DA, Geo<GEO>::NU> problem_goal(const CostParams<T>& cp, int64_t b) {
+    return problem_goal<Geo<GEO>::DA, Geo<GEO>::NU, T>(cp, b);
+}
 
 // ---- decoders (ref: utils/encoding.py:144-362) ----------------------------------------------
 template <int D, int ENC, class S, class T>
@@ -136,8 +155,9 @@ PDDP_HD void state_trig(const S* z, StateTrig<GEO, S>& tr) {
     for (int i = 0; i < Geo<GEO>::NANG; ++i) jsincos(z[Geo<GEO>::ang(i)], tr.s[i], tr.c[i]);
 }
 
+// xg: the problem's goal on the augmented state (problem_goal)
 template <int GEO, int ENC, class T, class S>
-PDDP_HD S cost_state(const CostParams<T>& cp, const S* z, bool terminal, const StateTrig<GEO, S>& tr) {
+PDDP_HD S cost_state(const CostParams<T>& cp, const T* xg, const S* z, bool terminal, const StateTrig<GEO, S>& tr) {
     typedef Geo<GEO> G;
     constexpr int D = G::D, DA = G::DA, NNA = G::NNA, NANG = G::NANG;
     const T* Q = terminal ? cp.Qt : cp.Q;
@@ -156,8 +176,8 @@ PDDP_HD S cost_state(const CostParams<T>& cp, const S* z, bool terminal, const S
         for (int i = 0; i < DA; ++i) {
             S row = S(T(0));
 #pragma unroll
-            for (int j = 0; j < DA; ++j) row = row + (Ma[j] - cp.xg[j]) * Q[i * DA + j];
-            val = val + (Ma[i] - cp.xg[i]) * row;
+            for (int j = 0; j < DA; ++j) row = row + (Ma[j] - xg[j]) * Q[i * DA + j];
+            val = val + (Ma[i] - xg[i]) * row;
         }
         return val;
     }
@@ -178,8 +198,8 @@ PDDP_HD S cost_state(const CostParams<T>& cp, const S* z, bool terminal, const S
     for (int i = 0; i < DA; ++i) {
         S row = S(T(0));
 #pragma unroll
-        for (int j = 0; j < DA; ++j) row = row + (Ma[j] - cp.xg[j]) * Q[i * DA + j];
-        val = val + (Ma[i] - cp.xg[i]) * row;
+        for (int j = 0; j < DA; ++j) row = row + (Ma[j] - xg[j]) * Q[i * DA + j];
+        val = val + (Ma[i] - xg[i]) * row;
     }
     // trace term sum_ij Ca[i][j] * Q[j][i], block by block
 #pragma unroll
@@ -226,16 +246,16 @@ PDDP_HD S cost_state(const CostParams<T>& cp, const S* z, bool terminal, const S
 }
 
 template <int GEO, int ENC, class T, class S>
-PDDP_HD S cost_state(const CostParams<T>& cp, const S* z, bool terminal) {
+PDDP_HD S cost_state(const CostParams<T>& cp, const T* xg, const S* z, bool terminal) {
     StateTrig<GEO, S> tr;
     state_trig<GEO, S>(z, tr);
-    return cost_state<GEO, ENC, T, S>(cp, z, terminal, tr);
+    return cost_state<GEO, ENC, T, S>(cp, xg, z, terminal, tr);
 }
 
-// action part of the cost: value, gradient, Hessian (NU == 1)   ref: costs/quadratic.py:86-89
+// action part of the cost: value, gradient, Hessian (NU == 1; ug = the problem's goal)   ref: costs/quadratic.py:86-89
 template <class T>
-PDDP_HD void cost_action(const CostParams<T>& cp, T u, T& l, T& l_u, T& l_uu) {
-    T du = u - cp.ug[0];
+PDDP_HD void cost_action(const CostParams<T>& cp, T ug, T u, T& l, T& l_u, T& l_uu) {
+    T du = u - ug;
     l = du * cp.R[0] * du;
     l_u = T(2) * cp.R[0] * du;
     l_uu = T(2) * cp.R[0];

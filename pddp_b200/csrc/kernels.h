@@ -1,5 +1,6 @@
 // Internal (C++) launch interfaces between capi.cu and the kernel translation units.
 #pragma once
+#include "../../include/pddp_b200.h"
 #include "core.cuh"
 
 namespace pddp {
@@ -55,6 +56,9 @@ struct CostDerivArgs {
     T* L; T* L_z; T* L_u; T* L_zz; T* L_uz; T* L_uu; T* J_opt;
     Layout lZ, lU, lL, lLz, lLu, lLzz, lLuz, lLuu;
 };
+
+// pddp_cost (host, doubles) -> the kernels' CostParams; DA = the geometry's augmented state size (capi.cu)
+template <class T> void fill_cost(const pddp_cost* c, int DA, CostParams<T>& out);
 
 template <class T> cudaError_t linearize_known(int geo, int enc, const LinKnownArgs<T>&, cudaStream_t);
 template <class T> cudaError_t rollout_known(int geo, int enc, const RollKnownArgs<T>&, cudaStream_t);

@@ -15,7 +15,7 @@ namespace pddp {
 // cost value / gradient / Hessian w.r.t. the encoded state, one thread
 // ------------------------------------------------------------------------------------------
 template <class T, int GEO, int ENC, class EmitH>
-__device__ __forceinline__ void cost_derivs_thread(const CostParams<T>& cp, const T* z, bool terminal,
+__device__ __forceinline__ void cost_derivs_thread(const CostParams<T>& cp, const T* xg, const T* z, bool terminal,
                                                    T& l, T* lz, EmitH&& emit_h) {
     constexpr int D = Geo<GEO>::D;
     constexpr int NZ = enc_size(D, ENC);
@@ -28,7 +28,7 @@ __device__ __forceinline__ void cost_derivs_thread(const CostParams<T>& cp, cons
             zj[k] = S(z[k]);
             zj[k].g[k] = T(1);
         }
-        S r = cost_state<GEO, ENC, T, S>(cp, zj, terminal);
+        S r = cost_state<GEO, ENC, T, S>(cp, xg, zj, terminal);
         l = r.v;
 #pragma unroll
         for (int i = 0; i < D; ++i) lz[i] = r.g[i];
@@ -48,7 +48,7 @@ __device__ __forceinline__ void cost_derivs_thread(const CostParams<T>& cp, cons
                     zj[k].g[0] = k == i ? T(1) : T(0);
                     zj[k].g[1] = k == j ? T(1) : T(0);
                 }
-                S r = cost_state<GEO, ENC, T, S>(cp, zj, terminal);
+                S r = cost_state<GEO, ENC, T, S>(cp, xg, zj, terminal);
                 if (i == j) {
                     l = r.v;
                     lz[i] = r.g[0];
@@ -68,6 +68,7 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= a.B) return;
     if (a.active && a.active[b] != 1) return;   // 1 = (re)linearise, 2 = retry with the old one
+    const auto goal = problem_goal<GEO>(a.cost, b);
 
     T z[NZ];
 #pragma unroll
@@ -86,7 +87,7 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
         T l = T(0);
         if (ENC == ENC_IGNORE) {
             T lz[NZ];
-            cost_derivs_thread<T, GEO, ENC>(a.cost, z, terminal, l, lz, [&](int i, int j, T h) {
+            cost_derivs_thread<T, GEO, ENC>(a.cost, goal.x, z, terminal, l, lz, [&](int i, int j, T h) {
                 a.L_zz[a.lLzz.at(b, t, i * NZ + j)] = h;
                 if (i != j) a.L_zz[a.lLzz.at(b, t, j * NZ + i)] = h;
             });
@@ -103,7 +104,7 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
         if (a.U_clamped) a.U_clamped[a.lU.at(b, t, 0)] = u;
         if (ENC == ENC_IGNORE) {
             T la, lu, luu;
-            cost_action(a.cost, u, la, lu, luu);
+            cost_action(a.cost, goal.u[0], u, la, lu, luu);
             l += la;
             J += l;
             a.L[a.lL.at(b, t, 0)] = l;
@@ -159,6 +160,7 @@ template <class T, int GEO, int ENC, bool STORE>
 __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha, bool bounded, T lo, T hi) {
     typedef Geo<GEO> G;
     constexpr int D = G::D, NZ = enc_size(D, ENC);
+    const auto goal = problem_goal<GEO>(a.cost, b);           // (dead in the STORE pass, which evaluates no cost)
     T z[NZ];
 #pragma unroll
     for (int e = 0; e < NZ; ++e) z[e] = a.Z[a.lZ.at(b, 0, e)];
@@ -189,8 +191,8 @@ __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha,
         state_trig<GEO, T>(z, tr);
         if (!STORE) {
             T la, lu, luu;
-            cost_action(a.cost, u, la, lu, luu);
-            J += cost_state<GEO, ENC, T, T>(a.cost, z, false, tr) + la;
+            cost_action(a.cost, goal.u[0], u, la, lu, luu);
+            J += cost_state<GEO, ENC, T, T>(a.cost, goal.x, z, false, tr) + la;
         }
         T zn[NZ];
         known_mean_step<GEO, T, T>(a.dyn, z, u, zn, tr);
@@ -202,7 +204,7 @@ __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha,
 #pragma unroll
         for (int e = 0; e < NZ; ++e) pZn[e * seZ] = z[e];
     } else {
-        J += cost_state<GEO, ENC, T, T>(a.cost, z, true);
+        J += cost_state<GEO, ENC, T, T>(a.cost, goal.x, z, true);
     }
     return J;
 }

@@ -90,18 +90,19 @@ __device__ __forceinline__ bool rdv_uncertainty_step(const T* z, T* zn, T (&U)[R
 
 // ------------------------------------------------------------------------------------------
 // cost value / gradient / Hessian of one (problem, time) site in closed form; Args = LinKnownArgs or
-// CostDerivArgs (same member names).  Replaces batch_eval_cost (utils/evaluation.py:134-239).
+// CostDerivArgs (same member names), goal = problem b's goal.  Replaces batch_eval_cost (utils/evaluation.py:134-239).
 // ------------------------------------------------------------------------------------------
 template <class T, int ENC, class Args>
-__device__ __forceinline__ T lq_cost_site(const Args& a, int b, int t, const T* z, const T* u, bool terminal) {
+__device__ __forceinline__ T lq_cost_site(const Args& a, const Goal<T, RD, RNU>& goal, int b, int t, const T* z, const T* u,
+                                          bool terminal) {
     constexpr int D = RD, NU = RNU, NZ = enc_size(D, ENC);
     const T* Q = terminal ? a.cost.Qt : a.cost.Q;
-    T l = rdv_cost_state<ENC, T>(a.cost, z, terminal);
+    T l = rdv_cost_state<ENC, T>(a.cost, goal.x, z, terminal);
     for (int e = 0; e < NZ * NZ; ++e) a.L_zz[a.lLzz.at(b, t, e)] = T(0);
     for (int i = 0; i < D; ++i) {
         T g = T(0);
         for (int j = 0; j < D; ++j) {
-            g += (Q[i * D + j] + Q[j * D + i]) * (z[j] - a.cost.xg[j]);
+            g += (Q[i * D + j] + Q[j * D + i]) * (z[j] - goal.x[j]);
             a.L_zz[a.lLzz.at(b, t, i * NZ + j)] = Q[i * D + j] + Q[j * D + i];
         }
         a.L_z[a.lLz.at(b, t, i)] = g;
@@ -128,13 +129,13 @@ __device__ __forceinline__ T lq_cost_site(const Args& a, int b, int t, const T* 
         }
     }
     if (!terminal) {
-        l += rdv_cost_action(a.cost, u);
+        l += rdv_cost_action(a.cost, goal.u, u);
 #pragma unroll
         for (int i = 0; i < NU; ++i) {
             T g = T(0);
 #pragma unroll
             for (int j = 0; j < NU; ++j) {
-                g += (a.cost.R[i * NU + j] + a.cost.R[j * NU + i]) * (u[j] - a.cost.ug[j]);
+                g += (a.cost.R[i * NU + j] + a.cost.R[j * NU + i]) * (u[j] - goal.u[j]);
                 a.L_uu[a.lLuu.at(b, t, i * NU + j)] = a.cost.R[i * NU + j] + a.cost.R[j * NU + i];
             }
             a.L_u[a.lLu.at(b, t, i)] = g;
@@ -157,7 +158,7 @@ __global__ void __launch_bounds__(64) lq_cost_kernel(const CostDerivArgs<T> a) {
     for (int e = 0; e < NZ; ++e) z[e] = a.Z[a.lZ.at(b, t, e)];
     if (t < a.N)
         for (int i = 0; i < RNU; ++i) u[i] = a.U[a.lU.at(b, t, i)];
-    lq_cost_site<T, ENC>(a, b, t, z, u, t == a.N);
+    lq_cost_site<T, ENC>(a, problem_goal<RD, RNU>(a.cost, b), b, t, z, u, t == a.N);
 }
 template <class T>
 __global__ void lq_cost_sum_kernel(const CostDerivArgs<T> a) {
@@ -180,6 +181,7 @@ __global__ void __launch_bounds__(64) lq_linearize_kernel(const LinKnownArgs<T> 
     if (a.active && a.active[b] != 1) return;
     const RdvModel<T> md = rdv_model(a.dyn);
     const bool bounded = a.u_min != nullptr && a.u_max != nullptr;
+    const auto goal = problem_goal<RD, RNU>(a.cost, b);
     T z[NZ], zn[NZ];
     for (int e = 0; e < NZ; ++e) z[e] = a.z0[(int64_t)b * NZ + e];
     T J = T(0);
@@ -196,7 +198,7 @@ __global__ void __launch_bounds__(64) lq_linearize_kernel(const LinKnownArgs<T> 
                 if (bounded) u[i] = clampv(u[i], a.u_min[i], a.u_max[i]);   // ref: ilqr.py:459-462
             }
         }
-        J += lq_cost_site<T, ENC>(a, b, t, z, u, terminal);
+        J += lq_cost_site<T, ENC>(a, goal, b, t, z, u, terminal);
         if (terminal) break;
 
         // ---- dynamics + Jacobians ----
@@ -247,6 +249,7 @@ __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alp
     constexpr int D = RD, NU = RNU, NZ = enc_size(D, ENC);
     const RdvModel<T> md = rdv_model(a.dyn);
     const bool bounded = a.u_min != nullptr && a.u_max != nullptr;
+    const auto goal = problem_goal<RD, RNU>(a.cost, b);     // (dead in the STORE pass, which evaluates no cost)
     T z[NZ], zn[NZ];
     for (int e = 0; e < NZ; ++e) z[e] = a.Z[a.lZ.at(b, 0, e)];
     T J = T(0);
@@ -279,7 +282,7 @@ __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alp
             for (int i = 0; i < NU; ++i) pUn[i * seU] = u[i];
             pZn += a.lZ.st; pUn += a.lU.st;
         } else {
-            J += rdv_cost_state<ENC, T>(a.cost, z, false) + rdv_cost_action(a.cost, u);
+            J += rdv_cost_state<ENC, T>(a.cost, goal.x, z, false) + rdv_cost_action(a.cost, goal.u, u);
         }
         rdv_mean_step(md, z, u, zn);
         T U[D][D], Un[D][D];
@@ -289,7 +292,7 @@ __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alp
     if (STORE) {
         for (int e = 0; e < NZ; ++e) pZn[e * seZ] = z[e];
     } else {
-        J += rdv_cost_state<ENC, T>(a.cost, z, true);
+        J += rdv_cost_state<ENC, T>(a.cost, goal.x, z, true);
     }
     return J;
 }

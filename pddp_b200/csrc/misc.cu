@@ -221,6 +221,7 @@ __global__ void __launch_bounds__(128) cost_pairs_kernel(const CostDerivArgs<T> 
         while (p >= NZ - i) { p -= NZ - i; ++i; }
         j = i + p;
     }
+    const auto goal = problem_goal<GEO>(a.cost, b);
     typedef Jet2<T, 2> S;
     S zj[NZ];
 #pragma unroll
@@ -229,7 +230,7 @@ __global__ void __launch_bounds__(128) cost_pairs_kernel(const CostDerivArgs<T> 
         zj[k].g[0] = k == i ? T(1) : T(0);
         zj[k].g[1] = k == j ? T(1) : T(0);
     }
-    S r = cost_state<GEO, ENC, T, S>(a.cost, zj, terminal);
+    S r = cost_state<GEO, ENC, T, S>(a.cost, goal.x, zj, terminal);
     a.L_zz[a.lLzz.at(b, t, i * NZ + j)] = r.h[1];
     if (i != j) a.L_zz[a.lLzz.at(b, t, j * NZ + i)] = r.h[1];
     else a.L_z[a.lLz.at(b, t, i)] = r.g[0];
@@ -238,7 +239,7 @@ __global__ void __launch_bounds__(128) cost_pairs_kernel(const CostDerivArgs<T> 
         T l = r.v;
         if (!terminal) {
             T la, lu, luu;
-            cost_action(a.cost, a.U[a.lU.at(b, t, 0)], la, lu, luu);
+            cost_action(a.cost, goal.u[0], a.U[a.lU.at(b, t, 0)], la, lu, luu);
             l += la;
             a.L_u[a.lLu.at(b, t, 0)] = lu;
             a.L_uu[a.lLuu.at(b, t, 0)] = luu;

@@ -8,9 +8,9 @@ namespace pddp {
 
 constexpr int RDV_D = 8, RDV_NU = 4;
 
-// state part of the QR cost: (m - xg)^T Q (m - xg) + sum_ij C_ij Q_ji   ref: costs/quadratic.py:80-97
+// state part of the QR cost: (m - xg)^T Q (m - xg) + sum_ij C_ij Q_ji, xg = the problem's goal   ref: costs/quadratic.py:80-97
 template <int ENC, class T>
-__device__ __forceinline__ T rdv_cost_state(const CostParams<T>& cp, const T* z, bool terminal) {
+__device__ __forceinline__ T rdv_cost_state(const CostParams<T>& cp, const T* xg, const T* z, bool terminal) {
     constexpr int D = RDV_D;
     const T* Q = terminal ? cp.Qt : cp.Q;
     T val = T(0);
@@ -18,8 +18,8 @@ __device__ __forceinline__ T rdv_cost_state(const CostParams<T>& cp, const T* z,
     for (int i = 0; i < D; ++i) {
         T row = T(0);
 #pragma unroll
-        for (int j = 0; j < D; ++j) row += (z[j] - cp.xg[j]) * Q[j * D + i];
-        val += row * (z[i] - cp.xg[i]);
+        for (int j = 0; j < D; ++j) row += (z[j] - xg[j]) * Q[j * D + i];
+        val += row * (z[i] - xg[i]);
     }
     if (ENC == ENC_FULL) {
 #pragma unroll 1
@@ -44,14 +44,14 @@ __device__ __forceinline__ T rdv_cost_state(const CostParams<T>& cp, const T* z,
 }
 
 template <class T>
-__device__ __forceinline__ T rdv_cost_action(const CostParams<T>& cp, const T* u) {
+__device__ __forceinline__ T rdv_cost_action(const CostParams<T>& cp, const T* ug, const T* u) {
     T val = T(0);
 #pragma unroll
     for (int i = 0; i < RDV_NU; ++i) {
         T row = T(0);
 #pragma unroll
-        for (int j = 0; j < RDV_NU; ++j) row += (u[j] - cp.ug[j]) * cp.R[j * RDV_NU + i];
-        val += row * (u[i] - cp.ug[i]);
+        for (int j = 0; j < RDV_NU; ++j) row += (u[j] - ug[j]) * cp.R[j * RDV_NU + i];
+        val += row * (u[i] - ug[i]);
     }
     return val;
 }

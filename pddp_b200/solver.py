@@ -119,6 +119,23 @@ class BNNDynamics:
         return s
 
 
+def check_goals(x_goal, u_goal, B, geo, dtype):
+    """Per-problem goals as the kernels read them: x_goal [B, DA] on the angle-augmented state, u_goal [B, nu], CUDA
+    tensors, cast to the solver dtype (None stays None).  Raises before anything is launched."""
+    D, nu, ang, _ = _lib.GEO_INFO[geo]
+    out = []
+    for name, g, E in (("x_goal", x_goal, D + len(ang)), ("u_goal", u_goal, nu)):
+        if g is None:
+            out.append(None)
+            continue
+        if not isinstance(g, torch.Tensor) or not g.is_cuda:
+            raise RuntimeError("pddp_b200: per-problem %s must be a CUDA tensor (no CPU fallback)" % name)
+        if tuple(g.shape) != (B, E):
+            raise ValueError("per-problem %s must have shape [B, %d] = [%d, %d], got %s" % (name, E, B, E, list(g.shape)))
+        out.append(g.detach().to(dtype))
+    return out
+
+
 class QRCostConstants:
     """Q, R, Q_term, x_goal, u_goal of a QRCost on the augmented state (ref: costs/quadratic.py)."""
 
@@ -138,7 +155,7 @@ class QRCostConstants:
         nu = int(round(self.R.numel() ** 0.5))
         if nu * nu != self.R.numel() or nu > _lib.MAX_NU or self.u_goal.numel() not in (1, nu):
             raise ValueError("R must be nu x nu with nu <= %d, u_goal a scalar or [nu]" % _lib.MAX_NU)
-        s = _lib.Cost()
+        s = _lib.CostGoals()
         for i, v in enumerate(self.Q.reshape(-1).tolist()):
             s.Q[i] = v
         for i, v in enumerate(self.Q_term.reshape(-1).tolist()):
@@ -197,6 +214,8 @@ class BatchedSolver:
         self.roll_status = torch.zeros(self.B, dtype=torch.int32, **o)
         self.n_active = torch.zeros(1, dtype=torch.int32, **o)
         self.u_min = self.u_max = None
+        self.goals = {}            # per-problem goal buffers ("x_goal" [B, DA], "u_goal" [B, nu]), made on first use
+        self._goal_ptrs = (None, None)
         self.alphas = fit_alphas(dtype, self.device)
         self.launches = 0          # CUDA kernels enqueued by this solver (bench.py reports it)
         self.workspace = None
@@ -241,7 +260,30 @@ class BatchedSolver:
         return v
 
     # ---------------------------------------------------------------- setup
-    def set_problem(self, z0, U, u_min=None, u_max=None, alphas=None, iterations=1):
+    def set_goals(self, x_goal=None, u_goal=None):
+        """Gives every problem its own goal: x_goal [B, DA] in the cost's coordinates (the angle-augmented state,
+        like QRCost.x_goal), u_goal [B, nu].  A goal left None is the cost's own, shared by every problem."""
+        goals = check_goals(x_goal, u_goal, self.B, self.geo, self.dtype)
+        ptrs = []
+        for name, g in zip(("x_goal", "u_goal"), goals):
+            if g is None:
+                ptrs.append(None)
+                continue
+            if name not in self.goals:
+                self.goals[name] = torch.empty(g.shape, dtype=self.dtype, device=self.device)
+            self.goals[name].copy_(g)
+            ptrs.append(self.goals[name].data_ptr())
+        self._goal_ptrs = tuple(ptrs)
+
+    def _cost(self):
+        """The cost argument of a C ABI call, carrying this solver's per-problem goals (or NULL)."""
+        self.c_cost.x_goal_b, self.c_cost.u_goal_b = self._goal_ptrs
+        return C.byref(self.c_cost)
+
+    def set_problem(self, z0, U, u_min=None, u_max=None, alphas=None, iterations=1, x_goal=None, u_goal=None):
+        """Initial states z0 [B, nz], controls U [B, N, nu], bounds, line-search candidates and the per-problem
+        goals of set_goals; goals not given are cleared."""
+        self.set_goals(x_goal, u_goal)
         # (no torch.as_tensor on tensors: under torch.set_default_device it would MOVE them to the default device)
         z0 = (z0 if isinstance(z0, torch.Tensor) else torch.as_tensor(z0)).detach()
         _lib.require_cuda(z0, "z0")
@@ -275,13 +317,13 @@ class BatchedSolver:
         self.lin_status.zero_()
         if self.dyn.is_bnn:
             code = self.lib.pddp_linearize_bnn(
-                C.byref(self.shape), C.byref(self.c_bnn), C.byref(self.c_cost), p(self.z0), p(b["U"]),
+                C.byref(self.shape), C.byref(self.c_bnn), self._cost(), p(self.z0), p(b["U"]),
                 p(self.u_min), p(self.u_max), act, *[p(b[n]) for n in LIN_NAMES], p(self.J_opt),
                 p(self.lin_status), p(self.workspace), self.workspace.numel(), _lib.stream_ptr())
             _lib.check(code, "linearize_bnn")
         else:
             code = self.lib.pddp_linearize_known(
-                C.byref(self.shape), C.byref(self.c_dyn), C.byref(self.c_cost), p(self.z0), p(b["U"]),
+                C.byref(self.shape), C.byref(self.c_dyn), self._cost(), p(self.z0), p(b["U"]),
                 p(self.u_min), p(self.u_max), act, *[p(b[n]) for n in LIN_NAMES], p(self.J_opt),
                 p(self.lin_status), _lib.stream_ptr())
             _lib.check(code, "linearize_known")
@@ -291,7 +333,7 @@ class BatchedSolver:
         """Cost value / gradient / Hessian of whatever is stored in Z, U (no rollout)."""
         b, p = self.buf, _lib.ptr
         code = self.lib.pddp_cost_derivatives(
-            C.byref(self.shape), C.byref(self.c_cost), p(b["Z"]), p(b["U"]), None, p(b["L"]), p(b["L_z"]),
+            C.byref(self.shape), self._cost(), p(b["Z"]), p(b["U"]), None, p(b["L"]), p(b["L_z"]),
             p(b["L_u"]), p(b["L_zz"]), p(b["L_uz"]), p(b["L_uu"]), p(self.J_opt), _lib.stream_ptr())
         _lib.check(code, "cost_derivatives")
 
@@ -315,12 +357,12 @@ class BatchedSolver:
                   p(self.J_new), p(b["Z_new"]), p(b["U_new"]))
         if self.dyn.is_bnn:
             code = self.lib.pddp_rollout_bnn(
-                C.byref(self.shape), C.byref(self.c_bnn), C.byref(self.c_cost), *common,
+                C.byref(self.shape), C.byref(self.c_bnn), self._cost(), *common,
                 p(self.roll_status), p(self.workspace), self.workspace.numel(), _lib.stream_ptr())
             _lib.check(code, "rollout_bnn")
         else:
             code = self.lib.pddp_rollout_known(C.byref(self.shape), C.byref(self.c_dyn),
-                                               C.byref(self.c_cost), *common, _lib.stream_ptr())
+                                               self._cost(), *common, _lib.stream_ptr())
             _lib.check(code, "rollout_known")
 
     @on_own_device
@@ -343,12 +385,12 @@ class BatchedSolver:
 
     # ---------------------------------------------------------------- driver
     def fit(self, z0, U, n_iterations=50, tol=5e-6, max_reg=1e10, u_min=None, u_max=None,
-            alphas=None, max_passes=None, on_pass=None):
+            alphas=None, max_passes=None, on_pass=None, x_goal=None, u_goal=None):
         """Runs every problem until it has done `n_iterations` accepted steps or reached a
         terminal state (CONVERGED / MAX_REG), exactly like B sequential reference `fit` calls
         (ref: ilqr.py:237-316); rejected / not-PD attempts retry with a larger mu and do not
-        consume iterations (ref: ilqr.py:213)."""
-        self.set_problem(z0, U, u_min, u_max, alphas, iterations=n_iterations)
+        consume iterations (ref: ilqr.py:213).  x_goal [B, DA] / u_goal [B, nu]: per-problem goals (set_goals)."""
+        self.set_problem(z0, U, u_min, u_max, alphas, iterations=n_iterations, x_goal=x_goal, u_goal=u_goal)
         passes = 0
         limit = max_passes if max_passes is not None else n_iterations * 64
         while passes < limit:
