@@ -82,8 +82,13 @@ typedef struct pddp_shape {
  * Replaces: pddp/costs/quadratic.py:39-58 + pddp/examples/<problem>/cost.py constructor.
  * x_goal_b / u_goal_b give every problem of the batch its own goal, in the cost's coordinates (the angle-augmented
  * state for the pendulum family, e.g. cartpole [x, xdot, thetadot, sin theta, cos theta]; the state for rendezvous).
- * Either may be given on its own; pddp_linearize_known / _bnn, pddp_rollout_known / _bnn and pddp_cost_derivatives
- * read them.  A zero-initialised struct (both NULL) steers every problem to x_goal / u_goal. */
+ * x_goal_bt / u_goal_bt give every problem a goal per step, in the same coordinates, to track a reference trajectory:
+ * row t of x_goal_bt [B, N+1, DA] is the goal of the state at step t (row N goes with Q_term in the terminal cost),
+ * row t of u_goal_bt [B, N, nu] the goal of the control at step t.  Both are [B, Nt, E] tensors in shape.layout, like
+ * Z and U.  x and u choose their source independently: x_goal_bt if given, else x_goal_b, else x_goal (likewise u).
+ * Giving both x_goal_b and x_goal_bt (or u_goal_b and u_goal_bt) is PDDP_E_BADARG.
+ * pddp_linearize_known / _bnn, pddp_rollout_known / _bnn and pddp_cost_derivatives read all four pointers.
+ * A zero-initialised struct (all NULL) steers every problem to x_goal / u_goal. */
 typedef struct pddp_cost {
     double Q[PDDP_MAX_DA * PDDP_MAX_DA];
     double Q_term[PDDP_MAX_DA * PDDP_MAX_DA];
@@ -92,6 +97,8 @@ typedef struct pddp_cost {
     double u_goal[PDDP_MAX_NU];
     const void* x_goal_b;   /* [B, DA] device, shape.dtype, row-major whatever shape.layout; NULL = x_goal above */
     const void* u_goal_b;   /* [B, nu] device, shape.dtype;                                   NULL = u_goal above */
+    const void* x_goal_bt;  /* [B, N+1, DA] device, shape.dtype, in shape.layout; NULL = x_goal_b, then x_goal */
+    const void* u_goal_bt;  /* [B, N, nu] device, shape.dtype, in shape.layout;   NULL = u_goal_b, then u_goal */
 } pddp_cost;
 
 /* Known-dynamics constants (host memory). p[] = pendulum: dt,m,l,mu,g ; cartpole: dt,mc,mp,l,mu,g ;

@@ -35,10 +35,12 @@ class Cost(C.Structure):
 
 
 class CostGoals(Cost):
-    """The whole pddp_cost: the constants above plus the per-problem goals x_goal_b [B, DA] / u_goal_b [B, nu]
-    (device pointers, NULL = the shared x_goal / u_goal).  The C entry points take this type, so a bare Cost, which
-    is shorter than pddp_cost, cannot reach them."""
-    _fields_ = [("x_goal_b", C.c_void_p), ("u_goal_b", C.c_void_p)]
+    """The whole pddp_cost: the constants above plus the per-problem goals x_goal_b [B, DA] / u_goal_b [B, nu] and
+    the per-step goals x_goal_bt [B, N+1, DA] / u_goal_bt [B, N, nu] in the shape's layout (device pointers, NULL =
+    the next source: x_goal_bt, then x_goal_b, then the shared x_goal; likewise u).  The C entry points take this
+    type, so a bare Cost, which is shorter than pddp_cost, cannot reach them."""
+    _fields_ = [("x_goal_b", C.c_void_p), ("u_goal_b", C.c_void_p), ("x_goal_bt", C.c_void_p),
+                ("u_goal_bt", C.c_void_p)]
 
 
 class KnownDynamics(C.Structure):

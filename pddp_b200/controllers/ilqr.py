@@ -36,10 +36,37 @@ class iLQRState(IntEnum):
         return self in (iLQRState.CONVERGED, iLQRState.MAX_REG)
 
 
-def _no_goals_unbatched(batched, x_goal, u_goal):
-    if not batched and (x_goal is not None or u_goal is not None):
-        raise ValueError("per-problem x_goal / u_goal need a batched call (U [B, N, nu]); a single problem's goal "
-                         "is its cost's x_goal / u_goal")
+def batch_goals(batched, N, x_goal, u_goal):
+    """The goals of a call in the batched solver's form.  A batched call passes them through: x_goal [B, DA] or
+    [B, N+1, DA], u_goal [B, nu] or [B, N, nu].  A single problem (U [N, nu]) takes only the per-step forms
+    x_goal [N+1, DA] / u_goal [N, nu], returned as a batch of one; its fixed goal is its cost's x_goal / u_goal.
+    Raises ValueError on a row count that fits neither rule (widths are checked by solver.check_goals)."""
+    if batched:
+        return x_goal, u_goal
+    out = []
+    for name, g, Nt in (("x_goal", x_goal, N + 1), ("u_goal", u_goal, N)):
+        if g is None:
+            out.append(None)
+        elif isinstance(g, torch.Tensor) and g.dim() == 2 and g.shape[0] == Nt:
+            out.append(g.unsqueeze(0))
+        else:
+            raise ValueError("a single problem (U [N, nu]) takes a per-step %s of %d rows ([%d, E]), got %s; "
+                             "per-problem goals need a batched call (U [B, N, nu])"
+                             % (name, Nt, Nt, list(g.shape) if isinstance(g, torch.Tensor) else type(g).__name__))
+    return out
+
+
+def reference_window(ref, i, n, batched):
+    """Rows min(i + t, T - 1), t = 0 .. n-1, of a reference with a time axis of length T >= 1 (ref [B, T, E]
+    batched, [T, E] unbatched): the goals that MPC step i optimises against, held at the reference's last row past
+    its end.  A goal without a time axis ([B, E] batched) and None pass through."""
+    if ref is None or ref.dim() != (3 if batched else 2):
+        return ref
+    T = ref.shape[-2]
+    if T < 1:
+        raise ValueError("a reference needs at least one row")
+    rows = torch.arange(i, i + n, device=ref.device).clamp(max=T - 1)
+    return ref.index_select(ref.dim() - 2, rows)
 
 
 def _bounds(u_min, u_max):
@@ -100,11 +127,11 @@ class iLQRController(Controller):
         """One optimisation step: linearise once, then retry backward + rollout with a larger
         regularisation while the state is NOT_PD / REJECTED (ref: ilqr.py:183-235).  `batch_rollout` is accepted
         for signature compatibility: the kernels always evaluate every alpha and every tangent in parallel.
-        With a batched U, x_goal [B, DA] / u_goal [B, nu] give every problem its own goal (see `fit`)."""
+        x_goal / u_goal give every problem its own goal, fixed or per step (see `fit`)."""
         if U is None:
             U = self._U_nominal
         _lib.require_cuda(U, "U")
-        _no_goals_unbatched(U.dim() == 3, x_goal, u_goal)
+        x_goal, u_goal = batch_goals(U.dim() == 3, U.shape[-2], x_goal, u_goal)
         self._batched = U.dim() == 3
         Ub = U if self._batched else U.unsqueeze(0)
         zb = z0.reshape(Ub.shape[0], -1)
@@ -141,12 +168,14 @@ class iLQRController(Controller):
         (Z, U, K, state).  shard=False keeps the whole batch on this rank.  max_passes bounds the number of
         whole-batch passes (a pass = linearise / backward / rollout / accept for every problem still in play).
 
-        Per-problem goals (batched calls only): x_goal [B, DA] in the cost's coordinates -- the angle-augmented state
+        Per-problem goals (batched calls): x_goal [B, DA] in the cost's coordinates -- the angle-augmented state
         for the pendulum family (cartpole: [x, xdot, thetadot, sin theta, cos theta]), the state for rendezvous -- and
-        u_goal [B, nu], CUDA tensors.  Either may be given alone; a goal not given is the cost's x_goal / u_goal.
-        A sharded fit splits them like z0."""
+        u_goal [B, nu], CUDA tensors.  Per-step goals track a reference: x_goal [B, N+1, DA] (row t = the goal of the
+        state at step t, row N with Q_term), u_goal [B, N, nu]; a single problem (U [N, nu]) takes them as
+        [N+1, DA] / [N, nu].  x and u choose their form independently; a goal not given is the cost's x_goal /
+        u_goal.  A sharded fit splits them like z0."""
         _lib.require_cuda(U, "U")
-        _no_goals_unbatched(U.dim() == 3, x_goal, u_goal)
+        x_goal, u_goal = batch_goals(U.dim() == 3, U.shape[-2], x_goal, u_goal)
         self._batched = U.dim() == 3
         Ub = (U if self._batched else U.unsqueeze(0)).detach()
         if z0 is None:
@@ -156,8 +185,7 @@ class iLQRController(Controller):
         world, rank = sharding.world_and_rank()
         sharded = self._batched and world > 1 and shard is not False and Ub.shape[0] >= world
         B_total = Ub.shape[0]
-        if self._batched:
-            x_goal, u_goal = check_goals(x_goal, u_goal, B_total, self.cost.geometry(), U.dtype)
+        x_goal, u_goal = check_goals(x_goal, u_goal, B_total, self.cost.geometry(), U.dtype, Ub.shape[1])
         if sharded:
             Ub, zb = sharding.shard(Ub, world, rank).contiguous(), sharding.shard(zb, world, rank).contiguous()
             x_goal, u_goal = (None if g is None else sharding.shard(g, world, rank).contiguous() for g in (x_goal, u_goal))
@@ -189,7 +217,12 @@ class iLQRController(Controller):
     def forward(self, z, i, encoding=StateEncoding.DEFAULT, mpc=False, ignore_uncertainty=True, u_min=None,
                 u_max=None, **kwargs):
         """ref: pddp/controllers/ilqr.py:318-362 -- time-varying feedback law, or one MPC iteration
-        from the measured state followed by a left shift of the nominal controls."""
+        from the measured state followed by a left shift of the nominal controls.
+
+        Receding-horizon tracking: under mpc, an x_goal with a time axis ([B, T, DA] batched, [T, DA] for one
+        problem) is a reference for the whole trial, of any length T >= 1; MPC step i optimises against its rows
+        min(i + t, T - 1), t = 0 .. N (reference_window).  A u_goal with a time axis likewise, t = 0 .. N-1.  Goals
+        without one ([B, DA] / [B, nu]) pass through to `step` as they are."""
         if self._U_nominal is None:
             raise RuntimeError("You need to either call fit or initialize _U_nominal")
         if not mpc:
@@ -204,6 +237,10 @@ class iLQRController(Controller):
                 dx = decode_mean(z, encoding, D) - decode_mean(Zn, encoding, D)
                 return Un + (Kn[..., :D] @ dx.unsqueeze(-1)).squeeze(-1)
             return Un + (Kn @ (z - Zn).unsqueeze(-1)).squeeze(-1)
+        batched, N = self._U_nominal.dim() == 3, self._U_nominal.shape[-2]
+        for name, n in (("x_goal", N + 1), ("u_goal", N)):
+            if kwargs.get(name) is not None:
+                kwargs[name] = reference_window(kwargs[name], i, n, batched)
         self.step(z, i=i, encoding=encoding, u_min=u_min, u_max=u_max, _keep_reg=False, **kwargs)
         if self._batched:
             u = self._U_nominal[:, 0].clone()
@@ -315,10 +352,10 @@ def _control_law(model, Z, U, k, K, alpha, encoding=StateEncoding.DEFAULT, model
 def _trajectory_cost(cost, Z, U, encoding=StateEncoding.DEFAULT, cost_opts={}):
     """ref: pddp/controllers/ilqr.py:764-791 -> J (scalar, or [A] for Z [N+1, A, nz]).  The reference hands cost_opts
     to the cost; here they may carry per-trajectory goals: for Z [N+1, B, nz], cost_opts["x_goal"] [B, DA] /
-    cost_opts["u_goal"] [B, nu] give trajectory b its own goal (as in iLQRController.fit)."""
+    cost_opts["u_goal"] [B, nu] give trajectory b its own goal, and x_goal [B, N+1, DA] / u_goal [B, N, nu] (problem
+    major, as in iLQRController.fit) a goal per step; for an unbatched Z [N+1, nz], [N+1, DA] / [N, nu]."""
     batched = Z.dim() == 3
-    x_goal, u_goal = cost_opts.get("x_goal"), cost_opts.get("u_goal")
-    _no_goals_unbatched(batched, x_goal, u_goal)
+    x_goal, u_goal = batch_goals(batched, U.shape[0], cost_opts.get("x_goal"), cost_opts.get("u_goal"))
     Zb = Z.permute(1, 0, 2) if batched else Z.unsqueeze(0)
     Ub = U.permute(1, 0, 2) if batched else U.unsqueeze(0)
     s = cached_solver(None, cost, encoding, Zb.shape[0], Ub.shape[1], Z.dtype, Z.device, layout=_lib.PROBLEM_MAJOR)

@@ -413,7 +413,8 @@ struct RollStepArgs {
 // (History: one thread per pair issued 2 x P strided 4-byte loads per sector and ran at 9 % issue utilisation; 8 lanes
 // per pair reading global memory directly spent the launch in 2 x P / LPP dependent round trips to L2: 28 us.)
 // STAGE = false: the particles of 32 pairs do not fit shared memory (very large P): phase A reads them from global memory.
-template <class T, int GEO, int ENC, int LPP, bool STAGE = true>
+// STEP: the cost reads per-step goals (CostParams::xg_bt / ug_bt); launched only when they are given.
+template <class T, int GEO, int ENC, int LPP, bool STAGE = true, bool STEP = false>
 __global__ void __launch_bounds__(256) bnn_roll_step_kernel(const RollStepArgs<T> a) {
     typedef Geo<GEO> G;
     constexpr int D = G::D, NU = G::NU, NZ = enc_size(D, ENC), NT = D * (D + 1) / 2, PPC = 256 / LPP;
@@ -530,7 +531,7 @@ __global__ void __launch_bounds__(256) bnn_roll_step_kernel(const RollStepArgs<T
 #pragma unroll
     for (int e = 0; e < NZ; ++e) zrow[e] = zn[e];
     if (!ok && a.status) atomicOr(&a.status[b], 2);
-    const auto goal = problem_goal<GEO>(a.cost, b);
+    const auto goal = STEP ? site_goal<GEO>(a.cost, b, t1, t1 == a.N) : problem_goal<GEO>(a.cost, b);
     T J = Jprev;
     if (t1 < a.N) {                                       // control law (ref: ilqr.py:701-719)
         T du[NU];
@@ -740,7 +741,7 @@ static cudaError_t linearize_bnn_impl(const BnnCall& c) {
     // cost value / gradient / Hessian over the whole nominal trajectory (clamped u parked in L_u)
     CostDerivArgs<T> cd;
     cd.B = B; cd.N = N;
-    fill_cost<T>(c.cost, G::DA, cd.cost);
+    fill_cost<T>(c.cost, s, cd.cost);
     cd.Z = Z; cd.U = (const T*)c.L_u; cd.active = c.active;
     cd.L = (T*)c.L; cd.L_z = (T*)c.L_z; cd.L_u = (T*)c.L_u; cd.L_zz = (T*)c.L_zz; cd.L_uz = (T*)c.L_uz;
     cd.L_uu = (T*)c.L_uu; cd.J_opt = (T*)c.J_opt;
@@ -777,7 +778,7 @@ static cudaError_t rollout_bnn_impl(const BnnRollCall& c) {
     const long long S = (long long)B * A, total = S * P;
     RollStepArgs<T> r;
     r.B = B; r.N = N; r.A = A; r.P = P;
-    fill_cost<T>(c.cost, G::DA, r.cost);
+    fill_cost<T>(c.cost, s, r.cost);
     r.Z = (const T*)c.Z; r.U = (const T*)c.U; r.k = (const T*)c.k; r.K = (const T*)c.K; r.alphas = (const T*)c.alphas;
     r.u_min = (const T*)c.u_min; r.u_max = (const T*)c.u_max; r.active = c.active; r.bw_status = c.bw_status;
     r.Zall = w.Zall; r.Uall = w.Uall; r.ucur = w.ucur; r.J = w.J; r.status = c.status;
@@ -795,11 +796,16 @@ static cudaError_t rollout_bnn_impl(const BnnRollCall& c) {
                                                                     nullptr, w.Xa, c.status);
     // 8 lanes per (problem, alpha) pair while that grid fits the SMs in one wave, else 4 (cfg 2: 1 280 CTAs were 1.7 waves)
     const size_t pair_bytes = (size_t)P * D * sizeof(T);
-    const bool lpp4 = (S + 31) / 32 > (long long)num_sms() * 4 && 64 * pair_bytes <= 100 * 1024;
+    // per-step goals: always 8 lanes per pair, one instantiation fewer (where shared / per-problem goals take 4, the
+    // particle covariances then sum in another order: equal to the last bits)
+    const bool step = r.cost.xg_bt || r.cost.ug_bt;
+    const bool lpp4 = !step && (S + 31) / 32 > (long long)num_sms() * 4 && 64 * pair_bytes <= 100 * 1024;
     const unsigned rgrid = (unsigned)(lpp4 ? (S + 63) / 64 : (S + 31) / 32);
     const bool stage = 32 * pair_bytes + 16 <= 200 * 1024;       // else: particles straight from global memory
     const size_t rsmem = stage ? (lpp4 ? 64 : 32) * pair_bytes + 16 : 0;
-    auto roll_step = !stage ? bnn_roll_step_kernel<T, GEO, ENC, 8, false>
+    auto roll_step = step ? (stage ? bnn_roll_step_kernel<T, GEO, ENC, 8, true, true>
+                                   : bnn_roll_step_kernel<T, GEO, ENC, 8, false, true>)
+                   : !stage ? bnn_roll_step_kernel<T, GEO, ENC, 8, false>
                    : lpp4 ? bnn_roll_step_kernel<T, GEO, ENC, 4> : bnn_roll_step_kernel<T, GEO, ENC, 8>;
     CK(cudaFuncSetAttribute(roll_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rsmem));
     r.t = -1; r.Xn = w.Xa;
@@ -865,6 +871,7 @@ using namespace pddp;
 int pddp_capi_fail(int code, const char* msg);          // capi.cu
 int pddp_capi_cuda(cudaError_t e, const char* what);    // capi.cu
 int pddp_capi_check_shape(const pddp_shape* s);         // capi.cu
+int pddp_capi_check_cost(const pddp_cost* c);           // capi.cu
 
 static int check_bnn(const pddp_shape* s, const pddp_bnn* n) {
     if (int e = pddp_capi_check_shape(s)) return e;
@@ -897,6 +904,7 @@ extern "C" int pddp_linearize_bnn(const pddp_shape* s, const pddp_bnn* n, const 
     if (int e = check_bnn(s, n)) return e;
     if (!cost || !z0 || !U || !Z || !F_z || !F_u || !L || !L_z || !L_u || !L_zz || !L_uz || !L_uu || !J_opt || !workspace)
         return pddp_capi_fail(PDDP_E_BADARG, "pddp_linearize_bnn: NULL argument");
+    if (int e = pddp_capi_check_cost(cost)) return e;
     if ((u_min == nullptr) != (u_max == nullptr)) return pddp_capi_fail(PDDP_E_BADARG, "u_min and u_max must be given together");
     if (workspace_bytes < pddp_bnn_workspace_bytes(s, n, 1)) return pddp_capi_fail(PDDP_E_BADARG, "workspace too small");
     BnnCall c{s, n, cost, z0, U, u_min, u_max, active, Z, F_z, F_u, L, L_z, L_u, L_zz, L_uz, L_uu, J_opt, status,
@@ -914,6 +922,7 @@ extern "C" int pddp_rollout_bnn(const pddp_shape* s, const pddp_bnn* n, const pd
     if (int e = check_bnn(s, n)) return e;
     if (!cost || !Z || !U || !k || !K || !alphas || !J_all || !amin || !J_new || !Z_new || !U_new || !workspace)
         return pddp_capi_fail(PDDP_E_BADARG, "pddp_rollout_bnn: NULL argument");
+    if (int e = pddp_capi_check_cost(cost)) return e;
     if (A < 1 || A > 64) return pddp_capi_fail(PDDP_E_BADARG, "1 <= A <= 64");
     if ((u_min == nullptr) != (u_max == nullptr)) return pddp_capi_fail(PDDP_E_BADARG, "u_min and u_max must be given together");
     if (workspace_bytes < pddp_bnn_workspace_bytes(s, n, A)) return pddp_capi_fail(PDDP_E_BADARG, "workspace too small");

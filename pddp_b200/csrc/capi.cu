@@ -36,8 +36,16 @@ static int check_shape(const pddp_shape* s) {
     return 0;
 }
 
+// a goal comes from one source: per problem ([B, .]) or per problem and step ([B, Nt, .]), not both
+static int check_cost(const pddp_cost* c) {
+    if (c->x_goal_b && c->x_goal_bt) return fail(PDDP_E_BADARG, "pddp_cost: x_goal_b and x_goal_bt are exclusive");
+    if (c->u_goal_b && c->u_goal_bt) return fail(PDDP_E_BADARG, "pddp_cost: u_goal_b and u_goal_bt are exclusive");
+    return 0;
+}
+
 template <class T>
-void pddp::fill_cost(const pddp_cost* c, int DA, CostParams<T>& out) {
+void pddp::fill_cost(const pddp_cost* c, const pddp_shape* s, CostParams<T>& out) {
+    const int DA = geo_DA(s->geo);
     memset(&out, 0, sizeof(out));
     for (int i = 0; i < DA * DA; ++i) { out.Q[i] = (T)c->Q[i]; out.Qt[i] = (T)c->Q_term[i]; }
     for (int i = 0; i < DA; ++i) out.xg[i] = (T)c->x_goal[i];
@@ -45,9 +53,13 @@ void pddp::fill_cost(const pddp_cost* c, int DA, CostParams<T>& out) {
     for (int i = 0; i < MAX_NU; ++i) out.ug[i] = (T)c->u_goal[i];
     out.xg_b = (const T*)c->x_goal_b;
     out.ug_b = (const T*)c->u_goal_b;
+    out.xg_bt = (const T*)c->x_goal_bt;
+    out.ug_bt = (const T*)c->u_goal_bt;
+    out.lXg = make_layout(s->layout, s->B, (int64_t)s->N + 1, DA);
+    out.lUg = make_layout(s->layout, s->B, s->N, s->nu);
 }
-template void pddp::fill_cost<float>(const pddp_cost*, int, CostParams<float>&);
-template void pddp::fill_cost<double>(const pddp_cost*, int, CostParams<double>&);
+template void pddp::fill_cost<float>(const pddp_cost*, const pddp_shape*, CostParams<float>&);
+template void pddp::fill_cost<double>(const pddp_cost*, const pddp_shape*, CostParams<double>&);
 
 // pddp_backward only sees derivative tensors: no geometry / encoding constraints
 static int check_shape_backward(const pddp_shape* s) {
@@ -63,6 +75,7 @@ static int check_shape_backward(const pddp_shape* s) {
 int pddp_capi_fail(int code, const char* msg) { return fail(code, msg); }
 int pddp_capi_cuda(cudaError_t e, const char* what) { return cuda_result(e, what); }
 int pddp_capi_check_shape(const pddp_shape* s) { return check_shape(s); }
+int pddp_capi_check_cost(const pddp_cost* c) { return check_cost(c); }
 
 extern "C" const char* pddp_version(void) { return "pddp_b200 0.2 (sm_100a)"; }
 extern "C" const char* pddp_last_error(void) { return g_err; }
@@ -76,7 +89,7 @@ static int linearize_known_t(const pddp_shape* s, const pddp_known_dynamics* dyn
                              cudaStream_t st) {
     LinKnownArgs<T> a;
     a.B = s->B; a.N = s->N;
-    fill_cost(cost, geo_DA(s->geo), a.cost);
+    fill_cost(cost, s, a.cost);
     for (int i = 0; i < 8; ++i) a.dyn.p[i] = (T)dyn->p[i];
     a.z0 = (const T*)z0; a.U = (const T*)U; a.u_min = (const T*)u_min; a.u_max = (const T*)u_max;
     a.active = active;
@@ -124,6 +137,7 @@ extern "C" int pddp_linearize_known(const pddp_shape* s, const pddp_known_dynami
     if (int e = check_shape(s)) return e;
     if (!dyn || !cost || !z0 || !U || !Z || !F_z || !F_u || !L || !L_z || !L_u || !L_zz || !L_uz || !L_uu || !J_opt)
         return fail(PDDP_E_BADARG, "pddp_linearize_known: NULL argument");
+    if (int e = check_cost(cost)) return e;
     if ((u_min == nullptr) != (u_max == nullptr)) return fail(PDDP_E_BADARG, "u_min and u_max must be given together");
     cudaStream_t st = (cudaStream_t)stream;
     if (s->dtype == PDDP_F32)
@@ -202,7 +216,7 @@ static int rollout_known_t(const pddp_shape* s, const pddp_known_dynamics* dyn, 
                            void* U_new, cudaStream_t st) {
     RollKnownArgs<T> a;
     a.B = s->B; a.N = s->N; a.A = A;
-    fill_cost(cost, geo_DA(s->geo), a.cost);
+    fill_cost(cost, s, a.cost);
     for (int i = 0; i < 8; ++i) a.dyn.p[i] = (T)dyn->p[i];
     a.Z = (const T*)Z; a.U = (const T*)U; a.k = (const T*)k; a.K = (const T*)K; a.alphas = (const T*)alphas;
     a.u_min = (const T*)u_min; a.u_max = (const T*)u_max; a.active = active; a.bw_status = bw_status;
@@ -225,6 +239,7 @@ extern "C" int pddp_rollout_known(const pddp_shape* s, const pddp_known_dynamics
     if (int e = check_shape(s)) return e;
     if (!dyn || !cost || !Z || !U || !k || !K || !alphas || !J_all || !amin || !J_new || !Z_new || !U_new)
         return fail(PDDP_E_BADARG, "pddp_rollout_known: NULL argument");
+    if (int e = check_cost(cost)) return e;
     if (A < 1 || A > 32) return fail(PDDP_E_UNSUPPORTED, "1 <= A <= 32 line-search candidates");
     if ((u_min == nullptr) != (u_max == nullptr)) return fail(PDDP_E_BADARG, "u_min and u_max must be given together");
     cudaStream_t st = (cudaStream_t)stream;
@@ -278,7 +293,7 @@ static int cost_derivs_t(const pddp_shape* s, const pddp_cost* cost, const void*
                          void* L_uu, void* J_opt, cudaStream_t st) {
     CostDerivArgs<T> a;
     a.B = s->B; a.N = s->N;
-    fill_cost(cost, geo_DA(s->geo), a.cost);
+    fill_cost(cost, s, a.cost);
     a.Z = (const T*)Z; a.U = (const T*)U; a.active = active;
     a.L = (T*)L; a.L_z = (T*)L_z; a.L_u = (T*)L_u; a.L_zz = (T*)L_zz; a.L_uz = (T*)L_uz; a.L_uu = (T*)L_uu;
     a.J_opt = (T*)J_opt;
@@ -301,6 +316,7 @@ extern "C" int pddp_cost_derivatives(const pddp_shape* s, const pddp_cost* cost,
     if (int e = check_shape(s)) return e;
     if (!cost || !Z || !U || !L || !L_z || !L_u || !L_zz || !L_uz || !L_uu)
         return fail(PDDP_E_BADARG, "pddp_cost_derivatives: NULL argument");
+    if (int e = check_cost(cost)) return e;
     cudaStream_t st = (cudaStream_t)stream;
     if (s->dtype == PDDP_F32) return cost_derivs_t<float>(s, cost, Z, U, active, L, L_z, L_u, L_zz, L_uz, L_uu, J_opt, st);
     return cost_derivs_t<double>(s, cost, Z, U, active, L, L_z, L_u, L_zz, L_uz, L_uu, J_opt, st);

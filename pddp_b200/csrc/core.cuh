@@ -74,6 +74,9 @@ struct CostParams {          // ref: costs/quadratic.py:39-58 ; Q acts on the AU
     T ug[MAX_NU];
     const T* xg_b;           // [B, DA] goal of every problem, or NULL: every problem steers to xg
     const T* ug_b;           // [B, nu] or NULL: ug
+    const T* xg_bt;          // [B, N+1, DA] goal of every problem and step (layout lXg), or NULL: xg_b / xg
+    const T* ug_bt;          // [B, N, nu] (layout lUg) or NULL: ug_b / ug
+    Layout lXg, lUg;
 };
 
 // The goal of problem b, loaded once into registers by every kernel that evaluates the cost.
@@ -91,6 +94,34 @@ PDDP_HD Goal<T, DA, NU> problem_goal(const CostParams<T>& cp, int64_t b) {
 template <int GEO, class T>
 PDDP_HD Goal<T, Geo<GEO>::DA, Geo<GEO>::NU> problem_goal(const CostParams<T>& cp, int64_t b) {
     return problem_goal<Geo<GEO>::DA, Geo<GEO>::NU, T>(cp, b);
+}
+
+// Per-step goals: where xg_bt / ug_bt are given, row t replaces the problem's goal at step t (x: t = 0..N, row N
+// with Q_term; u: t = 0..N-1).  Only the load changes; the cost arithmetic after it is the shared-goal arithmetic.
+// Time-loop kernels call these per step (or advance running pointers); the per-(problem, step) kernels take
+// site_goal.
+template <int DA, int NU, class T>
+PDDP_HD void step_goal_x(const CostParams<T>& cp, int64_t b, int64_t t, Goal<T, DA, NU>& g) {
+    if (!cp.xg_bt) return;
+#pragma unroll
+    for (int j = 0; j < DA; ++j) g.x[j] = cp.xg_bt[cp.lXg.at(b, t, j)];
+}
+template <int DA, int NU, class T>
+PDDP_HD void step_goal_u(const CostParams<T>& cp, int64_t b, int64_t t, Goal<T, DA, NU>& g) {
+    if (!cp.ug_bt) return;
+#pragma unroll
+    for (int j = 0; j < NU; ++j) g.u[j] = cp.ug_bt[cp.lUg.at(b, t, j)];
+}
+template <int DA, int NU, class T>
+PDDP_HD Goal<T, DA, NU> site_goal(const CostParams<T>& cp, int64_t b, int64_t t, bool terminal) {
+    Goal<T, DA, NU> g = problem_goal<DA, NU, T>(cp, b);
+    step_goal_x<DA, NU, T>(cp, b, t, g);
+    if (!terminal) step_goal_u<DA, NU, T>(cp, b, t, g);
+    return g;
+}
+template <int GEO, class T>
+PDDP_HD Goal<T, Geo<GEO>::DA, Geo<GEO>::NU> site_goal(const CostParams<T>& cp, int64_t b, int64_t t, bool terminal) {
+    return site_goal<Geo<GEO>::DA, Geo<GEO>::NU, T>(cp, b, t, terminal);
 }
 
 // ---- decoders (ref: utils/encoding.py:144-362) ----------------------------------------------

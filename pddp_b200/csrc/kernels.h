@@ -57,8 +57,8 @@ struct CostDerivArgs {
     Layout lZ, lU, lL, lLz, lLu, lLzz, lLuz, lLuu;
 };
 
-// pddp_cost (host, doubles) -> the kernels' CostParams; DA = the geometry's augmented state size (capi.cu)
-template <class T> void fill_cost(const pddp_cost* c, int DA, CostParams<T>& out);
+// pddp_cost (host, doubles) -> the kernels' CostParams, with the per-step goals' layouts from the shape (capi.cu)
+template <class T> void fill_cost(const pddp_cost* c, const pddp_shape* s, CostParams<T>& out);
 
 template <class T> cudaError_t linearize_known(int geo, int enc, const LinKnownArgs<T>&, cudaStream_t);
 template <class T> cudaError_t rollout_known(int geo, int enc, const RollKnownArgs<T>&, cudaStream_t);

@@ -61,14 +61,16 @@ __device__ __forceinline__ void cost_derivs_thread(const CostParams<T>& cp, cons
 // ------------------------------------------------------------------------------------------
 // linearise
 // ------------------------------------------------------------------------------------------
-template <class T, int GEO, int ENC>
+// STEP: the cost reads per-step goals (CostParams::xg_bt / ug_bt).  A separate instantiation, launched only when they
+// are given, so the shared and per-problem goals keep the code (and the registers) they had without them.
+template <class T, int GEO, int ENC, bool STEP>
 __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs<T> a) {
     typedef Geo<GEO> G;
     constexpr int D = G::D, NU = G::NU, NZ = enc_size(D, ENC);
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= a.B) return;
     if (a.active && a.active[b] != 1) return;   // 1 = (re)linearise, 2 = retry with the old one
-    const auto goal = problem_goal<GEO>(a.cost, b);
+    auto goal = problem_goal<GEO>(a.cost, b);
 
     T z[NZ];
 #pragma unroll
@@ -81,6 +83,7 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
         const bool terminal = t == a.N;
 #pragma unroll
         for (int e = 0; e < NZ; ++e) a.Z[a.lZ.at(b, t, e)] = z[e];
+        if (STEP) step_goal_x(a.cost, b, t, goal);
 
         // ---- cost (fused for IGNORE_UNCERTAINTY; the uncertain encodings run the
         //      (problem, time, Hessian-pair)-parallel cost_pairs_kernel on Z afterwards) ----
@@ -103,6 +106,7 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
         if (bounded) u = clampv(u, lo, hi);      // ref: ilqr.py:459-462, derivatives w.r.t. the clamped u
         if (a.U_clamped) a.U_clamped[a.lU.at(b, t, 0)] = u;
         if (ENC == ENC_IGNORE) {
+            if (STEP) step_goal_u(a.cost, b, t, goal);
             T la, lu, luu;
             cost_action(a.cost, goal.u[0], u, la, lu, luu);
             l += la;
@@ -156,11 +160,11 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
 //         wins outright like torch.argmin).
 // pass 2: the winning lane replays its rollout and stores Z_new / U_new.
 // ------------------------------------------------------------------------------------------
-template <class T, int GEO, int ENC, bool STORE>
+template <class T, int GEO, int ENC, bool STORE, bool STEP = false>
 __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha, bool bounded, T lo, T hi) {
     typedef Geo<GEO> G;
     constexpr int D = G::D, NZ = enc_size(D, ENC);
-    const auto goal = problem_goal<GEO>(a.cost, b);           // (dead in the STORE pass, which evaluates no cost)
+    auto goal = problem_goal<GEO>(a.cost, b);                 // (dead in the STORE pass, which evaluates no cost)
     T z[NZ];
 #pragma unroll
     for (int e = 0; e < NZ; ++e) z[e] = a.Z[a.lZ.at(b, 0, e)];
@@ -174,6 +178,9 @@ __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha,
     T* pZn = STORE ? a.Z_new + a.lZ.at(b, 0, 0) : nullptr;
     T* pUn = STORE ? a.U_new + a.lU.at(b, 0, 0) : nullptr;
     const int64_t seZ = a.lZ.se, seK = a.lK.se;
+    // per-step goals (NULL unless given): rows shared by the GA lanes of the problem, a broadcast load
+    const T* pXg = STEP && !STORE && a.cost.xg_bt ? a.cost.xg_bt + a.cost.lXg.at(b, 0, 0) : nullptr;
+    const T* pUg = STEP && !STORE && a.cost.ug_bt ? a.cost.ug_bt + a.cost.lUg.at(b, 0, 0) : nullptr;
     for (int t = 0; t < a.N; ++t) {
         T du = alpha * pk[0];
 #pragma unroll
@@ -190,6 +197,15 @@ __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha,
         StateTrig<GEO, T> tr;                               // shared by the cost and the dynamics of this step
         state_trig<GEO, T>(z, tr);
         if (!STORE) {
+            if (pXg) {
+#pragma unroll
+                for (int j = 0; j < G::DA; ++j) goal.x[j] = pXg[j * a.cost.lXg.se];
+                pXg += a.cost.lXg.st;
+            }
+            if (pUg) {
+                goal.u[0] = pUg[0];
+                pUg += a.cost.lUg.st;
+            }
             T la, lu, luu;
             cost_action(a.cost, goal.u[0], u, la, lu, luu);
             J += cost_state<GEO, ENC, T, T>(a.cost, goal.x, z, false, tr) + la;
@@ -204,6 +220,10 @@ __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha,
 #pragma unroll
         for (int e = 0; e < NZ; ++e) pZn[e * seZ] = z[e];
     } else {
+        if (pXg) {
+#pragma unroll
+            for (int j = 0; j < G::DA; ++j) goal.x[j] = pXg[j * a.cost.lXg.se];     // row N
+        }
         J += cost_state<GEO, ENC, T, T>(a.cost, goal.x, z, true);
     }
     return J;
@@ -211,7 +231,7 @@ __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha,
 
 // GA lanes = the alphas of one problem, 32/GA problems per warp (GA = 10: three problems on 30 lanes,
 // the reference's default line search has 10 alphas; GA = 16 / 32 for longer searches).
-template <class T, int GEO, int ENC, int GA>
+template <class T, int GEO, int ENC, int GA, bool STEP>
 __global__ void __launch_bounds__(128) rollout_known_kernel(const RollKnownArgs<T> a) {
     constexpr int GPW = 32 / GA;                           // problems per warp
     const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -223,7 +243,7 @@ __global__ void __launch_bounds__(128) rollout_known_kernel(const RollKnownArgs<
     T lo = bounded ? a.u_min[0] : T(0), hi = bounded ? a.u_max[0] : T(0);
     const bool has_alpha = live && lane < a.A;
     T alpha = has_alpha ? a.alphas[lane] : T(0);
-    T J = has_alpha ? roll_one<T, GEO, ENC, false>(a, b, alpha, bounded, lo, hi) : T(INFINITY);
+    T J = has_alpha ? roll_one<T, GEO, ENC, false, STEP>(a, b, alpha, bounded, lo, hi) : T(INFINITY);
     if (has_alpha) a.J_all[(int64_t)b * a.A + lane] = J;
 
     // argmin with torch semantics (NaN beats everything, ties -> lowest index): every lane scans
@@ -267,22 +287,31 @@ __global__ void __launch_bounds__(128) rollout_known_store_kernel(const RollKnow
 // ------------------------------------------------------------------------------------------
 template <class T, int GEO, int ENC>
 static cudaError_t launch_lin(const LinKnownArgs<T>& a, cudaStream_t s) {
-    const int threads = 128;
-    linearize_known_kernel<T, GEO, ENC><<<(a.B + threads - 1) / threads, threads, 0, s>>>(a);
+    const int threads = 128, grid = (a.B + threads - 1) / threads;
+    // (the uncertain encodings evaluate the cost in cost_pairs_kernel: their linearisation reads no goal)
+    if (ENC == ENC_IGNORE && (a.cost.xg_bt || a.cost.ug_bt))
+        linearize_known_kernel<T, GEO, ENC, ENC == ENC_IGNORE><<<grid, threads, 0, s>>>(a);
+    else
+        linearize_known_kernel<T, GEO, ENC, false><<<grid, threads, 0, s>>>(a);
     return cudaGetLastError();
 }
 template <class T, int GEO, int ENC>
 static cudaError_t launch_roll(const RollKnownArgs<T>& a, cudaStream_t s) {
     const int threads = 128;
-    if (a.A <= 10) {
+    if (a.cost.xg_bt || a.cost.ug_bt) {          // per-step goals: GA = 10 or 32 (no third instantiation for 16)
+        const int64_t total = a.A <= 10 ? ((int64_t)a.B + 2) / 3 * 32 : (int64_t)a.B * 32;
+        const unsigned grid = (unsigned)((total + threads - 1) / threads);
+        if (a.A <= 10) rollout_known_kernel<T, GEO, ENC, 10, true><<<grid, threads, 0, s>>>(a);
+        else rollout_known_kernel<T, GEO, ENC, 32, true><<<grid, threads, 0, s>>>(a);
+    } else if (a.A <= 10) {
         const int64_t total = ((int64_t)a.B + 2) / 3 * 32;
-        rollout_known_kernel<T, GEO, ENC, 10><<<(unsigned)((total + threads - 1) / threads), threads, 0, s>>>(a);
+        rollout_known_kernel<T, GEO, ENC, 10, false><<<(unsigned)((total + threads - 1) / threads), threads, 0, s>>>(a);
     } else if (a.A <= 16) {
         const int64_t total = (int64_t)a.B * 16;
-        rollout_known_kernel<T, GEO, ENC, 16><<<(unsigned)((total + threads - 1) / threads), threads, 0, s>>>(a);
+        rollout_known_kernel<T, GEO, ENC, 16, false><<<(unsigned)((total + threads - 1) / threads), threads, 0, s>>>(a);
     } else {
         const int64_t total = (int64_t)a.B * 32;
-        rollout_known_kernel<T, GEO, ENC, 32><<<(unsigned)((total + threads - 1) / threads), threads, 0, s>>>(a);
+        rollout_known_kernel<T, GEO, ENC, 32, false><<<(unsigned)((total + threads - 1) / threads), threads, 0, s>>>(a);
     }
     rollout_known_store_kernel<T, GEO, ENC><<<(a.B + threads - 1) / threads, threads, 0, s>>>(a);
     return cudaGetLastError();

@@ -158,7 +158,7 @@ __global__ void __launch_bounds__(64) lq_cost_kernel(const CostDerivArgs<T> a) {
     for (int e = 0; e < NZ; ++e) z[e] = a.Z[a.lZ.at(b, t, e)];
     if (t < a.N)
         for (int i = 0; i < RNU; ++i) u[i] = a.U[a.lU.at(b, t, i)];
-    lq_cost_site<T, ENC>(a, problem_goal<RD, RNU>(a.cost, b), b, t, z, u, t == a.N);
+    lq_cost_site<T, ENC>(a, site_goal<RD, RNU>(a.cost, b, t, t == a.N), b, t, z, u, t == a.N);
 }
 template <class T>
 __global__ void lq_cost_sum_kernel(const CostDerivArgs<T> a) {
@@ -173,7 +173,8 @@ __global__ void lq_cost_sum_kernel(const CostDerivArgs<T> a) {
 // ------------------------------------------------------------------------------------------
 // linearise: thread = problem
 // ------------------------------------------------------------------------------------------
-template <class T, int ENC>
+// STEP: per-step goals (CostParams::xg_bt / ug_bt); a separate instantiation, launched only when they are given
+template <class T, int ENC, bool STEP>
 __global__ void __launch_bounds__(64) lq_linearize_kernel(const LinKnownArgs<T> a) {
     constexpr int D = RD, NU = RNU, NZ = enc_size(D, ENC);
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -181,7 +182,7 @@ __global__ void __launch_bounds__(64) lq_linearize_kernel(const LinKnownArgs<T> 
     if (a.active && a.active[b] != 1) return;
     const RdvModel<T> md = rdv_model(a.dyn);
     const bool bounded = a.u_min != nullptr && a.u_max != nullptr;
-    const auto goal = problem_goal<RD, RNU>(a.cost, b);
+    auto goal = problem_goal<RD, RNU>(a.cost, b);
     T z[NZ], zn[NZ];
     for (int e = 0; e < NZ; ++e) z[e] = a.z0[(int64_t)b * NZ + e];
     T J = T(0);
@@ -191,7 +192,9 @@ __global__ void __launch_bounds__(64) lq_linearize_kernel(const LinKnownArgs<T> 
         for (int e = 0; e < NZ; ++e) a.Z[a.lZ.at(b, t, e)] = z[e];
         // ---- cost: value, gradient, Hessian (closed form) ----
         T u[NU];
+        if (STEP) step_goal_x(a.cost, b, t, goal);
         if (!terminal) {
+            if (STEP) step_goal_u(a.cost, b, t, goal);
 #pragma unroll
             for (int i = 0; i < NU; ++i) {
                 u[i] = a.U[a.lU.at(b, t, i)];
@@ -244,12 +247,12 @@ __global__ void __launch_bounds__(64) lq_linearize_kernel(const LinKnownArgs<T> 
 // ------------------------------------------------------------------------------------------
 // rollout of one (problem, alpha)   ref: ilqr.py:677-723 + 764-791
 // ------------------------------------------------------------------------------------------
-template <class T, int ENC, bool STORE>
+template <class T, int ENC, bool STORE, bool STEP = false>
 __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alpha) {
     constexpr int D = RD, NU = RNU, NZ = enc_size(D, ENC);
     const RdvModel<T> md = rdv_model(a.dyn);
     const bool bounded = a.u_min != nullptr && a.u_max != nullptr;
-    const auto goal = problem_goal<RD, RNU>(a.cost, b);     // (dead in the STORE pass, which evaluates no cost)
+    auto goal = problem_goal<RD, RNU>(a.cost, b);           // (dead in the STORE pass, which evaluates no cost)
     T z[NZ], zn[NZ];
     for (int e = 0; e < NZ; ++e) z[e] = a.Z[a.lZ.at(b, 0, e)];
     T J = T(0);
@@ -261,6 +264,9 @@ __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alp
     T* pZn = STORE ? a.Z_new + a.lZ.at(b, 0, 0) : nullptr;
     T* pUn = STORE ? a.U_new + a.lU.at(b, 0, 0) : nullptr;
     const int64_t seZ = a.lZ.se, seK = a.lK.se, sek = a.lk.se, seU = a.lU.se;
+    // per-step goals (NULL unless given), advanced like the step records
+    const T* pXg = STEP && !STORE && a.cost.xg_bt ? a.cost.xg_bt + a.cost.lXg.at(b, 0, 0) : nullptr;
+    const T* pUg = STEP && !STORE && a.cost.ug_bt ? a.cost.ug_bt + a.cost.lUg.at(b, 0, 0) : nullptr;
     for (int t = 0; t < a.N; ++t) {
         T u[NU];
 #pragma unroll
@@ -282,6 +288,16 @@ __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alp
             for (int i = 0; i < NU; ++i) pUn[i * seU] = u[i];
             pZn += a.lZ.st; pUn += a.lU.st;
         } else {
+            if (pXg) {
+#pragma unroll
+                for (int j = 0; j < D; ++j) goal.x[j] = pXg[j * a.cost.lXg.se];
+                pXg += a.cost.lXg.st;
+            }
+            if (pUg) {
+#pragma unroll
+                for (int i = 0; i < NU; ++i) goal.u[i] = pUg[i * a.cost.lUg.se];
+                pUg += a.cost.lUg.st;
+            }
             J += rdv_cost_state<ENC, T>(a.cost, goal.x, z, false) + rdv_cost_action(a.cost, goal.u, u);
         }
         rdv_mean_step(md, z, u, zn);
@@ -292,18 +308,22 @@ __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alp
     if (STORE) {
         for (int e = 0; e < NZ; ++e) pZn[e * seZ] = z[e];
     } else {
+        if (pXg) {
+#pragma unroll
+            for (int j = 0; j < D; ++j) goal.x[j] = pXg[j * a.cost.lXg.se];         // row N
+        }
         J += rdv_cost_state<ENC, T>(a.cost, goal.x, z, true);
     }
     return J;
 }
 
-template <class T, int ENC>
+template <class T, int ENC, bool STEP>
 __global__ void __launch_bounds__(64) lq_rollout_kernel(const RollKnownArgs<T> a) {
     const int64_t id = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (id >= (int64_t)a.B * a.A) return;
     const int b = (int)(id / a.A), al = (int)(id - (int64_t)b * a.A);
     if ((a.active && a.active[b] == 0) || (a.bw_status && a.bw_status[b] != 0)) return;
-    a.J_all[id] = lq_roll_one<T, ENC, false>(a, b, a.alphas[al]);
+    a.J_all[id] = lq_roll_one<T, ENC, false, STEP>(a, b, a.alphas[al]);
 }
 
 // argmin with torch semantics (first minimum; a NaN wins outright) + the winner's trajectory
@@ -330,14 +350,18 @@ __global__ void __launch_bounds__(64) lq_select_store_kernel(const RollKnownArgs
 template <class T>
 cudaError_t linearize_lq(int enc, const LinKnownArgs<T>& a, cudaStream_t s) {
     const int th = 64, grid = (a.B + th - 1) / th;
+    const bool step = a.cost.xg_bt || a.cost.ug_bt;
+#define LQ_LIN(E) if (step) lq_linearize_kernel<T, E, true><<<grid, th, 0, s>>>(a); \
+                  else lq_linearize_kernel<T, E, false><<<grid, th, 0, s>>>(a); break;
     switch (enc) {
-        case ENC_FULL: lq_linearize_kernel<T, ENC_FULL><<<grid, th, 0, s>>>(a); break;
-        case ENC_UT: lq_linearize_kernel<T, ENC_UT><<<grid, th, 0, s>>>(a); break;
-        case ENC_VAR: lq_linearize_kernel<T, ENC_VAR><<<grid, th, 0, s>>>(a); break;
-        case ENC_STD: lq_linearize_kernel<T, ENC_STD><<<grid, th, 0, s>>>(a); break;
-        case ENC_IGNORE: lq_linearize_kernel<T, ENC_IGNORE><<<grid, th, 0, s>>>(a); break;
+        case ENC_FULL: LQ_LIN(ENC_FULL)
+        case ENC_UT: LQ_LIN(ENC_UT)
+        case ENC_VAR: LQ_LIN(ENC_VAR)
+        case ENC_STD: LQ_LIN(ENC_STD)
+        case ENC_IGNORE: LQ_LIN(ENC_IGNORE)
         default: return cudaErrorInvalidValue;
     }
+#undef LQ_LIN
     return cudaGetLastError();
 }
 
@@ -383,7 +407,10 @@ template <class T>
 cudaError_t rollout_lq(int enc, const RollKnownArgs<T>& a, cudaStream_t s) {
     const int th = 64;
     const unsigned g1 = (unsigned)(((int64_t)a.B * a.A + th - 1) / th), g2 = (a.B + th - 1) / th;
-#define LQ_ROLL(E) lq_rollout_kernel<T, E><<<g1, th, 0, s>>>(a); lq_select_store_kernel<T, E><<<g2, th, 0, s>>>(a); break;
+    const bool step = a.cost.xg_bt || a.cost.ug_bt;
+#define LQ_ROLL(E) if (step) lq_rollout_kernel<T, E, true><<<g1, th, 0, s>>>(a); \
+                   else lq_rollout_kernel<T, E, false><<<g1, th, 0, s>>>(a); \
+                   lq_select_store_kernel<T, E><<<g2, th, 0, s>>>(a); break;
     switch (enc) {
         case ENC_FULL: LQ_ROLL(ENC_FULL)
         case ENC_UT: LQ_ROLL(ENC_UT)

@@ -221,7 +221,7 @@ __global__ void __launch_bounds__(128) cost_pairs_kernel(const CostDerivArgs<T> 
         while (p >= NZ - i) { p -= NZ - i; ++i; }
         j = i + p;
     }
-    const auto goal = problem_goal<GEO>(a.cost, b);
+    const auto goal = site_goal<GEO>(a.cost, b, t, terminal);
     typedef Jet2<T, 2> S;
     S zj[NZ];
 #pragma unroll

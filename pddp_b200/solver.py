@@ -119,21 +119,37 @@ class BNNDynamics:
         return s
 
 
-def check_goals(x_goal, u_goal, B, geo, dtype):
-    """Per-problem goals as the kernels read them: x_goal [B, DA] on the angle-augmented state, u_goal [B, nu], CUDA
-    tensors, cast to the solver dtype (None stays None).  Raises before anything is launched."""
+def check_goal_shapes(x_goal, u_goal, B, geo, N=None):
+    """The shape rules of per-problem and per-step goals; raises ValueError on any other shape.  x_goal is [B, DA] on
+    the angle-augmented state, or with N given also [B, N+1, DA] (row t = the goal of the state at step t, row N the
+    terminal one); u_goal is [B, nu], or with N given [B, N, nu].  Returns, for x and u, whether the goal is per step
+    (None where no goal is given)."""
     D, nu, ang, _ = _lib.GEO_INFO[geo]
     out = []
-    for name, g, E in (("x_goal", x_goal, D + len(ang)), ("u_goal", u_goal, nu)):
+    for name, g, E, Nt in (("x_goal", x_goal, D + len(ang), None if N is None else N + 1),
+                           ("u_goal", u_goal, nu, N)):
         if g is None:
             out.append(None)
-            continue
-        if not isinstance(g, torch.Tensor) or not g.is_cuda:
-            raise RuntimeError("pddp_b200: per-problem %s must be a CUDA tensor (no CPU fallback)" % name)
-        if tuple(g.shape) != (B, E):
+        elif tuple(g.shape) == (B, E):
+            out.append(False)
+        elif Nt is not None and tuple(g.shape) == (B, Nt, E):
+            out.append(True)
+        elif Nt is None:
             raise ValueError("per-problem %s must have shape [B, %d] = [%d, %d], got %s" % (name, E, B, E, list(g.shape)))
-        out.append(g.detach().to(dtype))
+        else:
+            raise ValueError("%s must have shape [B, %d] = [%d, %d] (per problem) or [B, %d, %d] = [%d, %d, %d] (per "
+                             "step), got %s" % (name, E, B, E, Nt, E, B, Nt, E, list(g.shape)))
     return out
+
+
+def check_goals(x_goal, u_goal, B, geo, dtype, N=None):
+    """Per-problem (and, with N given, per-step) goals as the kernels read them -- shapes as in check_goal_shapes --
+    CUDA tensors, cast to the solver dtype (None stays None).  Raises before anything is launched."""
+    for name, g in (("x_goal", x_goal), ("u_goal", u_goal)):
+        if g is not None and (not isinstance(g, torch.Tensor) or not g.is_cuda):
+            raise RuntimeError("pddp_b200: per-problem %s must be a CUDA tensor (no CPU fallback)" % name)
+    check_goal_shapes(x_goal, u_goal, B, geo, N)
+    return [None if g is None else g.detach().to(dtype) for g in (x_goal, u_goal)]
 
 
 class QRCostConstants:
@@ -214,8 +230,10 @@ class BatchedSolver:
         self.roll_status = torch.zeros(self.B, dtype=torch.int32, **o)
         self.n_active = torch.zeros(1, dtype=torch.int32, **o)
         self.u_min = self.u_max = None
-        self.goals = {}            # per-problem goal buffers ("x_goal" [B, DA], "u_goal" [B, nu]), made on first use
-        self._goal_ptrs = (None, None)
+        # goal buffers, made on first use: per problem "x_goal" [B, DA], "u_goal" [B, nu]; per step "x_goal_t"
+        # [B, N+1, DA], "u_goal_t" [B, N, nu] in the solver's layout (view / store like the buffers above)
+        self.goals = {}
+        self._goal_ptrs = (None, None, None, None)       # x_goal_b, u_goal_b, x_goal_bt, u_goal_bt
         self.alphas = fit_alphas(dtype, self.device)
         self.launches = 0          # CUDA kernels enqueued by this solver (bench.py reports it)
         self.workspace = None
@@ -240,7 +258,7 @@ class BatchedSolver:
 
     def view(self, name):
         """[B, Nt, E] view of a buffer whatever the internal layout."""
-        t = self.buf[name]
+        t = self.buf[name] if name in self.buf else self.goals[name]
         return t.permute(2, 0, 1) if self.layout == _lib.BATCH_INNER else t
 
     def store(self, name, value):
@@ -262,22 +280,30 @@ class BatchedSolver:
     # ---------------------------------------------------------------- setup
     def set_goals(self, x_goal=None, u_goal=None):
         """Gives every problem its own goal: x_goal [B, DA] in the cost's coordinates (the angle-augmented state,
-        like QRCost.x_goal), u_goal [B, nu].  A goal left None is the cost's own, shared by every problem."""
-        goals = check_goals(x_goal, u_goal, self.B, self.geo, self.dtype)
-        ptrs = []
-        for name, g in zip(("x_goal", "u_goal"), goals):
+        like QRCost.x_goal), u_goal [B, nu]; or a goal per problem and step, to track a reference: x_goal
+        [B, N+1, DA] (row N goes with Q_term), u_goal [B, N, nu].  x and u choose their form independently.  A goal
+        left None is the cost's own, shared by every problem; setting goals clears the ones set before."""
+        goals = check_goals(x_goal, u_goal, self.B, self.geo, self.dtype, self.N)
+        ptrs = [None] * 4
+        for i, (name, g) in enumerate(zip(("x_goal", "u_goal"), goals)):
             if g is None:
-                ptrs.append(None)
                 continue
-            if name not in self.goals:
-                self.goals[name] = torch.empty(g.shape, dtype=self.dtype, device=self.device)
-            self.goals[name].copy_(g)
-            ptrs.append(self.goals[name].data_ptr())
+            if g.dim() == 3:
+                name, i = name + "_t", i + 2
+                if name not in self.goals:
+                    self.goals[name] = self._alloc(g.shape[1], g.shape[2])
+                self.store(name, g)
+            else:
+                if name not in self.goals:
+                    self.goals[name] = torch.empty(g.shape, dtype=self.dtype, device=self.device)
+                self.goals[name].copy_(g)
+            ptrs[i] = self.goals[name].data_ptr()
         self._goal_ptrs = tuple(ptrs)
 
     def _cost(self):
-        """The cost argument of a C ABI call, carrying this solver's per-problem goals (or NULL)."""
-        self.c_cost.x_goal_b, self.c_cost.u_goal_b = self._goal_ptrs
+        """The cost argument of a C ABI call, carrying this solver's per-problem / per-step goals (or NULL)."""
+        (self.c_cost.x_goal_b, self.c_cost.u_goal_b, self.c_cost.x_goal_bt,
+         self.c_cost.u_goal_bt) = self._goal_ptrs
         return C.byref(self.c_cost)
 
     def set_problem(self, z0, U, u_min=None, u_max=None, alphas=None, iterations=1, x_goal=None, u_goal=None):
@@ -389,7 +415,8 @@ class BatchedSolver:
         """Runs every problem until it has done `n_iterations` accepted steps or reached a
         terminal state (CONVERGED / MAX_REG), exactly like B sequential reference `fit` calls
         (ref: ilqr.py:237-316); rejected / not-PD attempts retry with a larger mu and do not
-        consume iterations (ref: ilqr.py:213).  x_goal [B, DA] / u_goal [B, nu]: per-problem goals (set_goals)."""
+        consume iterations (ref: ilqr.py:213).  x_goal [B, DA] or [B, N+1, DA] / u_goal [B, nu] or [B, N, nu]:
+        per-problem or per-step goals (set_goals)."""
         self.set_problem(z0, U, u_min, u_max, alphas, iterations=n_iterations, x_goal=x_goal, u_goal=u_goal)
         passes = 0
         limit = max_passes if max_passes is not None else n_iterations * 64
