@@ -103,9 +103,14 @@ typedef struct pddp_cost {
 
 /* Known-dynamics constants (host memory). p[] = pendulum: dt,m,l,mu,g ; cartpole: dt,mc,mp,l,mu,g ;
  * double cartpole: dt,mc,mp1,mp2,l1,l2,mu,g ; rendezvous: dt,m,alpha.
- * Replaces: pddp/examples/<problem>/model.py constructor Parameters. */
+ * Replaces: pddp/examples/<problem>/model.py constructor Parameters.
+ * p_b gives every problem of the batch its own system, to solve a family of systems (parameter sweeps, domain
+ * randomisation) in one batch: row b of p_b [B, 8] holds problem b's parameters in the p[] order above (trailing
+ * entries unused).  pddp_linearize_known, pddp_rollout_known and pddp_env_step_known (row b = instance b) read it.
+ * A zero-initialised p_b (NULL) gives every problem the system p[]. */
 typedef struct pddp_known_dynamics {
     double p[8];
+    const void* p_b;   /* [B, 8] device, shape.dtype, row-major whatever shape.layout; NULL = p[] above */
 } pddp_known_dynamics;
 
 /* Input particles of step i (pddp/models/bnn/modules.py:320-358):

@@ -47,6 +47,12 @@ class KnownDynamics(C.Structure):
     _fields_ = [("p", C.c_double * 8)]
 
 
+class KnownDynamicsBatch(KnownDynamics):
+    """The whole pddp_known_dynamics: the shared constants above plus p_b, the device pointer of per-problem
+    parameters [B, 8] (NULL = p for every problem).  The C entry points take this type."""
+    _fields_ = [("p_b", C.c_void_p)]
+
+
 class BNN(C.Structure):
     _fields_ = [("P", C.c_int32), ("H0", C.c_int32), ("H1", C.c_int32)] + [
         (n, C.c_void_p) for n in ("W0", "b0", "W1", "b1", "W2", "b2", "mask0", "mask1", "eps0",
@@ -58,10 +64,10 @@ _P = C.c_void_p
 _SIGNATURES = {
     "pddp_version": (C.c_char_p, []),
     "pddp_last_error": (C.c_char_p, []),
-    "pddp_linearize_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamics), C.POINTER(CostGoals)]
+    "pddp_linearize_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamicsBatch), C.POINTER(CostGoals)]
                              + [_P] * 17),
     "pddp_backward": (C.c_int, [C.POINTER(Shape)] + [_P] * 16),
-    "pddp_rollout_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamics), C.POINTER(CostGoals)]
+    "pddp_rollout_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamicsBatch), C.POINTER(CostGoals)]
                            + [_P] * 5 + [C.c_int32] + [_P] * 10),
     "pddp_accept_update": (C.c_int, [C.POINTER(Shape)] + [_P] * 4 + [C.c_double, C.c_double]
                            + [_P] * 13),
@@ -73,7 +79,7 @@ _SIGNATURES = {
                          + [C.c_int32] + [_P] * 10 + [_P, C.c_int64, _P]),
     "pddp_bnn_train_workspace_bytes": (C.c_int64, [_P]),
     "pddp_bnn_train": (C.c_int, [_P] * 12 + [_P, C.c_int64, _P]),
-    "pddp_env_step_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamics)] + [_P] * 4),
+    "pddp_env_step_known": (C.c_int, [C.POINTER(Shape), C.POINTER(KnownDynamicsBatch)] + [_P] * 4),
     "pddp_profile_enable": (None, [C.c_int]),
     "pddp_profile_read": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "pddp_launch_count": (C.c_int64, []),

@@ -15,7 +15,8 @@ import torch
 
 from .. import _lib, sharding
 from ..models.bnn.modules import check_model_opts
-from ..solver import LIN_NAMES, cached_solver, check_goals, expand_bound, fit_alphas, step_alphas
+from ..solver import (LIN_NAMES, cached_solver, check_dynamics_rows, check_goals, expand_bound, fit_alphas,
+                      require_single_system, step_alphas)
 from ..utils.encoding import StateEncoding, decode_mean
 from .base import Controller
 
@@ -100,12 +101,15 @@ class iLQRController(Controller):
         """Drops the device buffers (and the device copies of the model they captured)."""
         self._solver = None
 
-    def _get_solver(self, B, N, encoding, dtype, device, n_alphas):
+    def _get_solver(self, B, N, encoding, dtype, device, n_alphas, problems=None):
         """Buffers for this problem shape.  The cache is keyed on the model's `_version` (bumped by
         resample / fit / load_reference), and the cost / closed-form model constants are re-read on every call,
-        so an edited model or cost is never served from stale device copies."""
+        so an edited model or cost is never served from stale device copies.  problems = (lo, hi): the rows of a
+        closed-form model's per-problem parameters that this shard solves."""
+        if not self._batched:
+            require_single_system(self.model, "a single-problem call (U [N, nu])")
         s = cached_solver(self.model, self.cost, encoding, B, N, dtype, device, max_alphas=max(16, n_alphas),
-                          model_opts=self._model_opts)
+                          model_opts=self._model_opts, problems=problems)
         if s is not self._solver:
             s.view("K_nominal").zero_()
         self._solver = s
@@ -173,7 +177,11 @@ class iLQRController(Controller):
         u_goal [B, nu], CUDA tensors.  Per-step goals track a reference: x_goal [B, N+1, DA] (row t = the goal of the
         state at step t, row N with Q_term), u_goal [B, N, nu]; a single problem (U [N, nu]) takes them as
         [N+1, DA] / [N, nu].  x and u choose their form independently; a goal not given is the cost's x_goal /
-        u_goal.  A sharded fit splits them like z0."""
+        u_goal.  A sharded fit splits them like z0.
+
+        Per-problem dynamics (batched calls): a closed-form model whose parameters are 1-D tensors of length B solves
+        problem b with parameter set b (KnownDynamicsModel); a sharded fit splits the sets like z0.  A single
+        problem needs a model with one set."""
         _lib.require_cuda(U, "U")
         x_goal, u_goal = batch_goals(U.dim() == 3, U.shape[-2], x_goal, u_goal)
         self._batched = U.dim() == 3
@@ -186,10 +194,14 @@ class iLQRController(Controller):
         sharded = self._batched and world > 1 and shard is not False and Ub.shape[0] >= world
         B_total = Ub.shape[0]
         x_goal, u_goal = check_goals(x_goal, u_goal, B_total, self.cost.geometry(), U.dtype, Ub.shape[1])
+        problems = None
         if sharded:
             Ub, zb = sharding.shard(Ub, world, rank).contiguous(), sharding.shard(zb, world, rank).contiguous()
             x_goal, u_goal = (None if g is None else sharding.shard(g, world, rank).contiguous() for g in (x_goal, u_goal))
-        s = self._get_solver(Ub.shape[0], Ub.shape[1], encoding, U.dtype, U.device, 10)
+            if not getattr(self.model, "is_bnn", False):
+                check_dynamics_rows(self.model.descriptor(), B_total)
+                problems = sharding.shard_bounds(B_total, world, rank)      # per-problem parameters split like z0
+        s = self._get_solver(Ub.shape[0], Ub.shape[1], encoding, U.dtype, U.device, 10, problems)
         it = [0]
 
         def on_pass(p, sv):
@@ -256,8 +268,10 @@ class iLQRController(Controller):
 # ---------------------------------------------------------------------------------------------
 def forward(z0, U, model, cost, encoding=StateEncoding.DEFAULT, batch_rollout=True, model_opts={}, cost_opts={},
             u_min=None, u_max=None):
-    """ref: pddp/controllers/ilqr.py:393-486 -> (Z, F_z, F_u, L, L_z, L_u, L_zz, L_uz, L_uu)."""
+    """ref: pddp/controllers/ilqr.py:393-486 -> (Z, F_z, F_u, L, L_z, L_u, L_zz, L_uz, L_uu).  One problem, so one
+    system: a model with several parameter sets raises ValueError."""
     check_model_opts(model, model_opts)
+    require_single_system(model, "pddp_b200.controllers.ilqr.forward")
     _lib.require_cuda(U, "U")
     u_min, u_max = _bounds(u_min, u_max)
     s = cached_solver(model, cost, encoding, 1, U.shape[0], U.dtype, U.device, model_opts=model_opts)
@@ -328,8 +342,10 @@ def _control_law(model, Z, U, k, K, alpha, encoding=StateEncoding.DEFAULT, model
                  cost=None):
     """ref: pddp/controllers/ilqr.py:677-723 -> (Z_new [N+1, A, nz], U_new [N, A, nu]) for every
     alpha (the fused kernel only keeps the winner's trajectory, so this reference-shaped wrapper rolls the A
-    candidates as A problems of a batch with one alpha each)."""
+    candidates as A problems of a batch with one alpha each).  One trajectory, so one system: a model with several
+    parameter sets raises ValueError (the candidates are rolled as a batch, whose rows are not systems)."""
     check_model_opts(model, model_opts)
+    require_single_system(model, "_control_law (its line-search candidates are rolled as the problems of one batch)")
     u_min, u_max = _bounds(u_min, u_max)
     alpha = torch.as_tensor(alpha).reshape(-1)
     s = cached_solver(model, cost, encoding, 1, U.shape[0], U.dtype, U.device, model_opts=model_opts)

@@ -91,6 +91,7 @@ static int linearize_known_t(const pddp_shape* s, const pddp_known_dynamics* dyn
     a.B = s->B; a.N = s->N;
     fill_cost(cost, s, a.cost);
     for (int i = 0; i < 8; ++i) a.dyn.p[i] = (T)dyn->p[i];
+    a.p_b = (const T*)dyn->p_b;
     a.z0 = (const T*)z0; a.U = (const T*)U; a.u_min = (const T*)u_min; a.u_max = (const T*)u_max;
     a.active = active;
     a.Z = (T*)Z; a.F_z = (T*)F_z; a.F_u = (T*)F_u; a.L = (T*)L; a.L_z = (T*)L_z; a.L_u = (T*)L_u;
@@ -151,9 +152,11 @@ static int env_step_t(const pddp_shape* s, const pddp_known_dynamics* dyn, const
                       cudaStream_t st) {
     KnownParams<T> kp;
     for (int i = 0; i < 8; ++i) kp.p[i] = (T)dyn->p[i];
+    const T* p_b = (const T*)dyn->p_b;
     note_launches(1);
-    if (s->geo == GEO_RENDEZVOUS) return cuda_result(env_step_lq<T>(s->B, kp, (const T*)x, (const T*)u, (T*)xn, st), "pddp_env_step_known");
-    return cuda_result(env_step_known<T>(s->geo, s->B, kp, (const T*)x, (const T*)u, (T*)xn, st), "pddp_env_step_known");
+    if (s->geo == GEO_RENDEZVOUS)
+        return cuda_result(env_step_lq<T>(s->B, kp, p_b, (const T*)x, (const T*)u, (T*)xn, st), "pddp_env_step_known");
+    return cuda_result(env_step_known<T>(s->geo, s->B, kp, p_b, (const T*)x, (const T*)u, (T*)xn, st), "pddp_env_step_known");
 }
 
 extern "C" int pddp_env_step_known(const pddp_shape* s, const pddp_known_dynamics* dyn, const void* x, const void* u,
@@ -218,6 +221,7 @@ static int rollout_known_t(const pddp_shape* s, const pddp_known_dynamics* dyn, 
     a.B = s->B; a.N = s->N; a.A = A;
     fill_cost(cost, s, a.cost);
     for (int i = 0; i < 8; ++i) a.dyn.p[i] = (T)dyn->p[i];
+    a.p_b = (const T*)dyn->p_b;
     a.Z = (const T*)Z; a.U = (const T*)U; a.k = (const T*)k; a.K = (const T*)K; a.alphas = (const T*)alphas;
     a.u_min = (const T*)u_min; a.u_max = (const T*)u_max; a.active = active; a.bw_status = bw_status;
     a.J_all = (T*)J_all; a.amin = amin; a.J_new = (T*)J_new; a.Z_new = (T*)Z_new; a.U_new = (T*)U_new;

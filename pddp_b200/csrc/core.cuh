@@ -296,6 +296,21 @@ PDDP_HD void cost_action(const CostParams<T>& cp, T ug, T u, T& l, T& l_u, T& l_
 template <class T>
 struct KnownParams { T p[8]; };   // pendulum: dt,m,l,mu,g | cartpole: dt,mc,mp,l,mu,g | double: dt,mc,mp1,mp2,l1,l2,mu,g
 
+// Per-problem parameters (PB): row b of p_b [B, 8] replaces the shared p[].  Loaded ONCE per kernel, before the time
+// loop, into the same struct, so the step functions below run unchanged; only the geometry's own parameters are read
+// (the pendulum's 5, the rendezvous' 3).  PB is a separate instantiation, launched only when p_b is given, so the shared
+// path keeps reading its parameters as constant-bank operands.
+PDDP_HD constexpr int known_nparams(int geo) {
+    return geo == GEO_PENDULUM ? 5 : geo == GEO_CARTPOLE ? 6 : geo == GEO_DOUBLE_CARTPOLE ? 8 : 3;
+}
+template <int GEO, class T>
+PDDP_HD KnownParams<T> problem_params(const T* p_b, int64_t b) {
+    KnownParams<T> kp;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) kp.p[i] = i < known_nparams(GEO) ? p_b[b * 8 + i] : T(0);
+    return kp;
+}
+
 template <int GEO, class T, class S>
 PDDP_HD void known_mean_step(const KnownParams<T>& kp, const S* x, const S& u, S* xn, const StateTrig<GEO, S>& tr) {
     const T* p = kp.p;

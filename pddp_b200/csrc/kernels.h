@@ -15,6 +15,7 @@ struct LinKnownArgs {
     T* U_clamped;   // scratch [B,N,nu] (same layout as U) for the separate cost pass, or NULL
     int32_t* status;
     Layout lZ, lU, lFz, lFu, lL, lLz, lLu, lLzz, lLuz, lLuu;
+    const T* p_b;   // [B, 8] per-problem dynamics parameters, or NULL: dyn (pddp_known_dynamics::p_b)
 };
 
 template <class T>
@@ -26,6 +27,7 @@ struct RollKnownArgs {
     const int32_t* active; const int32_t* bw_status;
     T* J_all; int32_t* amin; T* J_new; T* Z_new; T* U_new;
     Layout lZ, lU, lk, lK;
+    const T* p_b;   // [B, 8] per-problem dynamics parameters, or NULL: dyn
 };
 
 template <class T>
@@ -62,8 +64,10 @@ template <class T> void fill_cost(const pddp_cost* c, const pddp_shape* s, CostP
 
 template <class T> cudaError_t linearize_known(int geo, int enc, const LinKnownArgs<T>&, cudaStream_t);
 template <class T> cudaError_t rollout_known(int geo, int enc, const RollKnownArgs<T>&, cudaStream_t);
-template <class T> cudaError_t env_step_known(int geo, int B, const KnownParams<T>&, const T* x, const T* u, T* xn, cudaStream_t);
-template <class T> cudaError_t env_step_lq(int B, const KnownParams<T>&, const T* x, const T* u, T* xn, cudaStream_t);
+// p_b: [B, 8] parameters of every instance, or NULL: the shared ones
+template <class T> cudaError_t env_step_known(int geo, int B, const KnownParams<T>&, const T* p_b, const T* x, const T* u, T* xn,
+                                              cudaStream_t);
+template <class T> cudaError_t env_step_lq(int B, const KnownParams<T>&, const T* p_b, const T* x, const T* u, T* xn, cudaStream_t);
 template <class T> cudaError_t linearize_lq(int enc, const LinKnownArgs<T>&, cudaStream_t);      // known_lq.cu (rendezvous)
 template <class T> cudaError_t rollout_lq(int enc, const RollKnownArgs<T>&, cudaStream_t);
 template <class T> cudaError_t cost_derivatives_lq(int enc, const CostDerivArgs<T>&, cudaStream_t);

@@ -63,7 +63,8 @@ __device__ __forceinline__ void cost_derivs_thread(const CostParams<T>& cp, cons
 // ------------------------------------------------------------------------------------------
 // STEP: the cost reads per-step goals (CostParams::xg_bt / ug_bt).  A separate instantiation, launched only when they
 // are given, so the shared and per-problem goals keep the code (and the registers) they had without them.
-template <class T, int GEO, int ENC, bool STEP>
+// PB: the dynamics read problem b's row of p_b (per-problem parameters), likewise a separate instantiation.
+template <class T, int GEO, int ENC, bool STEP, bool PB>
 __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs<T> a) {
     typedef Geo<GEO> G;
     constexpr int D = G::D, NU = G::NU, NZ = enc_size(D, ENC);
@@ -71,6 +72,9 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
     if (b >= a.B) return;
     if (a.active && a.active[b] != 1) return;   // 1 = (re)linearise, 2 = retry with the old one
     auto goal = problem_goal<GEO>(a.cost, b);
+    KnownParams<T> pb;
+    if (PB) pb = problem_params<GEO>(a.p_b, b);
+    const KnownParams<T>& dyn = PB ? pb : a.dyn;
 
     T z[NZ];
 #pragma unroll
@@ -123,7 +127,7 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
         S1 x[D], xn[D], uj = S1::variable(u, D);
 #pragma unroll
         for (int i = 0; i < D; ++i) x[i] = S1::variable(z[i], i);
-        known_mean_step<GEO, T, S1>(a.dyn, x, uj, xn);
+        known_mean_step<GEO, T, S1>(dyn, x, uj, xn);
         T zn[NZ];
 #pragma unroll
         for (int i = 0; i < D; ++i) zn[i] = xn[i].v;
@@ -160,11 +164,15 @@ __global__ void __launch_bounds__(128) linearize_known_kernel(const LinKnownArgs
 //         wins outright like torch.argmin).
 // pass 2: the winning lane replays its rollout and stores Z_new / U_new.
 // ------------------------------------------------------------------------------------------
-template <class T, int GEO, int ENC, bool STORE, bool STEP = false>
+template <class T, int GEO, int ENC, bool STORE, bool STEP = false, bool PB = false>
 __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha, bool bounded, T lo, T hi) {
     typedef Geo<GEO> G;
     constexpr int D = G::D, NZ = enc_size(D, ENC);
     auto goal = problem_goal<GEO>(a.cost, b);                 // (dead in the STORE pass, which evaluates no cost)
+    // per-problem parameters: the GA lanes of the problem read the same row, a broadcast load
+    KnownParams<T> pb;
+    if (PB) pb = problem_params<GEO>(a.p_b, b);
+    const KnownParams<T>& dyn = PB ? pb : a.dyn;
     T z[NZ];
 #pragma unroll
     for (int e = 0; e < NZ; ++e) z[e] = a.Z[a.lZ.at(b, 0, e)];
@@ -211,7 +219,7 @@ __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha,
             J += cost_state<GEO, ENC, T, T>(a.cost, goal.x, z, false, tr) + la;
         }
         T zn[NZ];
-        known_mean_step<GEO, T, T>(a.dyn, z, u, zn, tr);
+        known_mean_step<GEO, T, T>(dyn, z, u, zn, tr);
         known_uncertainty_step<D, ENC, T>(z, zn);
 #pragma unroll
         for (int e = 0; e < NZ; ++e) z[e] = zn[e];
@@ -231,7 +239,7 @@ __device__ __forceinline__ T roll_one(const RollKnownArgs<T>& a, int b, T alpha,
 
 // GA lanes = the alphas of one problem, 32/GA problems per warp (GA = 10: three problems on 30 lanes,
 // the reference's default line search has 10 alphas; GA = 16 / 32 for longer searches).
-template <class T, int GEO, int ENC, int GA, bool STEP>
+template <class T, int GEO, int ENC, int GA, bool STEP, bool PB = false>
 __global__ void __launch_bounds__(128) rollout_known_kernel(const RollKnownArgs<T> a) {
     constexpr int GPW = 32 / GA;                           // problems per warp
     const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -243,7 +251,7 @@ __global__ void __launch_bounds__(128) rollout_known_kernel(const RollKnownArgs<
     T lo = bounded ? a.u_min[0] : T(0), hi = bounded ? a.u_max[0] : T(0);
     const bool has_alpha = live && lane < a.A;
     T alpha = has_alpha ? a.alphas[lane] : T(0);
-    T J = has_alpha ? roll_one<T, GEO, ENC, false, STEP>(a, b, alpha, bounded, lo, hi) : T(INFINITY);
+    T J = has_alpha ? roll_one<T, GEO, ENC, false, STEP, PB>(a, b, alpha, bounded, lo, hi) : T(INFINITY);
     if (has_alpha) a.J_all[(int64_t)b * a.A + lane] = J;
 
     // argmin with torch semantics (NaN beats everything, ties -> lowest index): every lane scans
@@ -272,33 +280,52 @@ __global__ void __launch_bounds__(128) rollout_known_kernel(const RollKnownArgs<
 // inside the kernel above, only one lane of each alpha group would be busy: the same warp-level
 // instruction count as the all-alpha pass for 1/16 of the useful work.  Here every lane works, and
 // with the BATCH_INNER layout every store is a coalesced line.
-template <class T, int GEO, int ENC>
+template <class T, int GEO, int ENC, bool PB = false>
 __global__ void __launch_bounds__(128) rollout_known_store_kernel(const RollKnownArgs<T> a) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= a.B) return;
     if ((a.active && a.active[b] == 0) || (a.bw_status && a.bw_status[b] != 0)) return;
     const bool bounded = a.u_min != nullptr && a.u_max != nullptr;
     const T lo = bounded ? a.u_min[0] : T(0), hi = bounded ? a.u_max[0] : T(0);
-    roll_one<T, GEO, ENC, true>(a, b, a.alphas[a.amin[b]], bounded, lo, hi);
+    roll_one<T, GEO, ENC, true, false, PB>(a, b, a.alphas[a.amin[b]], bounded, lo, hi);
 }
 
 // ------------------------------------------------------------------------------------------
 // host dispatch
 // ------------------------------------------------------------------------------------------
-template <class T, int GEO, int ENC>
-static cudaError_t launch_lin(const LinKnownArgs<T>& a, cudaStream_t s) {
+template <class T, int GEO, int ENC, bool PB>
+static void launch_lin_pb(const LinKnownArgs<T>& a, cudaStream_t s) {
     const int threads = 128, grid = (a.B + threads - 1) / threads;
     // (the uncertain encodings evaluate the cost in cost_pairs_kernel: their linearisation reads no goal)
     if (ENC == ENC_IGNORE && (a.cost.xg_bt || a.cost.ug_bt))
-        linearize_known_kernel<T, GEO, ENC, ENC == ENC_IGNORE><<<grid, threads, 0, s>>>(a);
+        linearize_known_kernel<T, GEO, ENC, ENC == ENC_IGNORE, PB><<<grid, threads, 0, s>>>(a);
     else
-        linearize_known_kernel<T, GEO, ENC, false><<<grid, threads, 0, s>>>(a);
+        linearize_known_kernel<T, GEO, ENC, false, PB><<<grid, threads, 0, s>>>(a);
+}
+template <class T, int GEO, int ENC>
+static cudaError_t launch_lin(const LinKnownArgs<T>& a, cudaStream_t s) {
+    if (a.p_b) launch_lin_pb<T, GEO, ENC, true>(a, s);
+    else launch_lin_pb<T, GEO, ENC, false>(a, s);
     return cudaGetLastError();
 }
 template <class T, int GEO, int ENC>
 static cudaError_t launch_roll(const RollKnownArgs<T>& a, cudaStream_t s) {
     const int threads = 128;
-    if (a.cost.xg_bt || a.cost.ug_bt) {          // per-step goals: GA = 10 or 32 (no third instantiation for 16)
+    const bool step = a.cost.xg_bt || a.cost.ug_bt;
+    if (a.p_b) {                                 // per-problem parameters: GA = 10 or 32, with or without per-step goals
+        const int64_t total = a.A <= 10 ? ((int64_t)a.B + 2) / 3 * 32 : (int64_t)a.B * 32;
+        const unsigned grid = (unsigned)((total + threads - 1) / threads);
+        if (a.A <= 10) {
+            if (step) rollout_known_kernel<T, GEO, ENC, 10, true, true><<<grid, threads, 0, s>>>(a);
+            else rollout_known_kernel<T, GEO, ENC, 10, false, true><<<grid, threads, 0, s>>>(a);
+        } else {
+            if (step) rollout_known_kernel<T, GEO, ENC, 32, true, true><<<grid, threads, 0, s>>>(a);
+            else rollout_known_kernel<T, GEO, ENC, 32, false, true><<<grid, threads, 0, s>>>(a);
+        }
+        rollout_known_store_kernel<T, GEO, ENC, true><<<(a.B + threads - 1) / threads, threads, 0, s>>>(a);
+        return cudaGetLastError();
+    }
+    if (step) {                                  // per-step goals: GA = 10 or 32 (no third instantiation for 16)
         const int64_t total = a.A <= 10 ? ((int64_t)a.B + 2) / 3 * 32 : (int64_t)a.B * 32;
         const unsigned grid = (unsigned)((total + threads - 1) / threads);
         if (a.A <= 10) rollout_known_kernel<T, GEO, ENC, 10, true><<<grid, threads, 0, s>>>(a);
@@ -341,31 +368,41 @@ static cudaError_t launch_roll(const RollKnownArgs<T>& a, cudaStream_t s) {
 // ground-truth simulator step of the example environments, thread = environment instance
 // (ref: examples/*/env.py step(): x' = model(x, u, 0, IGNORE_UNCERTAINTY))
 // ------------------------------------------------------------------------------------------
-template <class T, int GEO>
-__global__ void __launch_bounds__(128) env_step_kernel(int B, KnownParams<T> dyn, const T* x, const T* u, T* xn) {
+// PB: instance b simulates the system of row b of p_b
+template <class T, int GEO, bool PB>
+__global__ void __launch_bounds__(128) env_step_kernel(int B, KnownParams<T> dyn, const T* p_b, const T* x, const T* u,
+                                                       T* xn) {
     constexpr int D = Geo<GEO>::D;
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
+    KnownParams<T> pb;
+    if (PB) pb = problem_params<GEO>(p_b, b);
     T xi[D], xo[D];
 #pragma unroll
     for (int i = 0; i < D; ++i) xi[i] = x[(int64_t)b * D + i];
-    known_mean_step<GEO, T, T>(dyn, xi, u[b], xo);
+    known_mean_step<GEO, T, T>(PB ? pb : dyn, xi, u[b], xo);
 #pragma unroll
     for (int i = 0; i < D; ++i) xn[(int64_t)b * D + i] = xo[i];
 }
-template <class T>
-cudaError_t env_step_known(int geo, int B, const KnownParams<T>& dyn, const T* x, const T* u, T* xn, cudaStream_t s) {
+template <class T, int GEO>
+static void launch_env_step(int B, const KnownParams<T>& dyn, const T* p_b, const T* x, const T* u, T* xn, cudaStream_t s) {
     const int th = 128, grid = (B + th - 1) / th;
+    if (p_b) env_step_kernel<T, GEO, true><<<grid, th, 0, s>>>(B, dyn, p_b, x, u, xn);
+    else env_step_kernel<T, GEO, false><<<grid, th, 0, s>>>(B, dyn, p_b, x, u, xn);
+}
+template <class T>
+cudaError_t env_step_known(int geo, int B, const KnownParams<T>& dyn, const T* p_b, const T* x, const T* u, T* xn,
+                           cudaStream_t s) {
     switch (geo) {
-        case GEO_PENDULUM: env_step_kernel<T, GEO_PENDULUM><<<grid, th, 0, s>>>(B, dyn, x, u, xn); break;
-        case GEO_CARTPOLE: env_step_kernel<T, GEO_CARTPOLE><<<grid, th, 0, s>>>(B, dyn, x, u, xn); break;
-        case GEO_DOUBLE_CARTPOLE: env_step_kernel<T, GEO_DOUBLE_CARTPOLE><<<grid, th, 0, s>>>(B, dyn, x, u, xn); break;
+        case GEO_PENDULUM: launch_env_step<T, GEO_PENDULUM>(B, dyn, p_b, x, u, xn, s); break;
+        case GEO_CARTPOLE: launch_env_step<T, GEO_CARTPOLE>(B, dyn, p_b, x, u, xn, s); break;
+        case GEO_DOUBLE_CARTPOLE: launch_env_step<T, GEO_DOUBLE_CARTPOLE>(B, dyn, p_b, x, u, xn, s); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
 }
 template cudaError_t env_step_known<PDDP_KNOWN_T>(int, int, const KnownParams<PDDP_KNOWN_T>&, const PDDP_KNOWN_T*,
-                                                  const PDDP_KNOWN_T*, PDDP_KNOWN_T*, cudaStream_t);
+                                                  const PDDP_KNOWN_T*, const PDDP_KNOWN_T*, PDDP_KNOWN_T*, cudaStream_t);
 
 template <class T>
 cudaError_t linearize_known(int geo, int enc, const LinKnownArgs<T>& a, cudaStream_t s) {

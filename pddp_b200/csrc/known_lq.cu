@@ -173,14 +173,15 @@ __global__ void lq_cost_sum_kernel(const CostDerivArgs<T> a) {
 // ------------------------------------------------------------------------------------------
 // linearise: thread = problem
 // ------------------------------------------------------------------------------------------
-// STEP: per-step goals (CostParams::xg_bt / ug_bt); a separate instantiation, launched only when they are given
-template <class T, int ENC, bool STEP>
+// STEP: per-step goals (CostParams::xg_bt / ug_bt); a separate instantiation, launched only when they are given.
+// PB: problem b's row of p_b (per-problem parameters) instead of dyn, likewise.
+template <class T, int ENC, bool STEP, bool PB>
 __global__ void __launch_bounds__(64) lq_linearize_kernel(const LinKnownArgs<T> a) {
     constexpr int D = RD, NU = RNU, NZ = enc_size(D, ENC);
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= a.B) return;
     if (a.active && a.active[b] != 1) return;
-    const RdvModel<T> md = rdv_model(a.dyn);
+    const RdvModel<T> md = rdv_model(PB ? problem_params<GEO_RENDEZVOUS>(a.p_b, b) : a.dyn);
     const bool bounded = a.u_min != nullptr && a.u_max != nullptr;
     auto goal = problem_goal<RD, RNU>(a.cost, b);
     T z[NZ], zn[NZ];
@@ -247,10 +248,10 @@ __global__ void __launch_bounds__(64) lq_linearize_kernel(const LinKnownArgs<T> 
 // ------------------------------------------------------------------------------------------
 // rollout of one (problem, alpha)   ref: ilqr.py:677-723 + 764-791
 // ------------------------------------------------------------------------------------------
-template <class T, int ENC, bool STORE, bool STEP = false>
+template <class T, int ENC, bool STORE, bool STEP = false, bool PB = false>
 __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alpha) {
     constexpr int D = RD, NU = RNU, NZ = enc_size(D, ENC);
-    const RdvModel<T> md = rdv_model(a.dyn);
+    const RdvModel<T> md = rdv_model(PB ? problem_params<GEO_RENDEZVOUS>(a.p_b, b) : a.dyn);
     const bool bounded = a.u_min != nullptr && a.u_max != nullptr;
     auto goal = problem_goal<RD, RNU>(a.cost, b);           // (dead in the STORE pass, which evaluates no cost)
     T z[NZ], zn[NZ];
@@ -317,17 +318,17 @@ __device__ __forceinline__ T lq_roll_one(const RollKnownArgs<T>& a, int b, T alp
     return J;
 }
 
-template <class T, int ENC, bool STEP>
+template <class T, int ENC, bool STEP, bool PB>
 __global__ void __launch_bounds__(64) lq_rollout_kernel(const RollKnownArgs<T> a) {
     const int64_t id = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (id >= (int64_t)a.B * a.A) return;
     const int b = (int)(id / a.A), al = (int)(id - (int64_t)b * a.A);
     if ((a.active && a.active[b] == 0) || (a.bw_status && a.bw_status[b] != 0)) return;
-    a.J_all[id] = lq_roll_one<T, ENC, false, STEP>(a, b, a.alphas[al]);
+    a.J_all[id] = lq_roll_one<T, ENC, false, STEP, PB>(a, b, a.alphas[al]);
 }
 
 // argmin with torch semantics (first minimum; a NaN wins outright) + the winner's trajectory
-template <class T, int ENC>
+template <class T, int ENC, bool PB>
 __global__ void __launch_bounds__(64) lq_select_store_kernel(const RollKnownArgs<T> a) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= a.B) return;
@@ -342,7 +343,7 @@ __global__ void __launch_bounds__(64) lq_select_store_kernel(const RollKnownArgs
     }
     a.amin[b] = best;
     a.J_new[b] = bj;
-    lq_roll_one<T, ENC, true>(a, b, a.alphas[best]);
+    lq_roll_one<T, ENC, true, false, PB>(a, b, a.alphas[best]);
 }
 
 }  // namespace
@@ -351,8 +352,10 @@ template <class T>
 cudaError_t linearize_lq(int enc, const LinKnownArgs<T>& a, cudaStream_t s) {
     const int th = 64, grid = (a.B + th - 1) / th;
     const bool step = a.cost.xg_bt || a.cost.ug_bt;
-#define LQ_LIN(E) if (step) lq_linearize_kernel<T, E, true><<<grid, th, 0, s>>>(a); \
-                  else lq_linearize_kernel<T, E, false><<<grid, th, 0, s>>>(a); break;
+#define LQ_LIN(E) if (a.p_b) { if (step) lq_linearize_kernel<T, E, true, true><<<grid, th, 0, s>>>(a); \
+                               else lq_linearize_kernel<T, E, false, true><<<grid, th, 0, s>>>(a); } \
+                  else if (step) lq_linearize_kernel<T, E, true, false><<<grid, th, 0, s>>>(a); \
+                  else lq_linearize_kernel<T, E, false, false><<<grid, th, 0, s>>>(a); break;
     switch (enc) {
         case ENC_FULL: LQ_LIN(ENC_FULL)
         case ENC_UT: LQ_LIN(ENC_UT)
@@ -365,11 +368,12 @@ cudaError_t linearize_lq(int enc, const LinKnownArgs<T>& a, cudaStream_t s) {
     return cudaGetLastError();
 }
 
-template <class T>
-__global__ void __launch_bounds__(128) lq_env_step_kernel(int B, KnownParams<T> dyn, const T* x, const T* u, T* xn) {
+template <class T, bool PB>
+__global__ void __launch_bounds__(128) lq_env_step_kernel(int B, KnownParams<T> dyn, const T* p_b, const T* x, const T* u,
+                                                          T* xn) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
-    const RdvModel<T> md = rdv_model(dyn);
+    const RdvModel<T> md = rdv_model(PB ? problem_params<GEO_RENDEZVOUS>(p_b, b) : dyn);
     T xi[RD], ui[RNU], xo[RD];
 #pragma unroll
     for (int i = 0; i < RD; ++i) xi[i] = x[(int64_t)b * RD + i];
@@ -380,12 +384,15 @@ __global__ void __launch_bounds__(128) lq_env_step_kernel(int B, KnownParams<T> 
     for (int i = 0; i < RD; ++i) xn[(int64_t)b * RD + i] = xo[i];
 }
 template <class T>
-cudaError_t env_step_lq(int B, const KnownParams<T>& dyn, const T* x, const T* u, T* xn, cudaStream_t s) {
-    lq_env_step_kernel<T><<<(B + 127) / 128, 128, 0, s>>>(B, dyn, x, u, xn);
+cudaError_t env_step_lq(int B, const KnownParams<T>& dyn, const T* p_b, const T* x, const T* u, T* xn, cudaStream_t s) {
+    if (p_b) lq_env_step_kernel<T, true><<<(B + 127) / 128, 128, 0, s>>>(B, dyn, p_b, x, u, xn);
+    else lq_env_step_kernel<T, false><<<(B + 127) / 128, 128, 0, s>>>(B, dyn, p_b, x, u, xn);
     return cudaGetLastError();
 }
-template cudaError_t env_step_lq<float>(int, const KnownParams<float>&, const float*, const float*, float*, cudaStream_t);
-template cudaError_t env_step_lq<double>(int, const KnownParams<double>&, const double*, const double*, double*, cudaStream_t);
+template cudaError_t env_step_lq<float>(int, const KnownParams<float>&, const float*, const float*, const float*, float*,
+                                        cudaStream_t);
+template cudaError_t env_step_lq<double>(int, const KnownParams<double>&, const double*, const double*, const double*,
+                                         double*, cudaStream_t);
 
 template <class T>
 cudaError_t cost_derivatives_lq(int enc, const CostDerivArgs<T>& a, cudaStream_t s) {
@@ -408,9 +415,12 @@ cudaError_t rollout_lq(int enc, const RollKnownArgs<T>& a, cudaStream_t s) {
     const int th = 64;
     const unsigned g1 = (unsigned)(((int64_t)a.B * a.A + th - 1) / th), g2 = (a.B + th - 1) / th;
     const bool step = a.cost.xg_bt || a.cost.ug_bt;
-#define LQ_ROLL(E) if (step) lq_rollout_kernel<T, E, true><<<g1, th, 0, s>>>(a); \
-                   else lq_rollout_kernel<T, E, false><<<g1, th, 0, s>>>(a); \
-                   lq_select_store_kernel<T, E><<<g2, th, 0, s>>>(a); break;
+#define LQ_ROLL(E) if (a.p_b) { if (step) lq_rollout_kernel<T, E, true, true><<<g1, th, 0, s>>>(a); \
+                                else lq_rollout_kernel<T, E, false, true><<<g1, th, 0, s>>>(a); \
+                                lq_select_store_kernel<T, E, true><<<g2, th, 0, s>>>(a); } \
+                   else { if (step) lq_rollout_kernel<T, E, true, false><<<g1, th, 0, s>>>(a); \
+                          else lq_rollout_kernel<T, E, false, false><<<g1, th, 0, s>>>(a); \
+                          lq_select_store_kernel<T, E, false><<<g2, th, 0, s>>>(a); } break;
     switch (enc) {
         case ENC_FULL: LQ_ROLL(ENC_FULL)
         case ENC_UT: LQ_ROLL(ENC_UT)

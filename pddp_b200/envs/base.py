@@ -10,6 +10,7 @@ import ctypes as C
 import torch
 
 from .. import _lib
+from ..solver import check_dynamics_rows, require_single_system
 from ..utils.gaussian_variable import GaussianVariable
 
 
@@ -46,7 +47,9 @@ class Env(object):
 class KnownDynamicsEnv(Env):
     """`batch_size` instances of an environment whose step is `model(x, u, 0, IGNORE_UNCERTAINTY)`
     (ref: pddp/examples/*/env.py step()).  batch_size=None mirrors the reference exactly (state [D],
-    actions [nu]); with batch_size=B states are [B, D] and actions [B, nu]."""
+    actions [nu]); with batch_size=B states are [B, D] and actions [B, nu].  A model with B parameter sets
+    (KnownDynamicsModel) simulates instance b with set b, a fleet of different plants; batch_size=None needs one set.
+    The parameters are read when the environment is built."""
 
     initial_state = None      # mean of reset()
     reset_noise = 1e-2        # ref: examples/*/env.py reset(): state += 1e-2 * randn
@@ -61,8 +64,14 @@ class KnownDynamicsEnv(Env):
             raise RuntimeError("pddp_b200 environments live on CUDA devices only (no CPU fallback)")
         self._generator = generator
         self._desc = model.descriptor()
-        self._c_dyn = self._desc.c_struct()
         B = 1 if batch_size is None else int(batch_size)
+        if batch_size is None:
+            require_single_system(model, "KnownDynamicsEnv(batch_size=None)")
+        check_dynamics_rows(self._desc, B)
+        self._p_b = None                # device copy [B, 8] of per-instance parameters
+        if self._desc.params_b is not None:
+            self._p_b = torch.empty(B, 8, dtype=dtype, device=self.device).copy_(self._desc.params_b)
+        self._c_dyn = self._desc.c_struct(self._p_b)
         D, nu, _, _ = _lib.GEO_INFO[self._desc.geo]
         self._shape = _lib.Shape(_lib.dtype_code(dtype), _lib.PROBLEM_MAJOR, self._desc.geo, 4, B, 1, D, nu)
         self._state = torch.zeros(B, D, dtype=dtype, device=self.device)

@@ -4,7 +4,6 @@ device-resident environment whose ground truth is that model."""
 import math
 
 import torch
-from torch.nn import Parameter
 
 from ...costs.quadratic import QRCost
 from ...envs.base import KnownDynamicsEnv
@@ -26,9 +25,7 @@ class CartpoleDynamicsModel(KnownDynamicsModel):
 
     def __init__(self, dt, mc=0.5, mp=0.5, l=0.5, mu=0.1, g=9.82):
         super().__init__()
-        self.dt = Parameter(torch.tensor(dt), requires_grad=False)
-        for n, v in (("mc", mc), ("mp", mp), ("l", l), ("mu", mu), ("g", g)):
-            setattr(self, n, Parameter(torch.tensor(v), requires_grad=True))
+        self._init_params(dt, mc=mc, mp=mp, l=l, mu=mu, g=g)
 
 
 class CartpoleCost(QRCost):

@@ -4,7 +4,6 @@ device-resident environment whose ground truth is that model."""
 import math
 
 import torch
-from torch.nn import Parameter
 
 from ...costs.quadratic import QRCost
 from ...envs.base import KnownDynamicsEnv
@@ -26,9 +25,7 @@ class PendulumDynamicsModel(KnownDynamicsModel):
 
     def __init__(self, dt, m=1.0, l=1.0, mu=0.1, g=9.80665):
         super().__init__()
-        self.dt = Parameter(torch.tensor(dt), requires_grad=False)
-        for n, v in (("m", m), ("l", l), ("mu", mu), ("g", g)):
-            setattr(self, n, Parameter(torch.tensor(v), requires_grad=True))
+        self._init_params(dt, m=m, l=l, mu=mu, g=g)
 
 
 class PendulumCost(QRCost):

@@ -19,9 +19,12 @@ class SampleProblems(IntEnum):
                                             rendezvous.RendezvousDynamicsModel)}[self]
 
     def setup(self, dt, render=False, **kwargs):
-        """-> (env, cost, model)"""
+        """-> (env, cost, model).  Model parameters may be 1-D tensors of length B (e.g. m=masses): the model is then a
+        family of B systems and the environment simulates B instances, instance b with system b."""
         env_class, cost_class, model_class = self._classes()
-        return env_class(dt=dt, model=model_class(dt, **kwargs), render=render), cost_class(), model_class(dt, **kwargs)
+        model = model_class(dt, **kwargs)
+        env_opts = {"batch_size": model.n_sets} if model.n_sets > 1 else {}
+        return env_class(dt=dt, model=model_class(dt, **kwargs), render=render, **env_opts), cost_class(), model
 
     def get_env_class(self):
         return self._classes()[0]

@@ -4,7 +4,6 @@ device-resident environment whose ground truth is that model."""
 import math
 
 import torch
-from torch.nn import Parameter
 
 from ...costs.quadratic import QRCost
 from ...envs.base import KnownDynamicsEnv
@@ -23,9 +22,7 @@ class RendezvousDynamicsModel(KnownDynamicsModel):
 
     def __init__(self, dt, m=1.0, alpha=0.1):
         super().__init__()
-        self.dt = Parameter(torch.tensor(dt), requires_grad=False)
-        for n, v in (("m", m), ("alpha", alpha)):
-            setattr(self, n, Parameter(torch.tensor(v), requires_grad=True))
+        self._init_params(dt, m=m, alpha=alpha)
 
 
 class RendezvousCost(QRCost):

@@ -71,15 +71,67 @@ def _DA(model):
     return model.state_size + len(model.angular_indices)
 
 
+def _param_tensor(v):
+    """A closed-form model's parameter value: a scalar, or a 1-D tensor with one value per problem of a batch."""
+    t = v.detach().clone() if isinstance(v, torch.Tensor) else torch.tensor(v)
+    if not t.is_floating_point():
+        t = t.to(torch.get_default_dtype())
+    if t.dim() > 1:
+        raise ValueError("a dynamics parameter is a scalar or a 1-D tensor of one value per problem, got shape %s"
+                         % list(t.shape))
+    return t
+
+
 class KnownDynamicsModel(DynamicsModel):
     """Closed-form example dynamics (pddp/examples/<problem>/model.py): constants are Parameters like the
-    reference's; the step itself is a device function (csrc/core.cuh, csrc/known_lq.cu)."""
+    reference's; the step itself is a device function (csrc/core.cuh, csrc/known_lq.cu).
+
+    Every parameter, dt included, is a scalar or a 1-D tensor of length B: the model is then a family of B systems,
+    and like the reference's element-wise dynamics, row b of a [B, nz] batch integrates system b.  Scalars are shared
+    by all B.  Batched solves (iLQRController.fit / step with U [B, N, nu]), model(z [B, nz], u, i) and
+    KnownDynamicsEnv(model, batch_size=B) take such a model; entry points that evaluate one system need one set."""
     _param_order = ()
     action_size = 1
+
+    def _init_params(self, dt, **params):
+        """dt (a constant, like the reference's) and the named parameters (trainable), in _param_order."""
+        self.dt = torch.nn.Parameter(_param_tensor(dt), requires_grad=False)
+        for n, v in params.items():
+            setattr(self, n, torch.nn.Parameter(_param_tensor(v), requires_grad=True))
+        _ = self.n_sets                 # raises on 1-D parameters of different lengths
+
+    @property
+    def n_sets(self):
+        """Number of parameter sets: B when some parameter is a 1-D tensor of length B, else 1.  Raises ValueError
+        when 1-D parameters differ in length."""
+        lengths = {}
+        for n in self._param_order:
+            p = getattr(self, n)
+            if p.dim() > 1:
+                raise ValueError("dynamics parameter %s must be a scalar or 1-D, got shape %s" % (n, list(p.shape)))
+            if p.dim() == 1:
+                lengths[n] = int(p.shape[0])
+        if len(set(lengths.values())) > 1:
+            raise ValueError("per-problem dynamics parameters must have one length, got %s"
+                             % ", ".join("%s: %d" % kv for kv in lengths.items()))
+        n = next(iter(lengths.values()), 1)
+        if n < 1:
+            raise ValueError("per-problem dynamics parameters must not be empty")
+        return n
 
     def fit(self, X, U, dX, quiet=False, **kwargs):
         pass            # ref: examples/*/model.py -- known models have nothing to fit
 
     def descriptor(self):
+        """KnownDynamics: one shared parameter set, or with B sets the rows params_b [B, 8] (scalars repeated, in
+        _param_order, zero padded to 8)."""
         geo = geometry_of(self.state_size, self.angular_indices.tolist())
-        return KnownDynamics(geo, [float(getattr(self, n).detach()) for n in self._param_order])
+        n = self.n_sets
+        values = [getattr(self, k).detach() for k in self._param_order]
+        if n == 1:
+            return KnownDynamics(geo, [float(v.reshape(-1)[0]) for v in values])
+        dev = values[0].device
+        rows = torch.zeros(n, 8, dtype=torch.float64, device=dev)
+        for j, v in enumerate(values):
+            rows[:, j] = v.to(dtype=torch.float64, device=dev).expand(n)
+        return KnownDynamics(geo, [0.0] * len(values), rows)

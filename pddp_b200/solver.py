@@ -53,18 +53,55 @@ def step_alphas(dtype=torch.float32, device=None):
 
 
 class KnownDynamics:
-    """Closed-form dynamics constants (ref: pddp/examples/<problem>/model.py constructors)."""
+    """Closed-form dynamics constants (ref: pddp/examples/<problem>/model.py constructors).  `params` is the one
+    system every problem integrates; `params_b` [B, 8], if given, gives problem b its own system instead: row b holds
+    its parameters in the order of `params` (trailing entries unused)."""
 
-    def __init__(self, geo, params):
+    def __init__(self, geo, params, params_b=None):
         self.geo = geo
         self.params = [float(p) for p in params]
         self.is_bnn = False
+        if params_b is not None:
+            params_b = (params_b if isinstance(params_b, torch.Tensor) else torch.as_tensor(params_b)).detach()
+            if params_b.dim() != 2 or params_b.shape[1] != 8 or params_b.shape[0] < 1:
+                raise ValueError("per-problem dynamics parameters must have shape [B, 8], got %s"
+                                 % list(params_b.shape))
+        self.params_b = params_b
 
-    def c_struct(self):
-        s = _lib.KnownDynamics()
+    @property
+    def n_sets(self):
+        """Number of parameter sets: 1 (shared by every problem) or the B rows of params_b."""
+        return 1 if self.params_b is None else int(self.params_b.shape[0])
+
+    def rows(self, lo, hi):
+        """The dynamics of problems [lo, hi) (a shard of the batch)."""
+        return self if self.params_b is None else KnownDynamics(self.geo, self.params, self.params_b[lo:hi])
+
+    def c_struct(self, p_b=None):
+        """pddp_known_dynamics; p_b = the device copy of params_b the kernels read (BatchedSolver keeps it)."""
+        s = _lib.KnownDynamicsBatch()
         for i, p in enumerate(self.params):
             s.p[i] = p
+        s.p_b = None if p_b is None else p_b.data_ptr()
         return s
+
+
+def require_single_system(model, what):
+    """Raises ValueError when a closed-form model carries more than one parameter set: `what` evaluates one system."""
+    n = 1 if model is None or getattr(model, "is_bnn", False) else model.n_sets
+    if n != 1:
+        raise ValueError("%s evaluates one system, but the model carries %d parameter sets; per-problem dynamics run in "
+                         "batched calls (iLQRController.fit / step with U [B, N, nu], model(z [B, nz], u, i), "
+                         "KnownDynamicsEnv(model, batch_size=B))" % (what, n))
+
+
+def check_dynamics_rows(dyn, B):
+    """Raises ValueError unless a closed-form model's parameter sets fit a batch of B problems: one set (shared) or
+    B sets (one per problem)."""
+    n = dyn.n_sets
+    if n != 1 and n != B:
+        raise ValueError("the dynamics carry %d parameter sets, the batch has %d problem%s: per-problem parameters need "
+                         "one row per problem" % (n, B, "" if B == 1 else "s"))
 
 
 class BNNDynamics:
@@ -206,7 +243,10 @@ class BatchedSolver:
         self.shape = _lib.Shape(_lib.dtype_code(dtype), layout, self.geo, int(self.enc), self.B,
                                 self.N, self.nz, self.nu)
         self.c_cost = cost.c_struct()
-        self.c_dyn = dynamics.c_struct() if not dynamics.is_bnn else None
+        self.p_b = None            # device copy [B, 8] of per-problem dynamics parameters (set_dynamics)
+        self.c_dyn = None
+        if not dynamics.is_bnn:
+            self.set_dynamics(dynamics)
         nz, nu, N = self.nz, self.nu, self.N
         dims = dict(Z=(N + 1, nz), F_z=(N, nz * nz), F_u=(N, nz * nu), L=(N + 1, 1), L_z=(N + 1, nz),
                     L_u=(N, nu), L_zz=(N + 1, nz * nz), L_uz=(N, nu * nz), L_uu=(N, nu * nu),
@@ -278,6 +318,22 @@ class BatchedSolver:
         return v
 
     # ---------------------------------------------------------------- setup
+    def set_dynamics(self, dynamics):
+        """Closed-form dynamics constants: shared by every problem, or params_b [B, 8] with one row per problem,
+        copied to the device in the solver dtype.  Raises ValueError (before anything is launched) unless the rows
+        number B."""
+        if dynamics.is_bnn or dynamics.geo != self.geo:
+            raise ValueError("set_dynamics takes closed-form dynamics of the solver's geometry")
+        check_dynamics_rows(dynamics, self.B)
+        if dynamics.params_b is None:
+            self.p_b = None
+        else:
+            if self.p_b is None:
+                self.p_b = torch.empty(self.B, 8, dtype=self.dtype, device=self.device)
+            self.p_b.copy_(dynamics.params_b)
+        self.dyn = dynamics
+        self.c_dyn = dynamics.c_struct(self.p_b)
+
     def set_goals(self, x_goal=None, u_goal=None):
         """Gives every problem its own goal: x_goal [B, DA] in the cost's coordinates (the angle-augmented state,
         like QRCost.x_goal), u_goal [B, nu]; or a goal per problem and step, to track a reference: x_goal
@@ -447,9 +503,11 @@ def _zero_cost(geo):
     return QRCostConstants(torch.zeros(DA, DA), torch.zeros(nu, nu), torch.zeros(DA, DA), torch.zeros(DA))
 
 
-def cached_solver(model, cost, encoding, B, N, dtype, device, max_alphas=16, model_opts=None, layout=None):
+def cached_solver(model, cost, encoding, B, N, dtype, device, max_alphas=16, model_opts=None, layout=None,
+                  problems=None):
     """BatchedSolver for (model, cost) -- either may be None: a cost-only solver (pddp_cost_derivatives) or a
-    model-only one with a zero cost (model forward / eval_dynamics)."""
+    model-only one with a zero cost (model forward / eval_dynamics).  problems = (lo, hi): the solver holds problems
+    [lo, hi) of a larger batch (a shard), and takes those rows of a closed-form model's per-problem parameters."""
     if model is None and cost is None:
         raise ValueError("cached_solver needs a model or a cost")
     opts = tuple(sorted((model_opts or {}).items()))
@@ -468,6 +526,8 @@ def cached_solver(model, cost, encoding, B, N, dtype, device, max_alphas=16, mod
             desc = KnownDynamics(cost.geometry(), [0.0] * 8)
         else:
             desc = model.descriptor(dict(opts), N) if is_bnn else model.descriptor()
+            if not is_bnn and problems is not None:
+                desc = desc.rows(*problems)
         if cost is not None and model is not None and cost.geometry() != desc.geo:
             raise ValueError("model and cost disagree on the state geometry")
         consts = cost.constants() if cost is not None else _zero_cost(desc.geo)
@@ -481,8 +541,8 @@ def cached_solver(model, cost, encoding, B, N, dtype, device, max_alphas=16, mod
     if cost is not None:                                  # live constants, like the reference's live objects
         s.c_cost = cost.constants().c_struct()
     if model is not None and not s.dyn.is_bnn:
-        s.dyn = model.descriptor()
-        s.c_dyn = s.dyn.c_struct()
+        desc = model.descriptor()
+        s.set_dynamics(desc if problems is None else desc.rows(*problems))
     return s
 
 

@@ -9,7 +9,7 @@ cost), with B = 1, N = 1.  There is no CPU path.
 import torch
 
 from .. import _lib
-from ..solver import LIN_NAMES, cached_solver
+from ..solver import LIN_NAMES, cached_solver, require_single_system
 from .encoding import StateEncoding
 
 
@@ -43,6 +43,7 @@ def eval_cost(cost, z, u, i, terminal=False, encoding=StateEncoding.DEFAULT, app
 def eval_dynamics(model, z, u, i, encoding=StateEncoding.DEFAULT, **kwargs):
     """-> (z_next [nz], dz'/dz [nz, nz], dz'/du [nz, nu]).  ref: pddp/utils/evaluation.py:97-131.
     `kwargs` are the model options (use_predicted_std, infer_noise_variables, ...)."""
+    require_single_system(model, "eval_dynamics")
     _lib.require_cuda(z, "z")
     if getattr(model, "is_bnn", False) and int(i) != 0:
         raise NotImplementedError("pddp_b200: a stand-alone BNN evaluation is only defined for step 0 (particles drawn "
